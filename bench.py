@@ -49,7 +49,15 @@ def parse_args():
     ap.add_argument("--no-pipeline", action="store_true", help="skip the text -> BWT leg (parse + bwtparse + pfbwt, N=1 only)")
     ap.add_argument("--merge", default="partition", choices=["partition", "replicate"],
                     help="multi-GPU dictionary merge: range-partitioned all-to-all or replicated all-gather")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the five streams of the last timed step to DIR/<stream>.npy; covers the "
+                         "single-GPU path only (refused with --gpus > 1)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.gpus != 1:
+        ap.error("--dump-outputs needs --gpus 1")
+    return a
 
 
 def workload_name(a, world=None):
@@ -320,6 +328,37 @@ def parity_check(job, pkg, synth, world, rank, local, dev, merge):
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path handed its caller, for comparing two builds output by output
+# ------------------------------------------------------------------------------------------------
+DUMP_MAX_ELEMS, DUMP_SEED = 1 << 20, 12345     # at most 5 x 8 MB of float64
+
+
+def dump_outputs(files, out_dir):
+    """Each of the five streams as DIR/<stream>.npy: .dict and .last bytes as float32, .occ and .parse
+    ranks and the 5-byte .sai positions as float64 (all exact).  A stream longer than DUMP_MAX_ELEMS
+    is replaced by the elements at a sorted sample of positions drawn with DUMP_SEED, which depends on
+    nothing but the stream's length.  Returns {stream: [full length, elements stored]}."""
+    import numpy as np
+    sai = np.frombuffer(files.sai, np.uint8).reshape(-1, 5)
+    streams = {"dict": (np.frombuffer(files.dict, np.uint8), np.float32),
+               "occ": (np.frombuffer(files.occ, np.uint32), np.float64),
+               "parse": (np.frombuffer(files.parse, np.uint32), np.float64),
+               "last": (np.frombuffer(files.last, np.uint8), np.float32),
+               "sai": (sai, np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    info = {}
+    for name, (a, dtype) in streams.items():
+        n = len(a)
+        if n > DUMP_MAX_ELEMS:
+            a = a[np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_ELEMS, replace=False))]
+        if name == "sai":
+            a = sum(a[:, i].astype(np.uint64) << np.uint64(8 * i) for i in range(5)) if len(a) else a[:, 0]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(dtype))
+        info[name] = [n, len(a)]
+    return info
+
+
+# ------------------------------------------------------------------------------------------------
 # T2 (SURVEY 8d): page-cache-warm FASTA file -> five files closed, wall clock of the gpuscan.x process
 # ------------------------------------------------------------------------------------------------
 def pipeline_to_bwt(pkg, device, text, steps=3, cpu_sample_bytes=0):
@@ -515,6 +554,9 @@ def main():
         gathered = [None] * world
         dist.all_gather_object(gathered, {k: round(v, 3) for k, v in stage_ms.items() if k.startswith("ms_phase_")})
         per_rank = {k: [g.get(k, 0.0) for g in gathered] for k in gathered[0]}
+    dumped = None
+    if a.dump_outputs:                 # before the legs below run the parser again
+        dumped = dump_outputs(job.scanner.fetch(job.out), a.dump_outputs)
 
     # ---- the stages after the parse (SURVEY 8f rows 2-3), N = 1: text in HBM -> BWT in HBM ---------
     pipeline = None
@@ -619,6 +661,8 @@ def main():
         line["t2_file_to_files"] = t2
     if pipeline is not None:
         line["pipeline_to_bwt"] = pipeline
+    if dumped is not None:
+        line["dump_outputs"] = {"dir": a.dump_outputs, "length_and_stored": dumped}
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,7 +1,7 @@
 """The stage after the parse on the GPU (pfpb200_bwtparse_*, SURVEY 8(f) row 3) against the
 reference's bwtparse: byte-identical .ilist / .bwlast / .bwsai -- golden outputs of the unmodified
 binary (tests/golden/golden_bwtparse.npz), the numpy restatement at sizes the binary is not needed
-for, live runs of the binary, and the unchanged pfbwtNT.x downstream of our files."""
+for, and gpubwtparse.x on the files of the unmodified chain."""
 import os
 import shutil
 import subprocess
@@ -12,8 +12,7 @@ import pytest
 import torch
 
 from oracle import bwtparse_oracle as bo
-from oracle import pfp_oracle as orc
-from test_oracle_golden import _bwtparse_golden
+from test_oracle_golden import _bwtparse_golden, _pfbwt_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -84,42 +83,42 @@ def test_properties_at_40m_phrases_scale_model(pkg, sc):
     assert r.rounds <= 16
 
 
-@pytest.mark.skipif(not (orc.have_ref("bwtparse") and orc.have_ref("pfbwtNT.x")), reason="oracle/_ref not built")
 def test_cli_matches_reference_and_feeds_pfbwt(pkg):
-    """gpubwtparse.x as the drop-in for bwtparse: same files, with and without -t segments, and
-    the UNCHANGED pfbwtNT.x turns them into the same .bwt / .sa as the all-reference chain."""
-    recs = [r.numpy() for r in pkg.synth.pangenome_records(60_000, 8, 33)]
-    fa = pkg.synth.to_fasta(recs)
+    """gpubwtparse.x as the drop-in for bwtparse: on the files newscanNT.x wrote it writes the files
+    bwtparse wrote, with and without -t segments, and gpupfbwt.x turns them into the .bwt / .sa of the
+    all-reference chain (tests/golden: golden_bwtparse.npz and golden_pfbwt.npz hold the same text)."""
+    name = "pangenome_20k_x6_w10_p100"
+    ref = dict(_bwtparse_golden()[name])
+    ref.update(_pfbwt_golden()[name])
+    w, p = str(ref["w"]), str(ref["p"])
     tmp = tempfile.mkdtemp(prefix="bwtparsecli_")
     try:
-        ours, ref = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "ref.fa")
-        for pth in (ours, ref):
-            with open(pth, "wb") as f:
-                f.write(fa)
-            subprocess.run([pkg.pfp.CLI_PATH, pth, "-w", "10", "-p", "100", "-s", "-f"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("bwtparse"), ref, "-s"], check=True, stdout=subprocess.PIPE)
+        ours = os.path.join(tmp, "ours")
+        for ext in ("dict", "occ", "parse", "last", "sai"):
+            with open(ours + "." + ext, "wb") as f:
+                f.write(ref[ext])
         r = subprocess.run([pkg.pfp.BWTPARSE_CLI_PATH, ours, "-s"], check=True, stdout=subprocess.PIPE, text=True)
         assert "ilist positions written" in r.stdout and "bwlast chars written" in r.stdout
         for ext in ("ilist", "bwlast", "bwsai"):
-            assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), ext
-        for base in (ours, ref):
-            subprocess.run([orc.ref_exe("pfbwtNT.x"), "-w", "10", base, "-S"], check=True, stdout=subprocess.PIPE)
+            assert open(ours + "." + ext, "rb").read() == ref[ext], ext
+        subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", w, ours, "-S"], check=True, stdout=subprocess.PIPE)
         for ext in ("bwt", "sa"):
-            assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), ext
+            assert open(ours + "." + ext, "rb").read() == ref[ext], ext
         # segmented .last/.sai, as `bigbwt -t 3` leaves them for `bwtparse -t 3`
-        seg = os.path.join(tmp, "seg.fa")
-        shutil.copy(ref, seg)
-        subprocess.run([pkg.pfp.CLI_PATH, seg, "-w", "10", "-p", "100", "-s", "-f", "-t", "3"], check=True, stdout=subprocess.PIPE)
+        seg = os.path.join(tmp, "seg")
+        with open(seg, "wb") as f:
+            f.write(ref["text"])
+        subprocess.run([pkg.pfp.CLI_PATH, seg, "-w", w, "-p", p, "-s", "-t", "3"], check=True, stdout=subprocess.PIPE)
         subprocess.run([pkg.pfp.BWTPARSE_CLI_PATH, seg, "-s", "-t", "3"], check=True, stdout=subprocess.PIPE)
         for ext in ("ilist", "bwlast", "bwsai"):
-            assert open(seg + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), "-t 3 " + ext
+            assert open(seg + "." + ext, "rb").read() == ref[ext], "-t 3 " + ext
         # without -s: no .bwsai
-        nos = os.path.join(tmp, "nos.fa")
-        shutil.copy(ref, nos)
+        nos = os.path.join(tmp, "nos")
         for ext in ("parse", "last"):
-            shutil.copy(ref + "." + ext, nos + "." + ext)
+            with open(nos + "." + ext, "wb") as f:
+                f.write(ref[ext])
         subprocess.run([pkg.pfp.BWTPARSE_CLI_PATH, nos], check=True, stdout=subprocess.PIPE)
-        assert open(nos + ".ilist", "rb").read() == open(ref + ".ilist", "rb").read() and not os.path.exists(nos + ".bwsai")
+        assert open(nos + ".ilist", "rb").read() == ref["ilist"] and not os.path.exists(nos + ".bwsai")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
 

@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import assert_same_files
+from conftest import assert_same_files, golden
 from oracle import pfp_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -132,40 +132,36 @@ def test_multi_64mb_equals_single_gpu(pkg):
             ms.close()
 
 
-@pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built")
 def test_cli_multi_gpu_files_match_reference(pkg):
-    """`gpuscan.x -g 0,0,0` (or real GPUs) writes the same files as the unmodified newscanNT.x,
-    plain and FASTA, and `-t 2` segments concatenate to the same streams."""
+    """`gpuscan.x -g 0,0,0` (or real GPUs) writes the files the unmodified newscanNT.x wrote for the
+    stored plain and FASTA inputs (tests/golden, cases pangenome_plain / pangenome_fasta: the same
+    text), through gzip too, and `-t 2` segments concatenate to the same streams.  Shards down to
+    4 KB (the small_shards settings) so that these 36 KB inputs are cut at several seams."""
     n = torch.cuda.device_count()
     devs = ",".join(map(str, range(n))) if n > 1 else "0,0,0"
-    recs = [r.numpy() for r in pkg.synth.pangenome_records(60_000, 6, 177)]
+    env = dict(os.environ, PFPB200_MULTI_MIN_SHARD="4096", PFPB200_MULTI_FRONT="256")
+    run = lambda cmd: subprocess.run(cmd, check=True, stdout=subprocess.PIPE, text=True, env=env)  # noqa: E731
+    plain, fasta = golden().case("pangenome_plain"), golden().case("pangenome_fasta")
     tmp = tempfile.mkdtemp(prefix="pfpmulti_")
     try:
-        for fasta in (False, True):
-            data = pkg.synth.to_fasta(recs) if fasta else b"".join(r.tobytes() for r in recs)
-            ours, ref = os.path.join(tmp, f"ours{int(fasta)}"), os.path.join(tmp, f"ref{int(fasta)}")
-            for pth in (ours, ref):
-                with open(pth, "wb") as f:
-                    f.write(data)
-            extra = ["-f"] if fasta else []
-            r = subprocess.run([pkg.pfp.CLI_PATH, ours, "-w", "10", "-p", "100", "-s", "-g", devs, "-v"] + extra,
-                               check=True, stdout=subprocess.PIPE, text=True)
+        for c, extra in ((plain, []), (fasta, ["-f"])):
+            ours = os.path.join(tmp, c["name"])
+            with open(ours, "wb") as f:
+                f.write(c["input"])
+            r = run([pkg.pfp.CLI_PATH, ours, "-w", str(c["w"]), "-p", str(c["p"]), "-s", "-g", devs, "-v"] + extra)
             assert "merge" in r.stdout          # the per-GPU timeline of -v
-            subprocess.run([orc.ref_exe("newscanNT.x"), ref, "-w", "10", "-p", "100", "-s"] + extra, check=True,
-                           stdout=subprocess.PIPE)
-            assert_same_files(orc.collect_files(ours), orc.collect_files(ref), f"cli -g {devs} fasta={fasta}")
+            assert_same_files(orc.collect_files(ours), c, f"cli -g {devs} {c['name']}")
         # gzip-compressed FASTA goes through the host reader (zlib, as the reference's gzread)
         import gzip
         gzp = os.path.join(tmp, "ours.gz")
         with gzip.open(gzp, "wb") as f:
-            f.write(pkg.synth.to_fasta(recs))
-        subprocess.run([pkg.pfp.CLI_PATH, gzp, "-w", "10", "-p", "100", "-s", "-f", "-g", devs], check=True,
-                       stdout=subprocess.PIPE)
-        assert_same_files(orc.collect_files(gzp), orc.collect_files(os.path.join(tmp, "ref1")), "cli multi gzip")
+            f.write(fasta["input"])
+        run([pkg.pfp.CLI_PATH, gzp, "-w", str(fasta["w"]), "-p", str(fasta["p"]), "-s", "-f", "-g", devs])
+        assert_same_files(orc.collect_files(gzp), fasta, "cli multi gzip")
         seg = os.path.join(tmp, "seg")
-        shutil.copy(os.path.join(tmp, "ref0"), seg)
-        subprocess.run([pkg.pfp.CLI_PATH, seg, "-w", "10", "-p", "100", "-s", "-g", devs, "-t", "2"], check=True,
-                       stdout=subprocess.PIPE)
-        assert_same_files(orc.collect_files(seg, nseg=2), orc.collect_files(os.path.join(tmp, "ref0")), "cli -t 2")
+        with open(seg, "wb") as f:
+            f.write(plain["input"])
+        run([pkg.pfp.CLI_PATH, seg, "-w", str(plain["w"]), "-p", str(plain["p"]), "-s", "-g", devs, "-t", "2"])
+        assert_same_files(orc.collect_files(seg, nseg=2), plain, "cli -t 2")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)

@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from conftest import assert_same_files, golden, golden_dicz, golden_names
+from oracle import pfbwt_oracle as po
 from oracle import pfp_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -331,79 +332,67 @@ def test_round_trip_properties_32mb(pkg, sc):
     assert np.array_equal(last[:-1], tb[pos[:-1].astype(np.int64) - 1 - w]) and last[-1] == tb[-1]
 
 
-@pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built")
 def test_cli_files_and_bwt_match_reference(pkg):
-    """gpuscan.x as the drop-in for newscan.x: byte-identical files, and the UNCHANGED bwtparse +
-    pfbwtNT.x turn them into the same .bwt/.sa as the all-reference pipeline (bigbwt -f -S)."""
-    recs = [r.numpy() for r in pkg.synth.pangenome_records(40_000, 6, 95)]
-    fa = pkg.synth.to_fasta(recs)
+    """gpuscan.x as the drop-in for newscan.x: byte-identical to the files newscanNT.x -s -f wrote for a
+    stored FASTA (tests/golden, case pangenome_fasta), also as -t 3 segments and through gzip; and
+    gpubwtparse.x + gpupfbwt.x turn them into the BWT and suffix array of the text (bigbwt -f -S)."""
+    c = golden().case("pangenome_fasta")
+    w, p = str(c["w"]), str(c["p"])
     tmp = tempfile.mkdtemp(prefix="pfpcli_")
     try:
-        ours, ref = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "ref.fa")
-        for pth in (ours, ref):
+        ours, seg = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "seg.fa")
+        for pth in (ours, seg):
             with open(pth, "wb") as f:
-                f.write(fa)
-        subprocess.run([pkg.pfp.CLI_PATH, ours, "-w", "10", "-p", "100", "-s", "-f"], check=True,
-                       stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("newscanNT.x"), ref, "-w", "10", "-p", "100", "-s", "-f"], check=True,
-                       stdout=subprocess.PIPE)
-        assert_same_files(orc.collect_files(ours), orc.collect_files(ref), "cli")
-        for base in (ours, ref):
-            subprocess.run([orc.ref_exe("bwtparse"), base, "-s"], check=True, stdout=subprocess.PIPE)
-            subprocess.run([orc.ref_exe("pfbwtNT.x"), "-w", "10", base, "-S"], check=True, stdout=subprocess.PIPE)
+                f.write(c["input"])
+        subprocess.run([pkg.pfp.CLI_PATH, ours, "-w", w, "-p", p, "-s", "-f"], check=True, stdout=subprocess.PIPE)
+        assert_same_files(orc.collect_files(ours), c, "cli")
+        subprocess.run([pkg.pfp.BWTPARSE_CLI_PATH, ours, "-s"], check=True, stdout=subprocess.PIPE)
+        subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", w, ours, "-S"], check=True, stdout=subprocess.PIPE)
+        want = po.pfbwt(orc.fasta_extract(c["input"])[0])
         for ext in ("bwt", "sa"):
-            assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), ext
+            assert open(ours + "." + ext, "rb").read() == want[ext], ext
         # segmented .last/.sai (-t 3) concatenate to the same streams
-        seg = os.path.join(tmp, "seg.fa")
-        shutil.copy(ref, seg)
-        subprocess.run([pkg.pfp.CLI_PATH, seg, "-w", "10", "-p", "100", "-s", "-f", "-t", "3"], check=True,
+        subprocess.run([pkg.pfp.CLI_PATH, seg, "-w", w, "-p", p, "-s", "-f", "-t", "3"], check=True,
                        stdout=subprocess.PIPE)
-        assert_same_files(orc.collect_files(seg, nseg=3), orc.collect_files(ref), "cli -t 3")
+        assert_same_files(orc.collect_files(seg, nseg=3), c, "cli -t 3")
         # gzip-compressed FASTA, as the reference's kseq/gzread takes it
         import gzip
-        for base in ("ours", "ref"):
-            with gzip.open(os.path.join(tmp, base + ".gz"), "wb") as f:
-                f.write(fa)
-        subprocess.run([pkg.pfp.CLI_PATH, os.path.join(tmp, "ours.gz"), "-w", "10", "-p", "100", "-s", "-f"],
-                       check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("newscanNT.x"), os.path.join(tmp, "ref.gz"), "-w", "10", "-p", "100", "-s", "-f"],
-                       check=True, stdout=subprocess.PIPE)
-        assert_same_files(orc.collect_files(os.path.join(tmp, "ours.gz")), orc.collect_files(os.path.join(tmp, "ref.gz")),
-                          "cli gzip")
+        gz = os.path.join(tmp, "ours.gz")
+        with gzip.open(gz, "wb") as f:
+            f.write(c["input"])
+        subprocess.run([pkg.pfp.CLI_PATH, gz, "-w", w, "-p", p, "-s", "-f"], check=True, stdout=subprocess.PIPE)
+        assert_same_files(orc.collect_files(gz), c, "cli gzip")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
 
 
-@pytest.mark.skipif(not (orc.have_ref() and orc.have_ref("simplebwt")), reason="oracle/_ref not built")
 def test_config1_yeast_shaped_fasta_to_bwt(pkg):
-    """BASELINE config 1 (`bigbwt yeast.fasta -w 10 -p 100`; the bundled file is absent from the
-    mount, so a stand-in of its shape: 17 records, 12.16 Mbp, 60-column FASTA).  gpuscan.x replaces
-    the scanner; the UNCHANGED bwtparse + pfbwtNT.x turn its files into the .bwt/.sa of the
-    all-reference chain, and the .bwt equals the one SACA-K (simplebwt) computes from the extracted
-    text -- the check `bigbwt -c` does (bigbwt:176-195; on the extracted text, SURVEY App. B3)."""
+    """BASELINE config 1 (`bigbwt yeast.fasta -w 10 -p 100`; the bundled file is not in the repository,
+    so a stand-in of its shape: 17 records, 12.16 Mbp, 60-column FASTA).  gpuscan.x, gpubwtparse.x and
+    gpupfbwt.x write the files of newscanNT.x -s -f, bwtparse -s and pfbwtNT.x -S (sha256 in
+    tests/golden/config1_sha256.json), and the .bwt is the BWT of the extracted text -- the check
+    `bigbwt -c` does (bigbwt:176-195; on the extracted text, SURVEY App. B3)."""
+    import hashlib
+    import json
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "config1_sha256.json")) as f:
+        want_sha = json.load(f)["sha256"]
     recs = [r.numpy() for r in pkg.synth.yeast_like_records(1)]
     assert len(recs) == 17 and 12_000_000 < sum(r.size for r in recs) < 12_300_000
     fa = b"".join(pkg.synth.to_fasta_np(r, f"{nm} stand-in").tobytes() for r, nm in zip(recs, pkg.synth.YEAST_NAMES))
     tmp = tempfile.mkdtemp(prefix="pfpyeast_")
     try:
-        ours, ref, txt = (os.path.join(tmp, x) for x in ("ours.fa", "ref.fa", "text"))
-        for pth in (ours, ref):
-            with open(pth, "wb") as f:
-                f.write(fa)
+        ours = os.path.join(tmp, "ours.fa")
+        with open(ours, "wb") as f:
+            f.write(fa)
         run = lambda cmd: subprocess.run(cmd, check=True, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)  # noqa: E731
         run([pkg.pfp.CLI_PATH, ours, "-w", "10", "-p", "100", "-s", "-f"])
-        run([orc.ref_exe("newscanNT.x"), ref, "-w", "10", "-p", "100", "-s", "-f"])
-        assert_same_files(orc.collect_files(ours), orc.collect_files(ref), "config 1 scanner files")
-        for base in (ours, ref):
-            run([orc.ref_exe("bwtparse"), base, "-s"])
-            run([orc.ref_exe("pfbwtNT.x"), "-w", "10", base, "-S"])
-        for ext in ("bwt", "sa"):
-            assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), ext
+        run([pkg.pfp.BWTPARSE_CLI_PATH, ours, "-s"])
+        run([pkg.pfp.PFBWT_CLI_PATH, "-w", "10", ours, "-S"])
+        for ext, sha in want_sha.items():
+            with open(ours + "." + ext, "rb") as f:
+                assert hashlib.sha256(f.read()).hexdigest() == sha, f".{ext} differs from the reference's"
         text, trunc = pkg.pfp.read_input(ours, fasta=True)
         assert not trunc and text == b"".join(r.tobytes() for r in recs)
-        with open(txt, "wb") as f:
-            f.write(text)
-        run([orc.ref_exe("simplebwt"), txt])
-        assert open(ours + ".bwt", "rb").read() == open(txt + ".Bwt", "rb").read(), "BWT differs from SACA-K"
+        assert open(ours + ".bwt", "rb").read() == po.pfbwt(text)["bwt"], "BWT differs from the suffix array of the text"
     finally:
         shutil.rmtree(tmp, ignore_errors=True)

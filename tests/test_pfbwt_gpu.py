@@ -1,7 +1,7 @@
 """The last stage on the GPU (pfpb200_pfbwt_*, SURVEY 8(f) row 2) against the reference's pfbwt:
 byte-identical .bwt / .sa / .ssa / .esa -- golden outputs of the unmodified chain
 (tests/golden/golden_pfbwt.npz), the whole pipeline parse -> bwtparse -> pfbwt in HBM against the
-suffix array of the text, and gpupfbwt.x against pfbwtNT.x on files."""
+suffix array of the text, and gpupfbwt.x / gpubigbwt.x against the files of the unmodified chain."""
 import os
 import shutil
 import subprocess
@@ -12,8 +12,7 @@ import pytest
 import torch
 
 from oracle import pfbwt_oracle as po
-from oracle import pfp_oracle as orc
-from test_oracle_golden import _pfbwt_golden
+from test_oracle_golden import _bwtparse_golden, _pfbwt_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -98,28 +97,42 @@ def test_tandem_repeats_words_with_thousands_of_occurrences(pkg, sc):
         assert _fetch(sc, r)["bwt"] == want["bwt"]
 
 
-@pytest.mark.skipif(not (po.have_reference() and orc.have_ref("bwtparse")), reason="oracle/_ref not built")
+def reference_chain(name="pangenome_20k_x6_w10_p100"):
+    """Every file the unmodified chain newscanNT.x -s -> bwtparse -s -> pfbwtNT.x wrote for one stored
+    text (tools/make_golden_bwtparse.py and tools/make_golden_pfbwt.py ran it on the same text)."""
+    c = dict(_bwtparse_golden()[name])
+    c.update(_pfbwt_golden()[name])
+    return c
+
+
+def write_fasta(pkg, path, text):
+    """`text` as a one-record FASTA file: the text the tools extract from it is `text` again."""
+    with open(path, "wb") as f:
+        f.write(pkg.synth.to_fasta([np.frombuffer(text, np.uint8)]))
+
+
 def test_cli_matches_reference(pkg):
-    """gpupfbwt.x as the drop-in for pfbwtNT.x, and the whole GPU chain gpuscan.x -> gpubwtparse.x ->
-    gpupfbwt.x against the all-reference chain: same .bwt / .sa / .ssa / .esa."""
-    recs = [r.numpy() for r in pkg.synth.pangenome_records(50_000, 8, 35)]
-    fa = pkg.synth.to_fasta(recs)
+    """gpupfbwt.x as the drop-in for pfbwtNT.x on the reference's own intermediate files, and the whole
+    GPU chain gpuscan.x -> gpubwtparse.x -> gpupfbwt.x on the text: the .bwt / .sa / .ssa / .esa the
+    all-reference chain wrote."""
+    ref = reference_chain()
+    w, p = str(ref["w"]), str(ref["p"])
     tmp = tempfile.mkdtemp(prefix="pfbwtcli_")
     try:
-        ours, ref = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "ref.fa")
-        for pth in (ours, ref):
-            with open(pth, "wb") as f:
-                f.write(fa)
-        subprocess.run([orc.ref_exe("newscanNT.x"), ref, "-w", "10", "-p", "100", "-s", "-f"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("bwtparse"), ref, "-s"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([pkg.pfp.CLI_PATH, ours, "-w", "10", "-p", "100", "-s", "-f"], check=True, stdout=subprocess.PIPE)
+        drop, ours = os.path.join(tmp, "drop"), os.path.join(tmp, "ours.fa")
+        for ext in ("dict", "occ", "ilist", "bwlast", "bwsai"):
+            with open(drop + "." + ext, "wb") as f:
+                f.write(ref[ext])
+        write_fasta(pkg, ours, ref["text"])
+        subprocess.run([pkg.pfp.CLI_PATH, ours, "-w", w, "-p", p, "-s", "-f"], check=True, stdout=subprocess.PIPE)
         subprocess.run([pkg.pfp.BWTPARSE_CLI_PATH, ours, "-s"], check=True, stdout=subprocess.PIPE)
         for flags, exts in ((["-S"], ("bwt", "sa")), (["-s", "-e"], ("bwt", "ssa", "esa")), ([], ("bwt",))):
-            subprocess.run([orc.ref_exe("pfbwtNT.x"), "-w", "10", *flags, ref], check=True, stdout=subprocess.PIPE)
-            r = subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", "10", *flags, ours], check=True, stdout=subprocess.PIPE, text=True)
-            assert "Easy bwt chars" in r.stdout and "Hard bwt chars" in r.stdout
-            for ext in exts:
-                assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), (flags, ext)
+            for base in (drop, ours):
+                r = subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", w, *flags, base], check=True, stdout=subprocess.PIPE,
+                                   text=True)
+                assert "Easy bwt chars" in r.stdout and "Hard bwt chars" in r.stdout
+                for ext in exts:
+                    assert open(base + "." + ext, "rb").read() == ref[ext], (base, flags, ext)
         r = subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", "10", "-S", "-s", ours], capture_output=True, text=True)
         assert r.returncode == 1 and "not both" in r.stdout
         r = subprocess.run([pkg.pfp.PFBWT_CLI_PATH, "-w", "10", os.path.join(tmp, "missing")], capture_output=True, text=True)
@@ -128,30 +141,23 @@ def test_cli_matches_reference(pkg):
         shutil.rmtree(tmp, ignore_errors=True)
 
 
-@pytest.mark.skipif(not (po.have_reference() and orc.have_ref("bwtparse")), reason="oracle/_ref not built")
 def test_gpubigbwt_one_process_matches_the_reference_chain(pkg):
-    """gpubigbwt.x: file in, .bwt / .sa out, the three stages in HBM in one process -- against
-    newscanNT.x + bwtparse + pfbwtNT.x; with -k the intermediate files are the reference's too."""
-    recs = [r.numpy() for r in pkg.synth.pangenome_records(50_000, 6, 37)]
-    fa = pkg.synth.to_fasta(recs)
+    """gpubigbwt.x: file in, .bwt / .sa out, the three stages in HBM in one process -- against the
+    files newscanNT.x + bwtparse + pfbwtNT.x wrote; with -k the intermediate files are the reference's too."""
+    ref = reference_chain()
+    assert (ref["w"], ref["p"]) == (10, 100)            # the defaults the run without -w / -p relies on
     tmp = tempfile.mkdtemp(prefix="bigbwtcli_")
     try:
-        ours, ref = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "ref.fa")
-        for pth in (ours, ref):
-            with open(pth, "wb") as f:
-                f.write(fa)
-        subprocess.run([orc.ref_exe("newscanNT.x"), ref, "-w", "10", "-p", "100", "-s", "-f"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("bwtparse"), ref, "-s"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("pfbwtNT.x"), "-w", "10", "-S", ref], check=True, stdout=subprocess.PIPE)
+        ours, plain = os.path.join(tmp, "ours.fa"), os.path.join(tmp, "plain.fa")
+        for pth in (ours, plain):
+            write_fasta(pkg, pth, ref["text"])
         r = subprocess.run([pkg.pfp.BIGBWT_CLI_PATH, ours, "-w", "10", "-p", "100", "-f", "-S", "-k"], check=True,
                            stdout=subprocess.PIPE, text=True)
         assert "Hard bwt chars" in r.stdout
         for ext in ("bwt", "sa", "dict", "occ", "parse", "last", "sai", "ilist", "bwlast", "bwsai"):
-            assert open(ours + "." + ext, "rb").read() == open(ref + "." + ext, "rb").read(), ext
-        plain = os.path.join(tmp, "plain.fa")
-        shutil.copy(ref, plain)
+            assert open(ours + "." + ext, "rb").read() == ref[ext], ext
         subprocess.run([pkg.pfp.BIGBWT_CLI_PATH, plain, "-f"], check=True, stdout=subprocess.PIPE)
-        assert open(plain + ".bwt", "rb").read() == open(ref + ".bwt", "rb").read()
+        assert open(plain + ".bwt", "rb").read() == ref["bwt"]
         assert not os.path.exists(plain + ".dict") and not os.path.exists(plain + ".sa")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)

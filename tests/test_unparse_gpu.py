@@ -10,8 +10,6 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import pfp_oracle as orc
-
 pytestmark = pytest.mark.gpu
 
 
@@ -68,8 +66,9 @@ def test_invalid_word_id(pkg, sc):
     assert e.value.code == -1
 
 
-@pytest.mark.skipif(not orc.have_ref("unparse"), reason="oracle/_ref not built")
 def test_cli_matches_reference_unparse(pkg):
+    """gpuunparse.x on the -c files of gpuscan.x writes <base>.out (or -o) holding the text, as the
+    reference's unparse does."""
     text = pkg.synth.pangenome_text(80_000, 7, 21).numpy().tobytes()
     tmp = tempfile.mkdtemp(prefix="unparsecli_")
     try:
@@ -77,11 +76,8 @@ def test_cli_matches_reference_unparse(pkg):
         with open(base, "wb") as f:
             f.write(text)
         subprocess.run([pkg.pfp.CLI_PATH, base, "-w", "10", "-p", "100", "-c"], check=True, stdout=subprocess.PIPE)
-        subprocess.run([orc.ref_exe("unparse"), base, "-o", base + ".ref"], check=True, stdout=subprocess.PIPE,
-                       stderr=subprocess.PIPE)
         subprocess.run([pkg.pfp.UNPARSE_CLI_PATH, base], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-        got = open(base + ".out", "rb").read()
-        assert got == open(base + ".ref", "rb").read() == text
+        assert open(base + ".out", "rb").read() == text
         subprocess.run([pkg.pfp.UNPARSE_CLI_PATH, base, "-o", os.path.join(tmp, "named")], check=True,
                        stdout=subprocess.PIPE, stderr=subprocess.PIPE)
         assert open(os.path.join(tmp, "named"), "rb").read() == text
