@@ -98,6 +98,7 @@ extern "C" int pfpb200_create(int device, pfpb200_ctx **out) {
     { const char *ev = getenv("PFPB200_NO_SCAN_ALPHA"); ctx->no_scan_alpha = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_RANK_FULL_SORT"); ctx->rank_full_sort = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_RANK_CHUNK_PASSES"); ctx->rank_chunk_passes = ev && atoi(ev) != 0; }
+    { const char *ev = getenv("PFPB200_RANK_WARP_PASSES"); ctx->rank_warp_passes = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_POOL_BY_WORD"); ctx->pool_by_word = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_FUSE_K3"); ctx->fuse_k3 = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_TABLE_SCALE"); if (ev && atof(ev) >= 1.2) ctx->table_scale = atof(ev); }

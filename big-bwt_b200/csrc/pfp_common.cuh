@@ -77,6 +77,7 @@ struct pfpb200_ctx {
     bool no_scan_alpha = false;      // PFPB200_NO_SCAN_ALPHA=1: the ranking finds the alphabet of the words itself (A/B)
     bool rank_full_sort = false;     // PFPB200_RANK_FULL_SORT=1: radix-sort all 64 bits of the first key (A/B)
     bool rank_chunk_passes = false;  // PFPB200_RANK_CHUNK_PASSES=1: mid-size tie groups by chunk passes instead of LCP walks (A/B)
+    bool rank_warp_passes = false;   // PFPB200_RANK_WARP_PASSES=1: tie groups of 2..32 words by warp chunk passes instead of LCP walks (A/B)
     bool pool_by_word = false;       // PFPB200_POOL_BY_WORD=1: pool copy with eight lanes per word (A/B)
     bool fuse_k3 = false;          // PFPB200_FUSE_K3=1: K3 + pool fused into the K2 pass (A/B; measured slower, see pfp_stream.cu)
     double pool_ratio = 0.0;       // pool bytes / text bytes of the previous parse (pool sizing hint of the fused K2+K3)

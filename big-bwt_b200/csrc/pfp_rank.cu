@@ -5,10 +5,11 @@
 //
 // The distinct words sit in a pool, each zero-padded to 8-byte words.  Ranking: one global LSD
 // radix sort on an alphabet-compacted first key (21 symbols for DNA), then MSD refinement of the
-// tie groups on 8-byte big-endian chunks -- inside a warp for groups of up to 32 words
-// (rank_window_k / rank_warp_k), in shared memory up to 2048 (rank_mid_k / rank_cta_k:
-// multikey-quicksort passes, one segmented scan per pass), and by further global radix-sort
-// rounds on (tie group, chunk) only for larger groups.  A word's padding is 0x00, below every
+// tie groups on 8-byte big-endian chunks -- by LCP walks along each group's most frequent word,
+// inside a warp for groups of up to 32 (rank_small_lcp_k) and 256 words (rank_lcp_k) and in a
+// CTA up to 2048 (rank_lcp_cta_k), and by further global radix-sort rounds on (tie group, chunk)
+// only for larger groups.  The chunk-pass kernels the walks replaced (rank_window_k / rank_warp_k,
+// rank_mid_k / rank_cta_k) stay as A/B paths and for words of 8 MB and more.  A word's padding is 0x00, below every
 // text byte (> 0x02), so shorter-is-smaller falls out.  Also here: routing of a shard's words to
 // the owners of their lexicographic range (multi-GPU).
 #include "pfp_common.cuh"
@@ -152,8 +153,9 @@ __global__ void groups_compact_k(const u8 *__restrict__ head, const u32 *__restr
     if (i == 0) hp[*nheads] = (u32)d;
 }
 
-// positions in groups larger than LOCAL_MAX go through another global round
-__global__ void rank_active_k(const u8 *__restrict__ head, const u32 *__restrict__ gid,
+// positions in groups larger than LOCAL_MAX go through another global round; the other groups were
+// finished on chip in this round and become singletons
+__global__ void rank_active_k(u8 *__restrict__ head, const u32 *__restrict__ gid,
                               const u32 *__restrict__ hp, u64 d, u8 *__restrict__ act,
                               u8 *__restrict__ gh) {
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
@@ -162,6 +164,7 @@ __global__ void rank_active_k(const u8 *__restrict__ head, const u32 *__restrict
     bool big = (hp[g + 1] - hp[g]) > LOCAL_MAX;
     act[i] = big ? 1 : 0;
     gh[i] = (big && head[i]) ? 1 : 0;
+    if (!big) head[i] = 1;
 }
 
 __global__ void rank_compact_k(const u8 *__restrict__ act, const u8 *__restrict__ gh,
@@ -499,19 +502,21 @@ __device__ __forceinline__ void tie_refine(TieSort<CAP> &S, u64 *sm_v, u32 *sm_f
     else tie_refine_e<NT, CAP, 8>(S, sm_v, sm_f, t, s, m, r0, pool, uoff, uwords, max_chunks, ord, flags);
 }
 
-// lists of the groups for the two shared-memory kernels
+// lists of the groups for the kernels above; warp_list == nullptr: rank_small_lcp_k takes every
+// group of 2..32 words.  counts[3] != 0: some group is larger than LOCAL_MAX (another global round).
 __global__ void rank_lists_k(const u32 *__restrict__ hp, const u32 *__restrict__ nheads, u64 d,
                              u32 *__restrict__ mid_list, u32 *__restrict__ big_list,
                              u32 *__restrict__ warp_list,
-                             u32 *__restrict__ counts /* [0]=mid, [1]=big, [2]=warp */) {
+                             u32 *__restrict__ counts /* [0]=mid, [1]=big, [2]=warp, [3]=global */) {
     u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= d || g >= *nheads) return;
     const u32 s = hp[g], m = hp[g + 1] - s;
     if (m < 2) return;
     if (m <= WARP_MAX) {                      // inside one window of 32 positions: rank_window_k has it
-        if ((s >> 5) != ((s + m - 1) >> 5)) warp_list[atomicAdd(&counts[2], 1u)] = (u32)g;
+        if (warp_list && (s >> 5) != ((s + m - 1) >> 5)) warp_list[atomicAdd(&counts[2], 1u)] = (u32)g;
     } else if (m <= MID_MAX) mid_list[atomicAdd(&counts[0], 1u)] = (u32)g;
     else if (m <= LOCAL_MAX) big_list[atomicAdd(&counts[1], 1u)] = (u32)g;
+    else counts[3] = 1u;
 }
 
 __global__ void __launch_bounds__(256) rank_mid_k(const u32 *__restrict__ hp,
@@ -878,6 +883,171 @@ __global__ void __launch_bounds__(256) rank_lcp_cta_k(const u32 *__restrict__ hp
     }
 }
 
+// ---- LCP walks for the small tie groups (2..32 words), one warp per window of 32 group starts -------------
+// Warp k owns every group of 2..32 words whose first position lies in [32k, 32k + 32): they cover at
+// most the 63 positions [32k, 32k + 63), so a lane holds up to two words (entries e = 0, 1 at
+// positions 32k + 32e + lane; entry id = 32e + lane).  Entries never move: each knows its position
+// inside the warp's span, the range [lo, lo + sz) it is tied in and the chunks dep its range shares.
+// A round is lcp_refine's: the range's most frequent word is the head, every other word walks along
+// it to the first chunk c where they differ (own chunk v), and the range is ordered by
+// (code, v) with code = c below the head, LCP_HEAD for the head, 2 LCP_HEAD - 1 - c above it;
+// equal keys are the ranges of the next round, at depth c + 1.  Families of variants of one
+// consensus phrase are done in one or two rounds, whatever their depth.
+constexpr u32 SMALL_WALK = 4;                 // 16-byte loads per word per memory round trip: 8 chunks
+
+// Walk the word at `mine` (wm chunks) along `head` (wh chunks) from chunk c; returns the first chunk
+// where they differ, with both chunks there (big-endian) in v, h.  Chunks past a word's end are 0.
+// The loads are 16-byte aligned: a block that starts inside a word stays in its 16-byte line.
+__device__ __forceinline__ u32 small_walk(const u64 *mine, u32 wm, const u64 *head, u32 wh, u32 c, u32 max_chunks,
+                                          u64 &v, u64 &h, bool &bad) {
+    constexpr u32 NC = 2 * SMALL_WALK;
+    for (;;) {
+        const u32 sa = (u32)((uintptr_t)(mine + c) >> 3) & 1u, sb = (u32)((uintptr_t)(head + c) >> 3) & 1u;
+        const ulonglong2 *A = reinterpret_cast<const ulonglong2 *>(mine + c - sa);
+        const ulonglong2 *B = reinterpret_cast<const ulonglong2 *>(head + c - sb);
+        u64 a[NC], b[NC];
+#pragma unroll
+        for (u32 i = 0; i < SMALL_WALK; i++) {
+            ulonglong2 x = make_ulonglong2(0ull, 0ull), y = make_ulonglong2(0ull, 0ull);
+            if (c + 2 * i < wm + sa) x = __ldg(A + i);
+            if (c + 2 * i < wh + sb) y = __ldg(B + i);
+            a[2 * i] = x.x; a[2 * i + 1] = x.y;
+            b[2 * i] = y.x; b[2 * i + 1] = y.y;
+        }
+        const u32 n = NC - (sa | sb);                 // chunks c .. c + n - 1 are in a, b
+        bool found = false;
+#pragma unroll
+        for (u32 i = 0; i < NC; i++) {
+            u64 x = (i + 1 < NC && sa) ? a[i + 1] : a[i];
+            u64 y = (i + 1 < NC && sb) ? b[i + 1] : b[i];
+            if (c + i >= wm) x = 0ull;
+            if (c + i >= wh) y = 0ull;
+            if (!found && i < n && x != y) { found = true; v = bswap64(x); h = bswap64(y); c += i; }
+        }
+        if (found) return c;
+        c += n;
+        if (c >= max_chunks) { bad = true; return c; }   // two equal words: cannot happen
+    }
+}
+
+__global__ void __launch_bounds__(256, 4) rank_small_lcp_k(const u32 *__restrict__ hp, const u32 *__restrict__ gid,
+                                                           const u32 *__restrict__ depth, const u64 *__restrict__ pool,
+                                                           const u64 *__restrict__ uoff, const u32 *__restrict__ uwords,
+                                                           const u32 *__restrict__ occ_of_word, u64 d, u32 max_chunks,
+                                                           u32 *__restrict__ ord, u64 *__restrict__ flags) {
+    __shared__ const u64 *s_ptr[8][64];        // per entry id: the word in the pool
+    __shared__ u32 s_wn[8][64];                // ... its length in chunks
+    __shared__ u32 s_uid[8][64];               // ... its id
+    __shared__ u32 s_hkey[8][64];              // ... occurrences << 6 | entry id: the most frequent word heads its range
+    __shared__ u32 s_best[8][64];              // per range start: (occurrences << 6 | entry id) of its head
+    __shared__ u32 s_ka[8][64];                // per position: class/depth code of this round
+    __shared__ u64 s_kb[8][64];                // ... and the chunk where the word left its head
+    const u32 lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+    const u64 nwin = (d + 31) / 32;
+    const u64 nwarps = (u64)gridDim.x * 8;
+    for (u64 k = (u64)blockIdx.x * 8 + wp; k < nwin; k += nwarps) {
+        const u64 w0 = k * 32;
+        // entry 0: a group that starts inside the window; entry 1: the rest of the one group that crosses its end
+        u32 s = 0, m = 0;
+        if (w0 + lane < d) {
+            const u32 g = gid[w0 + lane];
+            s = hp[g];
+            m = hp[g + 1] - s;
+        }
+        const bool in0 = m >= 2 && m <= WARP_MAX && s >= w0;
+        const u32 end31 = __shfl_sync(0xffffffffu, in0 ? s + m : 0u, 31);   // end of the group at position 31
+        const bool in1 = (u64)end31 > w0 + 32 + lane;
+        if (!__any_sync(0xffffffffu, in0)) continue;
+        const u32 s31 = __shfl_sync(0xffffffffu, s, 31), m31 = __shfl_sync(0xffffffffu, m, 31);
+        u32 pos[2], lo[2], sz[2], dep[2];
+#pragma unroll
+        for (u32 e = 0; e < 2; e++) {
+            const bool in = e ? in1 : in0;
+            const u32 gs = e ? s31 : s, gm = e ? m31 : m;
+            pos[e] = 32 * e + lane;
+            s_uid[wp][pos[e]] = in ? ord[w0 + pos[e]] : 0u;
+            lo[e] = in ? (u32)(gs - w0) : pos[e];
+            sz[e] = in ? gm : 1u;
+            dep[e] = in ? depth[gs] : 0u;
+        }
+#pragma unroll
+        for (u32 e = 0; e < 2; e++) {
+            const bool in = sz[e] > 1;
+            const u32 u = s_uid[wp][pos[e]];
+            const u32 c = in ? occ_of_word[u] : 0u;
+            s_hkey[wp][pos[e]] = ((c < (1u << 26) ? c : (1u << 26) - 1) << 6) | pos[e];
+            if (in) {
+                s_ptr[wp][pos[e]] = pool + uoff[u];
+                s_wn[wp][pos[e]] = uwords[u];
+            }
+        }
+        for (;;) {
+            const bool act0 = sz[0] > 1, act1 = sz[1] > 1;
+            if (!__any_sync(0xffffffffu, act0 || act1)) break;
+            // ---- head of every range: its most frequent word ----------------------------------------------
+            if (act0 && pos[0] == lo[0]) s_best[wp][lo[0]] = 0;
+            if (act1 && pos[1] == lo[1]) s_best[wp][lo[1]] = 0;
+            __syncwarp();
+            if (act0) atomicMax(&s_best[wp][lo[0]], s_hkey[wp][lane]);
+            if (act1) atomicMax(&s_best[wp][lo[1]], s_hkey[wp][32 + lane]);
+            __syncwarp();
+            // ---- every other word of the range walks along the head -------------------------------------------
+            // (one call site for both entries: the walk's loads take most of the registers)
+            bool bad = false;
+#pragma unroll 1
+            for (u32 e = 0; e < 2; e++) {
+                const u32 esz = e ? sz[1] : sz[0], elo = e ? lo[1] : lo[0], epos = e ? pos[1] : pos[0];
+                if (esz > 1) {
+                    const u32 hid = s_best[wp][elo] & 63u, me = 32 * e + lane;
+                    u32 code = LCP_HEAD;
+                    u64 v = 0, h = 0;
+                    if (hid != me) {
+                        const u32 c = small_walk(s_ptr[wp][me], s_wn[wp][me], s_ptr[wp][hid], s_wn[wp][hid],
+                                                 e ? dep[1] : dep[0], max_chunks, v, h, bad);
+                        code = v < h ? c : 2u * LCP_HEAD - 1u - c;
+                    }
+                    s_ka[wp][epos] = code;
+                    s_kb[wp][epos] = v;
+                }
+            }
+            if (__any_sync(0xffffffffu, bad)) {
+                if (lane == 0) atomicOr((unsigned long long *)&flags[0], PFP_ERRBIT_INTERNAL);
+                break;
+            }
+            __syncwarp();
+            // ---- place every word among the words of its range; equal keys tie in the next round -------------
+            u32 nlo[2], nsz[2], npos[2];
+#pragma unroll
+            for (u32 e = 0; e < 2; e++) {
+                nlo[e] = lo[e]; nsz[e] = sz[e]; npos[e] = pos[e];
+                if (sz[e] > 1) {
+                    const u32 code = s_ka[wp][pos[e]];
+                    const u64 kv = s_kb[wp][pos[e]];
+                    u32 less = 0, eq = 0, eq_before = 0;
+                    for (u32 q = lo[e]; q < lo[e] + sz[e]; q++) {
+                        const u32 a1 = s_ka[wp][q];
+                        const u64 b1 = s_kb[wp][q];
+                        const bool same = a1 == code && b1 == kv;
+                        less += lcp_less(a1, b1, code, kv) ? 1u : 0u;
+                        eq += same ? 1u : 0u;
+                        eq_before += (same && q < pos[e]) ? 1u : 0u;
+                    }
+                    nlo[e] = lo[e] + less;
+                    nsz[e] = eq;
+                    npos[e] = nlo[e] + eq_before;
+                    if (code != LCP_HEAD) dep[e] = (code < LCP_HEAD ? code : 2u * LCP_HEAD - 1u - code) + 1;
+                }
+            }
+            __syncwarp();
+#pragma unroll
+            for (u32 e = 0; e < 2; e++) { lo[e] = nlo[e]; sz[e] = nsz[e]; pos[e] = npos[e]; }
+        }
+        if (in0) ord[w0 + pos[0]] = s_uid[wp][lane];
+        if (in1) ord[w0 + pos[1]] = s_uid[wp][32 + lane];
+        __syncwarp();
+    }
+}
+
 __global__ void __launch_bounds__(256) rank_cta_k(const u32 *__restrict__ hp,
                                                   const u32 *__restrict__ list,
                                                   const u32 *__restrict__ count,
@@ -964,6 +1134,9 @@ int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bo
     u8 *act = nullptr, *gh = nullptr;
     u32 *ascan = nullptr, *gscan = nullptr, *apos = nullptr, *gid_of_u = nullptr, *depth2 = nullptr;
     u32 *d_nheads = reinterpret_cast<u32 *>(&ctx->d_flags[4]);
+    // A/B (and words of 8 MB and more): the kernels the LCP walks replaced, one 8-byte chunk per pass
+    const bool chunk_passes = ctx->rank_chunk_passes || max_chunks >= LCP_MAX_CHUNKS;
+    const bool warp_passes = ctx->rank_warp_passes || max_chunks >= LCP_MAX_CHUNKS;
     u32 r = 1;
     bool big_bufs = false;
     for (;; r++) {
@@ -973,6 +1146,51 @@ int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bo
         groups_compact_k<<<nbd, TB, 0, ctx->stream>>>(head, hscan, d, d_nheads, hp, gid);
         PFP_LAUNCHED(ctx);
         if (d < 2) break;
+        // finish every tie group of up to LOCAL_MAX words on chip; the larger ones (none, unless a
+        // family has thousands of members) go through a global round and come back here split
+        u32 *mid_list = v1, *big_list = v0;      // sort buffers are free until the global round
+        u32 *counts = reinterpret_cast<u32 *>(&ctx->d_flags[5]);
+        PFP_CUDA(ctx, cudaMemsetAsync(counts, 0, 4 * sizeof(u32), ctx->stream));
+        rank_lists_k<<<nbd, TB, 0, ctx->stream>>>(hp, d_nheads, d, mid_list, big_list,
+                                                  warp_passes ? reinterpret_cast<u32 *>(k1) : nullptr, counts);
+        PFP_LAUNCHED(ctx);
+        u64 want = (d / 2 + 7) / 8;
+        u64 maxb = (u64)ctx->sm_count * 16;
+        u32 nbw = (u32)(want < maxb ? want : maxb);
+        if (nbw == 0) nbw = 1;
+        if (warp_passes) {
+            rank_window_k<<<nbw, 256, 0, ctx->stream>>>(hp, gid, depth, D.pool, D.uoff, D.uwords, d, max_chunks, 0,
+                                                        ord, ctx->d_flags);
+            PFP_LAUNCHED(ctx);
+            // (a second pass over windows shifted by 16 for the groups straddling a border was measured:
+            //  it costs what it saves -- the kernels are bound by their chains of dependent loads)
+            rank_warp_k<<<nbw, 256, 0, ctx->stream>>>(hp, reinterpret_cast<u32 *>(k1), counts + 2, depth, D.pool,
+                                                      D.uoff, D.uwords, max_chunks, ord, ctx->d_flags);
+        } else {
+            rank_small_lcp_k<<<nbw, 256, 0, ctx->stream>>>(hp, gid, depth, D.pool, D.uoff, D.uwords, D.count, d,
+                                                           max_chunks, ord, ctx->d_flags);
+        }
+        PFP_LAUNCHED(ctx);
+        if (chunk_passes)
+            rank_mid_k<<<ctx->sm_count * 4, 256, 8 * sizeof(TieSort<MID_MAX>), ctx->stream>>>(
+                hp, mid_list, counts, depth, D.pool, D.uoff, D.uwords, max_chunks, ord, ctx->d_flags);
+        else
+            rank_lcp_k<<<ctx->sm_count * 6, 256, 8 * sizeof(LcpSort<LCP_MAX>), ctx->stream>>>(
+                hp, mid_list, counts, depth, D.pool, D.uoff, D.uwords, D.count, max_chunks, ord, ctx->d_flags);
+        PFP_LAUNCHED(ctx);
+        if (chunk_passes)
+            rank_cta_k<<<ctx->sm_count * 4, 256, sizeof(TieSort<LOCAL_MAX>), ctx->stream>>>(
+                hp, big_list, counts + 1, depth, D.pool, D.uoff, D.uwords, max_chunks, ord, ctx->d_flags);
+        else
+            rank_lcp_cta_k<<<ctx->sm_count * 3, 256, sizeof(LcpSort<LOCAL_MAX>), ctx->stream>>>(
+                hp, big_list, counts + 1, depth, D.pool, D.uoff, D.uwords, D.count, max_chunks, ord, ctx->d_flags);
+        PFP_LAUNCHED(ctx);
+        PFP_CUDA(ctx, cudaMemcpyAsync(ctx->h_flags, ctx->d_flags, 7 * sizeof(u64), cudaMemcpyDeviceToHost,
+                                      ctx->stream));
+        PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        if (ctx->h_flags[0] & PFP_ERRBIT_INTERNAL)
+            return pfp_fail(ctx, PFPB200_E_INTERNAL, "ranking found words that never differ (duplicates?)");
+        if (reinterpret_cast<const u32 *>(&ctx->h_flags[5])[3] == 0) break;
         if (!big_bufs) {
             PFP_TRY(pfp_alloc_t(ctx, &act, d));
             PFP_TRY(pfp_alloc_t(ctx, &gh, d));
@@ -988,7 +1206,6 @@ int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bo
                                       cudaMemcpyDeviceToHost, ctx->stream));
         PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         u64 m = (u32)ctx->h_flags[1], ng = (u32)ctx->h_flags[2];
-        if (m == 0) break;
         if (r > max_chunks + 1)
             return pfp_fail(ctx, PFPB200_E_INTERNAL,
                             "ranking did not separate %llu words after %u rounds (duplicate words?)",
@@ -1018,48 +1235,6 @@ int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bo
                                                       D.uwords, ord, head, depth2);
         PFP_LAUNCHED(ctx);
         u32 *tdp = depth; depth = depth2; depth2 = tdp;
-    }
-    // finish every remaining tie group on chip
-    if (d >= 2) {
-        u32 *mid_list = v1, *big_list = v0;      // sort buffers are free again
-        u32 *warp_list = reinterpret_cast<u32 *>(k1);
-        u32 *counts = reinterpret_cast<u32 *>(&ctx->d_flags[5]);
-        PFP_CUDA(ctx, cudaMemsetAsync(counts, 0, 4 * sizeof(u32), ctx->stream));
-        rank_lists_k<<<nbd, TB, 0, ctx->stream>>>(hp, d_nheads, d, mid_list, big_list, warp_list, counts);
-        PFP_LAUNCHED(ctx);
-        u64 want = (d / 2 + 7) / 8;
-        u64 maxb = (u64)ctx->sm_count * 16;
-        u32 nbw = (u32)(want < maxb ? want : maxb);
-        if (nbw == 0) nbw = 1;
-        rank_window_k<<<nbw, 256, 0, ctx->stream>>>(hp, gid, depth, D.pool, D.uoff, D.uwords, d, max_chunks, 0, ord,
-                                                    ctx->d_flags);
-        PFP_LAUNCHED(ctx);
-        // (a second pass over windows shifted by 16 for the groups straddling a border was measured:
-        //  it costs what it saves -- the kernels are bound by their chains of dependent loads)
-        rank_warp_k<<<nbw, 256, 0, ctx->stream>>>(hp, warp_list, counts + 2, depth, D.pool, D.uoff, D.uwords, max_chunks,
-                                                  ord, ctx->d_flags);
-        PFP_LAUNCHED(ctx);
-        // A/B (and words of 8 MB and more): one 8-byte chunk per pass, the kernels the LCP walks replaced
-        const bool chunk_passes = ctx->rank_chunk_passes || max_chunks >= LCP_MAX_CHUNKS;
-        if (chunk_passes)
-            rank_mid_k<<<ctx->sm_count * 4, 256, 8 * sizeof(TieSort<MID_MAX>), ctx->stream>>>(
-                hp, mid_list, counts, depth, D.pool, D.uoff, D.uwords, max_chunks, ord, ctx->d_flags);
-        else
-            rank_lcp_k<<<ctx->sm_count * 6, 256, 8 * sizeof(LcpSort<LCP_MAX>), ctx->stream>>>(
-                hp, mid_list, counts, depth, D.pool, D.uoff, D.uwords, D.count, max_chunks, ord, ctx->d_flags);
-        PFP_LAUNCHED(ctx);
-        if (chunk_passes)
-            rank_cta_k<<<ctx->sm_count * 4, 256, sizeof(TieSort<LOCAL_MAX>), ctx->stream>>>(
-                hp, big_list, counts + 1, depth, D.pool, D.uoff, D.uwords, max_chunks, ord, ctx->d_flags);
-        else
-            rank_lcp_cta_k<<<ctx->sm_count * 3, 256, sizeof(LcpSort<LOCAL_MAX>), ctx->stream>>>(
-                hp, big_list, counts + 1, depth, D.pool, D.uoff, D.uwords, D.count, max_chunks, ord, ctx->d_flags);
-        PFP_LAUNCHED(ctx);
-        PFP_CUDA(ctx, cudaMemcpyAsync(ctx->h_flags, ctx->d_flags, sizeof(u64), cudaMemcpyDeviceToHost,
-                                      ctx->stream));
-        PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (ctx->h_flags[0] & PFP_ERRBIT_INTERNAL)
-            return pfp_fail(ctx, PFPB200_E_INTERNAL, "ranking found words that never differ (duplicates?)");
     }
     *rounds = r;
     *order = ord;
