@@ -296,7 +296,10 @@ static int parse_device_impl(pfpb200_ctx *ctx, const u8 *d_text, u64 n, const pf
             PFP_TRY(pfp_free_now(ctx, ph.rec));
             PFP_TRY(pfp_pool_stage(ctx, tv, ends, -1, w, &D));
         }
-        if (o->flags & PFPB200_F_VERIFY) PFP_TRY(pfp_verify_stage(ctx, tv, ends, -1, w, P, D));
+        if (o->flags & PFPB200_F_VERIFY) {
+            PFP_TRY(pfp_uid_words(ctx, &D, P));
+            PFP_TRY(pfp_verify_stage(ctx, tv, ends, -1, w, P, D));
+        }
         tm.mark(ctx->stream);                                           // 3
         // K4
         u32 *order = nullptr, rounds = 0;
@@ -763,6 +766,7 @@ extern "C" int pfpb200_shard_words(pfpb200_ctx *ctx, int64_t first_start, pfpb20
             if (stream) PFP_TRY(pfp_stream_stage(ctx, ctx->sh.bits, tv, ph, P, first_start, w, !ctx->sh.ends_emitted));
             else PFP_TRY(pfp_hash_stage(ctx, tv, ph, P, first_start, w));
             PFP_TRY(pfp_dedup_stage(ctx, ph, P, first_start, w, &D));
+            PFP_TRY(pfp_uid_words(ctx, &D, P));
         }
         u64 *wfpa = nullptr, *wfpb = nullptr;
         PFP_TRY(pfp_alloc_t(ctx, &wfpa, D.d));

@@ -41,11 +41,19 @@ struct PhraseArrays {
 // these fields of every word anyway)
 struct __align__(16) WordMeta { u64 off; u32 len; u32 count; };
 
+constexpr u32 UID_CREATOR = 0x80000000u;   // uid[j] with slot_of_word: marks the word id held by the word's creator
+
 struct DictArrays {
     u64 d = 0;
     WordMeta *meta = nullptr;   // [d] filled by pfp_rank_stage
     u32 *uid = nullptr;     // [P] phrase -> uid
-    u32 *rep = nullptr;     // [d] first phrase index of the word
+    u32 *slot_of_word = nullptr;   // [d] non-null: uid[j] is word id | UID_CREATOR on the record that
+                                   // created a word (won its table slot), and the word's slot in a
+                                   // table of `slots` entries on the others; word u lives in slot
+                                   // slot_of_word[u] (pfp_dedup_stage; pfp_uid_words makes every
+                                   // uid[j] a word id)
+    u64 slots = 0;
+    u32 *rep = nullptr;     // [d] index of the phrase that created the word (won its table slot)
     i64 *ustart = nullptr;  // [d] global text position of that phrase's first byte (may be -1: virtual border)
     u32 *count = nullptr;   // [d] occurrences
     u32 *ulen = nullptr;    // [d] length in bytes
@@ -91,6 +99,7 @@ bool pfp_stream_ok(const ScanBits &sb, u32 w);   // false: w > 32 or a tile too 
 int pfp_stream_stage(pfpb200_ctx *ctx, const ScanBits &sb, const TextView &tv, const PhraseArrays &ph,
                      u64 P, i64 first_start, u32 w, bool emit_ends);
 int pfp_dedup_stage(pfpb200_ctx *ctx, const PhraseArrays &ph, u64 P, i64 first_start, u32 w, DictArrays *D);
+int pfp_uid_words(pfpb200_ctx *ctx, DictArrays *D, u64 n);   // uid[0..n) -> word ids, if D->slot_of_word is set
 int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 first_start, u32 w,
                    DictArrays *D);
 // Lexicographic order of the d pool words: order[i] = uid of the word of rank i+1.

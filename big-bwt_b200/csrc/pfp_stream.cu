@@ -106,9 +106,9 @@ __device__ __forceinline__ void fused_insert(const StreamArgs &a, u64 j, u32 q, 
         cq[i] = (u16)q;
         cs[i] = (u32)pr.slot;
         if (a.rec) store_rec(a.rec, j, pa, pb);          // sharded parsing exports the words' fingerprints
-    } else if (pr.seen_uid1) {
-        __stcs(a.uid + j, pr.seen_uid1 - 1);
-        atomicAdd(&a.count[pr.seen_uid1 - 1], 1u);
+    } else if (pr.seen_val) {
+        __stcs(a.uid + j, pr.seen_val - 1);
+        atomicAdd(&a.count[pr.seen_val - 1], 1u);
     } else {                                            // its creator has not stored the id yet: table_pending_k
         __stcs(a.uid + j, UID_PENDING | (u32)pr.slot);
         atomicOr((unsigned long long *)&a.flags[6], 1ull);
@@ -409,7 +409,7 @@ __global__ void __launch_bounds__(K2_T, 4) phrase_stream_k(const StreamArgs a) {
             a.ulen[u] = my_len[r];
             a.uwords[u] = (my_len[r] + 7) >> 3;
             a.uoff[u] = base_pool + my_off[r];
-            a.tab[cs[k]].uid1 = u + 1;
+            a.tab[cs[k]].val = u + 1;
             __stcs(a.uid + j, u);
             atomicAdd(&a.count[u], 1u);
             cs[k] = my_off[r];                                      // the slot is no longer needed

@@ -5,14 +5,16 @@
 #include "pfp_stages.cuh"
 #include "pfp_fp.cuh"
 
-// Open addressing, linear probing, 16-byte slots {key, occurrences, check}; key 0 = empty.
+// Open addressing, linear probing, 16-byte slots {key, val, check}; key 0 = empty.
 // A warp first groups its lanes by key (match.any) so that runs of identical phrases cost one
 // atomic per warp instead of 32.  `chk` is a 32-bit digest of the full 128-bit fingerprint and
 // the length, independent of the key: every phrase that lands in a slot must agree with it, or
 // the parse stops with PFPB200_E_COLLISION (the reference compares strings, newscan.cpp:282-286).
-struct __align__(16) DictSlot { u64 key; u32 uid1; u32 chk; };   // uid1 = word id + 1; 0 until its creator stored it
+// `val` is the word's occurrence count in table_insert_k, and word id + 1 in the fused K2 pass
+// (0 until its creator stored it).
+struct __align__(16) DictSlot { u64 key; u32 val; u32 chk; };
 constexpr u32 TABLE_MAX_PROBES = 2048;
-constexpr u32 UID_PENDING = 0x80000000u;       // uid[j] = UID_PENDING | slot: resolved by table_pending_k
+constexpr u32 UID_PENDING = 0x80000000u;       // fused K2 pass: uid[j] = UID_PENDING | slot, resolved by table_pending_k
 
 __device__ __forceinline__ u32 check_of(const PhraseFp &r) {
     u64 x = (r.fpa + 0x632BE59BD9B4E019ULL) * 0xD1342543DE82EF95ULL;
@@ -25,19 +27,19 @@ __device__ __forceinline__ u32 check_of(const PhraseFp &r) {
 int pfp_table_init(pfpb200_ctx *ctx, DictSlot *tab, u64 cap);     // all slots empty (pfp_phrase.cu)
 
 // One probe sequence: a plain 16-byte load of the slot first -- on repetitive inputs nine phrases
-// in ten find their word already there, read its id from the slot and finish with one
-// fire-and-forget add to its count -- and a CAS only on an empty slot.  The thread that wins the
-// CAS is the word's creator: it draws the next word id from a counter (ids are dense, in creation
-// order: no flag / scan / compaction passes over the table afterwards), stores it in the slot and
-// records itself as the word's representative occurrence.
-struct Probe { u64 slot; bool placed; bool creator; u32 seen_chk; u32 seen_uid1; };
+// in ten find their word already there and finish with one fire-and-forget add to its count --
+// and a CAS only on an empty slot.  The thread that wins the CAS is the word's creator.  Word ids
+// are not handed out here: table_insert_k leaves the slot in uid[] with a creator bit, and
+// table_compact_k numbers the words afterwards, in the order of their creators' records (one scan
+// over the records, no counter that every creator has to wait for).
+struct Probe { u64 slot; bool placed; bool creator; u32 seen_chk; u32 seen_val; };
 
 __device__ __forceinline__ Probe table_probe(DictSlot *__restrict__ tab, u64 cap, u64 slot, uint4 sv, u64 k) {
     Probe r{slot, false, false, 0u, 0u};
     u32 probes = 0;
     for (;;) {
         const u64 key = ((u64)sv.y << 32) | sv.x;
-        if (key == k) { r.placed = true; r.seen_uid1 = sv.z; r.seen_chk = sv.w; break; }
+        if (key == k) { r.placed = true; r.seen_val = sv.z; r.seen_chk = sv.w; break; }
         if (key == 0ull) {
             const u64 prev = atomicCAS((unsigned long long *)&tab[r.slot].key, 0ull, (unsigned long long)k);
             if (prev == 0ull) { r.placed = true; r.creator = true; break; }
