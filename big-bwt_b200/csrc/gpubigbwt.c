@@ -22,14 +22,83 @@ static void usage(const char *exe) {
     printf("\t-S  \tcompute the full suffix array (.sa)\n");
     printf("\t-k  \tkeep the intermediate files of the three stages\n");
     printf("\t-t T\taccepted for compatibility (helper threads of the reference's stages)\n");
-    printf("\t-g G\tCUDA device index, def. 0\n");
+    printf("\t-g G\tCUDA device index, def. 0, or a comma-separated list (e.g. 0,1,2,3): parse and pfbwt\n"
+           "\t    \tsharded over those GPUs, bwtparse on the first, through files\n");
     exit(1);
+}
+
+static double since(const struct timespec *t0) {
+    struct timespec t1;
+    clock_gettime(CLOCK_MONOTONIC, &t1);
+    return (double)(t1.tv_sec - t0->tv_sec) + 1e-9 * (double)(t1.tv_nsec - t0->tv_nsec);
+}
+
+/* the three stages through files, as bigbwt runs them: newscan -> bwtparse -> pfbwt; the parse and
+ * pfbwt on all listed GPUs, bwtparse (about a tenth of the parse's size) on the first one */
+static int multi_bigbwt(const char *path, const pfpb200_opts *opts, unsigned flags, int keep, const int *devices,
+                        int n_dev, const struct timespec *t0) {
+    static const char *inter[] = {"dict", "occ", "parse", "last", "sai", "ilist", "bwlast", "bwsai"};
+    pfpb200_opts o = *opts;
+    o.flags |= PFPB200_F_SAI;                     /* the later stages take .sai whenever a suffix array is wanted */
+    pfpb200_multi *multi = NULL;
+    pfpb200_ctx *ctx = NULL;
+    pfpb200_stats st;
+    pfpb200_bwtparse_result bp;
+    pfpb200_pfbwt_result r;
+    int rc = pfpb200_multi_create(n_dev, devices, &multi);
+    if (rc != PFPB200_OK) {
+        fprintf(stderr, "gpubigbwt: cannot use the %d listed CUDA devices: %s\n", n_dev, pfpb200_strerror(rc));
+        return 1;
+    }
+    const char *stage = "parse";
+    rc = pfpb200_multi_parse_file(multi, path, &o, &st);
+    if (rc == PFPB200_OK) {
+        stage = "bwtparse";
+        rc = pfpb200_create(devices[0], &ctx);
+        if (rc == PFPB200_OK) rc = pfpb200_bwtparse_file(ctx, path, 1, 0, &bp);
+        if (rc == PFPB200_OK) {
+            pfpb200_destroy(ctx);                 /* its HBM goes back before the last stage */
+            ctx = NULL;
+            stage = "pfbwt";
+            rc = pfpb200_multi_pfbwt_file(multi, path, o.w, flags, &r);
+        }
+    }
+    if (rc != PFPB200_OK) {
+        fprintf(stderr, "gpubigbwt: %s: %s: %s\n", stage, pfpb200_strerror(rc),
+                ctx ? pfpb200_last_error(ctx) : pfpb200_multi_last_error(multi));
+    } else {
+        printf("Total input symbols: %llu\n", (unsigned long long)st.n_text);
+        printf("Found %llu distinct words\n", (unsigned long long)st.n_distinct);
+        printf("Total number of words: %llu\n", (unsigned long long)st.n_phrases);
+        printf("Easy bwt chars: %llu\n", (unsigned long long)r.easy);
+        printf("Hard bwt chars: %llu\n", (unsigned long long)r.hard);
+        printf("GPU: parse %.3f ms, bwtparse %.3f ms (%u rounds), pfbwt %.3f ms (suffix sort %.3f in %u rounds, BWT%s %.3f)\n",
+               st.ms_total, bp.ms_total, bp.rounds, r.ms_total, r.ms_sa, r.rounds, flags ? " + SA" : "", r.ms_fill);
+        pfpb200_pfbwt_rank pr[PFPB200_MAX_RANKS];
+        int k = pfpb200_multi_pfbwt_ranks(multi, pr, PFPB200_MAX_RANKS);
+        for (int g = 0; g < k; g++)
+            printf("GPU %d (rank %d): pfbwt %llu suffixes, %llu chars, sort %.3f ms, emit %.3f ms, write %.3f ms\n",
+                   devices[g], g, (unsigned long long)pr[g].suffixes, (unsigned long long)pr[g].chars, pr[g].ms_sort,
+                   pr[g].ms_emit, pr[g].ms_write);
+    }
+    if (!keep) {
+        char name[4096];
+        for (size_t i = 0; i < sizeof(inter) / sizeof(inter[0]); i++) {
+            snprintf(name, sizeof(name), "%s.%s", path, inter[i]);
+            unlink(name);
+        }
+    }
+    pfpb200_destroy(ctx);
+    pfpb200_multi_destroy(multi);
+    if (rc != PFPB200_OK) return 1;
+    printf("==== Elapsed time: %.3f wall clock seconds\n", since(t0));
+    return 0;
 }
 
 int main(int argc, char **argv) {
     pfpb200_opts o = {10, 100, 0, 0};
     long w = 10, p = 100;
-    int c, device = 0, keep = 0;
+    int c, keep = 0, devices[PFPB200_MAX_RANKS] = {0}, n_dev = 1;
     unsigned flags = 0;
     struct timespec t0, t1;
     clock_gettime(CLOCK_MONOTONIC, &t0);
@@ -47,7 +116,13 @@ int main(int argc, char **argv) {
             case 'k': keep = 1; break;
             case 't': break;                       /* bigbwt -t T: helper threads of the CPU stages, nothing to do here */
             case 'v': break;
-            case 'g': device = atoi(optarg); break;
+            case 'g': {
+                n_dev = 0;
+                for (char *tok = strtok(optarg, ","); tok && n_dev < PFPB200_MAX_RANKS; tok = strtok(NULL, ","))
+                    devices[n_dev++] = atoi(tok);
+                if (n_dev == 0) { puts("Invalid device list"); exit(1); }
+                break;
+            }
             case 'h': usage(argv[0]); break;
             default: puts("Unknown option. Use -h for help."); exit(1);
         }
@@ -61,10 +136,11 @@ int main(int argc, char **argv) {
     }
     if (w > 65536 || p > 0x7FFFFFFFL) { puts("Option value too large"); exit(1); }
     o.w = (uint32_t)w; o.p = (uint32_t)p;
+    if (n_dev > 1) return multi_bigbwt(argv[optind], &o, flags, keep, devices, n_dev, &t0);
     pfpb200_ctx *ctx = NULL;
-    int rc = pfpb200_create(device, &ctx);
+    int rc = pfpb200_create(devices[0], &ctx);
     if (rc != PFPB200_OK) {
-        fprintf(stderr, "gpubigbwt: cannot use CUDA device %d: %s\n", device, pfpb200_strerror(rc));
+        fprintf(stderr, "gpubigbwt: cannot use CUDA device %d: %s\n", devices[0], pfpb200_strerror(rc));
         return 1;
     }
     pfpb200_stats st;

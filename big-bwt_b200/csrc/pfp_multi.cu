@@ -54,11 +54,28 @@ struct Barrier {
     std::condition_variable cv;
     int n = 1, count = 0;
     unsigned gen = 0;
+    u64 acc = 0, result = 0;
+    int fails = 0, fails_result = 0;
     void wait() {
         std::unique_lock<std::mutex> l(mu);
         const unsigned g = gen;
         if (++count == n) { count = 0; gen++; cv.notify_all(); }
         else cv.wait(l, [&] { return gen != g; });
+    }
+    // a barrier that returns the sum of what every thread brought and whether any thread brought a
+    // failure: the same values for all of them
+    u64 sum(u64 v, bool failed, bool *any_failed) {
+        std::unique_lock<std::mutex> l(mu);
+        const unsigned g = gen;
+        acc += v;
+        fails += failed ? 1 : 0;
+        if (++count == n) {
+            result = acc; fails_result = fails;
+            acc = 0; fails = 0; count = 0; gen++;
+            cv.notify_all();
+        } else cv.wait(l, [&] { return gen != g; });
+        *any_failed = fails_result != 0;
+        return result;
     }
 };
 
@@ -91,6 +108,13 @@ struct Rank {
     const u32 *d_parse = nullptr;
     float ms_phase[PH_COUNT] = {0};
     u32 launches = 0;
+    // the sharded pfbwt (pfpb200_multi_pfbwt_file); published fields are read by the peers between barriers
+    PmState pb;
+    const void *pb_in[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // .dict .occ .ilist .bwlast .bwsai
+    u64 pb_n[5] = {0, 0, 0, 0, 0};
+    u64 *pb_rank = nullptr;               // my block of the rank array
+    pfpb200_pfbwt_rank pb_stat;
+    u32 pb_rounds = 0;
 };
 
 }  // namespace
@@ -121,6 +145,11 @@ struct pfpb200_multi {
     double sec_wall = 0;
     // PFPB200_MULTI_MIN_SHARD / PFPB200_MULTI_FRONT (tests): seams and front growth on small inputs
     u64 min_shard = MULTI_MIN_SHARD, front_cap = MULTI_FRONT;
+    // the current pfbwt job; PFPB200_MULTI_SPLIT_KEY=1 (tests): the two-sort key form of the
+    // sharded suffix sort even where one 64-bit key would do
+    const char *pb_base = nullptr;
+    u32 pb_w = 0, pb_flags = 0;
+    bool split_key = false;
 };
 
 namespace {
@@ -596,6 +625,7 @@ extern "C" int pfpb200_multi_create(int n_gpus, const int *gpu_ids, pfpb200_mult
     m->n = n_gpus;
     { const char *ev = getenv("PFPB200_MULTI_MIN_SHARD"); if (ev && atoll(ev) > 0) m->min_shard = (u64)atoll(ev); }
     { const char *ev = getenv("PFPB200_MULTI_FRONT"); if (ev && atoll(ev) >= 0) m->front_cap = (u64)atoll(ev); }
+    { const char *ev = getenv("PFPB200_MULTI_SPLIT_KEY"); m->split_key = ev && atoi(ev) != 0; }
     m->r.resize(n_gpus);
     m->bar.n = n_gpus;
     int rc = PFPB200_OK;
@@ -829,4 +859,302 @@ extern "C" int pfpb200_multi_parse_file(pfpb200_multi *m, const char *path, cons
         stats->sec_write = stats->ms_d2h * 1e-3f;       // the writes are the ranks' last phase
     }
     return PFPB200_OK;
+}
+
+// ---- the sharded pfbwt: pfpb200_multi_pfbwt_file ----------------------------------------------------------
+// One host thread per rank runs pfbwt_rank_main.  Every decision that changes the sequence of barriers
+// is taken on a value all ranks agree on (Barrier::sum), so a rank that fails keeps passing the same
+// barriers as the others; nobody frees memory a peer may still read before the last barrier.
+namespace {
+
+const char *const PB_EXT[5] = {"dict", "occ", "ilist", "bwlast", "bwsai"};
+const u64 PB_UNIT[5] = {1, 4, 4, 1, PFP_IBYTES};
+
+int pb_read_input(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count) {
+    char name[4096];
+    snprintf(name, sizeof(name), "%s.%s", base, PB_EXT[k]);
+    const int fd = open(name, O_RDONLY);
+    if (fd < 0) return pfp_fail(ctx, PFPB200_E_IO, "cannot open %s: %s", name, strerror(errno));
+    struct stat st;
+    if (fstat(fd, &st) != 0) { close(fd); return pfp_fail(ctx, PFPB200_E_IO, "cannot stat %s", name); }
+    const u64 bytes = (u64)st.st_size;
+    if (bytes % PB_UNIT[k] != 0) { close(fd); return pfp_fail(ctx, PFPB200_E_ARG, "invalid %s file", PB_EXT[k]); }
+    int rc = pfp_alloc(ctx, d, bytes, true);
+    if (rc == PFPB200_OK && bytes) rc = pfp_file_to_device(ctx, fd, 0, bytes, static_cast<u8 *>(*d));
+    close(fd);
+    *count = bytes / PB_UNIT[k];
+    return rc;
+}
+
+// rank 0: the input files into HBM, checked as pfpb200_pfbwt_file checks them
+int pb_inputs_rank0(pfpb200_multi *m, Rank &R) {
+    const bool want_sa = (m->pb_flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
+    void *p[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    for (int k = 0; k < 4; k++) PFP_TRY(pb_read_input(R.ctx, m->pb_base, k, &p[k], &R.pb_n[k]));
+    if (R.pb_n[3] != R.pb_n[2])
+        return pfp_fail(R.ctx, PFPB200_E_ARG, ".bwlast holds %llu bytes, .ilist %llu entries",
+                        (unsigned long long)R.pb_n[3], (unsigned long long)R.pb_n[2]);
+    if (want_sa) {
+        PFP_TRY(pb_read_input(R.ctx, m->pb_base, 4, &p[4], &R.pb_n[4]));
+        if (R.pb_n[4] != R.pb_n[2]) return pfp_fail(R.ctx, PFPB200_E_ARG, "bwsa info read");
+    }
+    const u64 N = R.pb_n[0], psize = R.pb_n[2];
+    if (N <= 1 + (u64)m->pb_w) return pfp_fail(R.ctx, PFPB200_E_ARG, "invalid dictionary file");
+    if (psize >= 0xFFFFFFFEull)
+        return pfp_fail(R.ctx, PFPB200_E_LIMIT, "more than 2^32-2 words in the parsing (.ilist is 32-bit)");
+    for (int k = 0; k < 5; k++) R.pb_in[k] = p[k];
+    return PFPB200_OK;
+}
+
+// the other ranks: rank 0's buffers when they share its device, otherwise copies peer to peer
+int pb_inputs_peer(pfpb200_multi *m, Rank &R) {
+    const Rank &R0 = m->r[0];
+    for (int k = 0; k < 5; k++) {
+        R.pb_n[k] = R0.pb_n[k];
+        R.pb_in[k] = R0.pb_in[k];
+        if (R.device == R0.device || !R0.pb_in[k]) continue;
+        const u64 bytes = R0.pb_n[k] * PB_UNIT[k];
+        void *d = nullptr;
+        PFP_TRY(pfp_alloc(R.ctx, &d, bytes, true));
+        if (bytes) PFP_CUDA(R.ctx, cudaMemcpyPeerAsync(d, R.device, R0.pb_in[k], R0.device, (size_t)bytes, R.ctx->stream));
+        R.pb_in[k] = d;
+    }
+    PFP_CUDA(R.ctx, cudaStreamSynchronize(R.ctx->stream));
+    return PFPB200_OK;
+}
+
+void pfbwt_rank_main(pfpb200_multi *m, int g) {
+    Rank &R = m->r[g];
+    const int G = m->n;
+    pfpb200_ctx *ctx = R.ctx;
+    PmState &S = R.pb;
+    cudaSetDevice(R.device);
+    auto ok = [&]() { return m->failed.load() == 0; };
+    auto agree = [&]() { bool f; m->bar.sum(0, !ok(), &f); return !f; };    // a barrier: true when no rank has failed
+    auto run = [&](int rc) { if (rc != PFPB200_OK) multi_fail(m, g, rc, pfpb200_last_error(ctx)); };
+    const double t0 = wall_sec();
+    double t_read = t0, t_sort = t0, t_emit = t0, t_write = t0;
+    const u32 launches0 = ctx->launches;
+    memset(&R.pb_stat, 0, sizeof(R.pb_stat));
+    R.pb_rounds = 0;
+    R.pb_rank = nullptr;
+    S = PmState();
+    pfp_release_scratch(ctx);
+    pfp_release_held(ctx);
+    ctx->arena.peak = ctx->arena.in_use;                    // the peak reported is this call's
+    // the shard and exchange buffers of an earlier parse go back to the driver (a parse grows them again)
+    if (R.buf) { cudaFree(R.buf); R.buf = nullptr; R.buf_cap = 0; }
+    if (R.rx_words) { cudaFree(R.rx_words); R.rx_words = nullptr; R.rx_words_cap = 0; }
+    if (R.rx_pool) { cudaFree(R.rx_pool); R.rx_pool = nullptr; R.rx_pool_cap = 0; }
+    if (R.rx_ranks) { cudaFree(R.rx_ranks); R.rx_ranks = nullptr; R.rx_ranks_cap = 0; }
+    ctx->err[0] = 0;
+    cudaMemsetAsync(ctx->d_flags, 0, 12 * sizeof(u64), ctx->stream);
+    const bool want_sa = (m->pb_flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
+    do {
+        // ---- 1. inputs: read once by rank 0, to the other GPUs peer to peer ---------------------------------
+        for (int k = 0; k < 5; k++) { R.pb_in[k] = nullptr; R.pb_n[k] = 0; }
+        if (g == 0) run(pb_inputs_rank0(m, R));
+        if (!agree()) break;
+        if (g > 0) run(pb_inputs_peer(m, R));
+        S.d = (const u8 *)R.pb_in[0]; S.N = R.pb_n[0];
+        S.occ = (const u32 *)R.pb_in[1]; S.dwords = R.pb_n[1];
+        S.ilist = (const u32 *)R.pb_in[2]; S.psize = R.pb_n[2];
+        S.bwlast = (const u8 *)R.pb_in[3];
+        S.bwsai = want_sa ? (const u8 *)R.pb_in[4] : nullptr;
+        S.w = m->pb_w; S.flags = m->pb_flags;
+        if (ok()) run(pm_words(ctx, S));
+        t_read = wall_sec();
+        if (!agree()) break;
+        // ---- 2. partition by first key: splitters from a sample of every rank's block of positions ----------
+        const u64 N = S.N, per = (N + (u64)G - 1) / (u64)G;
+        R.n_sample = 0;
+        {
+            const u64 lo = std::min(N, per * (u64)g), hi = std::min(N, per * (u64)(g + 1));
+            u32 got = 0;
+            run(pm_sample(ctx, S, lo, hi, MULTI_SAMPLE, R.h_sample, &got));
+            R.n_sample = got;
+        }
+        if (!agree()) break;
+        u64 spl[PFPB200_MAX_RANKS] = {0};
+        {
+            std::vector<u64> all;
+            for (int q = 0; q < G; q++) all.insert(all.end(), m->r[q].h_sample, m->r[q].h_sample + m->r[q].n_sample);
+            std::sort(all.begin(), all.end());
+            for (int q = 0; q + 1 < G; q++) spl[q] = all[std::min<size_t>(all.size() - 1, (size_t)(q + 1) * all.size() / (size_t)G)];
+        }
+        u64 M0 = 0;
+        run(pm_count(ctx, S, g > 0 ? spl[g - 1] : 0, g + 1 < G ? spl[g] : 0, g > 0, g + 1 < G, &M0));
+        S.M0 = M0;
+        if (ok() && M0 >= 0xFFFFFFFFull) {
+            char b[200];
+            snprintf(b, sizeof(b), "%llu dictionary suffixes on one GPU, 2^32 or more: list more GPUs",
+                     (unsigned long long)M0);
+            multi_fail(m, g, PFPB200_E_LIMIT, b);
+        }
+        if (!agree()) break;
+        S.base = 0;
+        for (int q = 0; q < g; q++) S.base += m->r[q].pb.M0;
+        if (ok()) run(pfp_alloc_t(ctx, &R.pb_rank, per));
+        int bn = 1;
+        while (bn < 64 && (N >> bn) != 0) bn++;
+        if (ok()) {
+            u64 mx = 0;                                      // one key layout for every rank: the largest share decides
+            for (int q = 0; q < G; q++) mx = std::max(mx, m->r[q].pb.M0);
+            int b = 1;
+            while (b < 64 && (mx >> b) != 0) b++;
+            run(pm_collect(ctx, S, (m->split_key || b + bn + 1 > 64) ? 1 : 0));
+        }
+        if (!agree()) break;
+        // ---- 3. prefix doubling in lockstep -------------------------------------------------------------------
+        PmRanks ranks;
+        memset(&ranks, 0, sizeof(ranks));
+        for (int q = 0; q < G; q++) ranks.blk[q] = m->r[q].pb_rank;
+        ranks.per = per;
+        bool alive = true;
+        u32 rounds = 1;
+        for (u64 h = (u64)S.h0;; h *= 2, rounds++) {
+            u64 active = 0;
+            if (ok()) run(pm_update(ctx, S, ranks, h, rounds == 1 ? 1 : 0, &active));   // stores changed ranks
+            bool failed = false;
+            const u64 tot = m->bar.sum(active, !ok(), &failed);
+            if (failed) { alive = false; break; }
+            if (tot == 0) {                                 // every rank's kernels are done: no peer reads my block any more
+                run(pfp_free_now(ctx, R.pb_rank));
+                break;
+            }
+            if (h >= 2 * N) {
+                if (g == 0) multi_fail(m, g, PFPB200_E_INTERNAL, "pfbwt: prefix doubling did not converge");
+                alive = false;
+                break;
+            }
+            if (ok()) run(pm_gather(ctx, S, ranks, h));                                 // loads rank(i+h)
+            if (!agree()) { alive = false; break; }
+            if (ok()) run(pm_sort(ctx, S));
+        }
+        R.pb_rounds = rounds;
+        if (!alive) break;
+        if (ok()) run(pm_sort_done(ctx, S));
+        t_sort = wall_sec();
+        // ---- 4. emission on my slice ------------------------------------------------------------------------
+        if (ok()) run(pm_count_chars(ctx, S));
+        if (!agree()) break;
+        u64 off = 0, n_bwt = 0;
+        for (int q = 0; q < G; q++) {
+            if (q < g) off += m->r[q].pb.chars;
+            n_bwt += m->r[q].pb.chars;
+        }
+        if (ok()) run(pm_fill(ctx, S));
+        if (!agree()) break;
+        int prev = -1, next = -1;                           // chars of the nearest non-empty pieces around mine
+        for (int q = g - 1; q >= 0 && prev < 0; q--) prev = m->r[q].pb.c_last;
+        for (int q = g + 1; q < G && next < 0; q++) next = m->r[q].pb.c_first;
+        if (ok() && (m->pb_flags & PFPB200_PFBWT_SSA)) run(pm_samples(ctx, S, 0, prev, next, off));
+        if (ok() && (m->pb_flags & PFPB200_PFBWT_ESA)) run(pm_samples(ctx, S, 1, prev, next, off));
+        t_emit = wall_sec();
+        if (!agree()) break;
+        // ---- 5. files: created by rank 0 at their final sizes, every rank writes its piece ---------------------
+        u64 off_s = 0, off_e = 0, tot_s = 0, tot_e = 0;
+        for (int q = 0; q < G; q++) {
+            if (q < g) { off_s += m->r[q].pb.n_ssa; off_e += m->r[q].pb.n_esa; }
+            tot_s += m->r[q].pb.n_ssa; tot_e += m->r[q].pb.n_esa;
+        }
+        char name[4096];
+        auto fname = [&](const char *ext) { snprintf(name, sizeof(name), "%s.%s", m->pb_base, ext); return name; };
+        if (g == 0) {
+            int bad = create_sized(m, fname("bwt"), n_bwt);
+            if (!bad && (m->pb_flags & PFPB200_PFBWT_SA)) bad = create_sized(m, fname("sa"), (n_bwt - 1) * PFP_IBYTES);
+            if (!bad && (m->pb_flags & PFPB200_PFBWT_SSA)) bad = create_sized(m, fname("ssa"), tot_s * 2 * PFP_IBYTES);
+            if (!bad && (m->pb_flags & PFPB200_PFBWT_ESA)) bad = create_sized(m, fname("esa"), tot_e * 2 * PFP_IBYTES);
+            if (bad) multi_fail(m, g, PFPB200_E_IO, m->io_err);
+        }
+        if (!agree()) break;
+        const u64 n = S.chars;
+        run(piece_to_file(R, fname("bwt"), off, S.bwt, n));
+        if (ok() && (m->pb_flags & PFPB200_PFBWT_SA) && n) {
+            // the .sa file has no entry for BWT position 0
+            if (off == 0) run(piece_to_file(R, fname("sa"), 0, S.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES));
+            else run(piece_to_file(R, fname("sa"), (off - 1) * PFP_IBYTES, S.sa5, n * PFP_IBYTES));
+        }
+        if (ok() && S.n_ssa) run(piece_to_file(R, fname("ssa"), off_s * 2 * PFP_IBYTES, S.ssa, S.n_ssa * 2 * PFP_IBYTES));
+        if (ok() && S.n_esa) run(piece_to_file(R, fname("esa"), off_e * 2 * PFP_IBYTES, S.esa, S.n_esa * 2 * PFP_IBYTES));
+        t_write = wall_sec();
+    } while (0);
+    cudaStreamSynchronize(ctx->stream);
+    R.pb_stat.suffixes = S.M0;
+    R.pb_stat.chars = S.chars;
+    R.pb_stat.hard = S.n_hard;
+    R.pb_stat.peak_bytes = ctx->arena.peak;
+    R.pb_stat.ms_read = (float)(1e3 * (t_read - t0));
+    R.pb_stat.ms_sort = (float)(1e3 * std::max(0.0, t_sort - t_read));
+    R.pb_stat.ms_emit = (float)(1e3 * std::max(0.0, t_emit - t_sort));
+    R.pb_stat.ms_write = (float)(1e3 * std::max(0.0, t_write - t_emit));
+    R.launches = ctx->launches - launches0;
+    m->bar.wait();                                          // no peer reads my memory any more
+    pfp_release_scratch(ctx);
+    m->bar.wait();                                          // rank 0's inputs, shared on its device, go last
+    pfp_release_held(ctx);
+}
+
+}  // namespace
+
+extern "C" int pfpb200_multi_pfbwt_file(pfpb200_multi *m, const char *basename, uint32_t w, uint32_t flags,
+                                        pfpb200_pfbwt_result *res) {
+    if (!m || !basename || !res) return PFPB200_E_ARG;
+    memset(res, 0, sizeof(*res));
+    m->err[0] = 0;
+    if (w < 4) { snprintf(m->err, sizeof(m->err), "Windows size must be at least 4"); return PFPB200_E_ARG; }
+    if ((flags & PFPB200_PFBWT_SA) && (flags & (PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA))) {
+        snprintf(m->err, sizeof(m->err), "You can either require the sampled SA or the full SA, not both");
+        return PFPB200_E_ARG;
+    }
+    for (int a = 0; a < m->n; a++)                          // the rank array is read and written across the GPUs
+        for (int b = 0; b < m->n; b++) {
+            const int da = m->r[a].device, db = m->r[b].device;
+            int can = 0;
+            if (da == db) continue;
+            if (cudaDeviceCanAccessPeer(&can, da, db) != cudaSuccess || !can) {
+                cudaGetLastError();
+                snprintf(m->err, sizeof(m->err),
+                         "CUDA devices %d and %d have no peer access: the sharded pfbwt loads and stores its rank "
+                         "array across the GPUs directly (NVLink); list devices that reach each other", da, db);
+                return PFPB200_E_ARG;
+            }
+        }
+    m->pb_base = basename;
+    m->pb_w = w;
+    m->pb_flags = flags;
+    m->failed.store(0);
+    std::vector<std::thread> th;
+    for (int g = 1; g < m->n; g++) th.emplace_back(pfbwt_rank_main, m, g);
+    pfbwt_rank_main(m, 0);
+    for (auto &t : th) t.join();
+    m->pb_base = nullptr;
+    const int rc = m->failed.load();
+    if (rc != PFPB200_OK) return rc;
+    const Rank &R0 = m->r[0];
+    for (const Rank &R : m->r) {
+        const pfpb200_pfbwt_rank &s = R.pb_stat;
+        res->n_bwt += s.chars;
+        res->n_ssa += R.pb.n_ssa;
+        res->n_esa += R.pb.n_esa;
+        res->hard += s.hard;
+        res->launches += R.launches;
+        res->ms_sa = std::max(res->ms_sa, s.ms_sort);
+        res->ms_fill = std::max(res->ms_fill, s.ms_emit);
+    }
+    if (flags & PFPB200_PFBWT_SA) res->n_sa = res->n_bwt - 1;
+    res->easy = res->n_bwt - res->hard;
+    res->dict_bytes = R0.pb_n[0];
+    res->dict_words = R0.pb_n[1];
+    res->parse_size = R0.pb_n[2];
+    res->rounds = R0.pb_rounds;
+    res->ms_total = res->ms_sa + res->ms_fill;
+    return PFPB200_OK;
+}
+
+extern "C" int pfpb200_multi_pfbwt_ranks(const pfpb200_multi *m, pfpb200_pfbwt_rank *out, int cap) {
+    if (!m || !out) return PFPB200_E_ARG;
+    int k = 0;
+    for (; k < m->n && k < cap; k++) out[k] = m->r[k].pb_stat;
+    return k;
 }

@@ -367,6 +367,13 @@ __global__ void __launch_bounds__(PB_T) pb_widen_k(const u8 *__restrict__ f, u64
     if (i < n) out[i] = f[i];
 }
 
+int pfp_dict_alphabet(pfpb200_ctx *ctx, const u8 *d, u64 N, u32 *present) {
+    PFP_CUDA(ctx, cudaMemsetAsync(present, 0, 8 * sizeof(u32), ctx->stream));
+    pb_alpha_k<<<ctx->sm_count * 8, PB_T, 0, ctx->stream>>>(d, N, present);
+    PFP_LAUNCHED(ctx);
+    return PFPB200_OK;
+}
+
 static int pb_bits(u64 v) {
     int b = 1;
     while (b < 64 && (v >> b) != 0) b++;

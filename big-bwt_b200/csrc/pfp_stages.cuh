@@ -131,3 +131,53 @@ int pfp_merge_verify(pfpb200_ctx *ctx, u64 n, const u32 *uid_of_entry, const u32
                      const u32 *uwords_in, const u64 *pool);
 int pfp_verify_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 first_start, u32 w, u64 P,
                      const DictArrays &D);
+
+// ---- the last stage (pfp_pfbwt.cu) and its sharded form (pfp_pfbwt_multi.cu) ---------------------------------
+// present[0..8): bit c set when byte value c occurs in d[0..N)
+int pfp_dict_alphabet(pfpb200_ctx *ctx, const u8 *d, u64 N, u32 *present);
+
+// the rank array of the sharded suffix sort, stored by position: block o = [o * per, (o + 1) * per)
+// lives on rank o; kernels load and store it through the peers' block pointers
+struct PmRanks {
+    u64 *blk[PFPB200_MAX_RANKS];
+    u64 per;
+};
+
+// one rank's state of a sharded pfbwt call (pfpb200_multi_pfbwt_file)
+struct PmState {
+    // inputs: the whole dictionary and parse-side streams (device pointers valid on this rank)
+    const u8 *d = nullptr; u64 N = 0;
+    const u32 *occ = nullptr; u64 dwords = 0;
+    const u32 *ilist = nullptr; const u8 *bwlast = nullptr, *bwsai = nullptr; u64 psize = 0;
+    u32 w = 0, flags = 0;
+    // word structure and first-key coding
+    u8 *tflag = nullptr; u32 *wid = nullptr, *istart = nullptr; u64 *wend = nullptr;
+    u8 code[256]; int bs = 0, h0 = 0;
+    // the owned first-key range and suffixes
+    u64 rg_lo = 0, rg_hi = 0; int rg_has_lo = 0, rg_has_hi = 0;
+    u64 M0 = 0, base = 0, M = 0, M2 = 0;
+    int bn = 0, bm = 0, split = 0;                  // key layout: bits of N, bits of M0, two sorts
+    u64 *pos = nullptr, *lo = nullptr; u32 *sl = nullptr, *hi = nullptr;   // per element (hi, lo: split key form)
+    u64 *k0 = nullptr, *k1 = nullptr, *ks = nullptr, *ko = nullptr;
+    u32 *v0 = nullptr, *v1 = nullptr, *vs = nullptr, *vo = nullptr;
+    u32 *slot = nullptr, *slot2 = nullptr, *head = nullptr, *escan = nullptr, *rs = nullptr;
+    u8 *flag = nullptr, *keep = nullptr;
+    u64 *sa_pos = nullptr; u32 *sa_grp = nullptr;  // per local slot
+    // emission
+    uint2 *mrec = nullptr; u16 *mc = nullptr; u32 *cnt = nullptr, *gscan = nullptr; u8 *newgrp = nullptr;
+    u64 *off = nullptr; u64 ngroups = 0, chars = 0, n_hard = 0;
+    u8 *bwt = nullptr, *sa5 = nullptr, *ssa = nullptr, *esa = nullptr;
+    u64 n_ssa = 0, n_esa = 0;
+    int c_first = -1, c_last = -1;                  // first / last char of the piece (-1: empty)
+};
+int pm_words(pfpb200_ctx *ctx, PmState &S);
+int pm_sample(pfpb200_ctx *ctx, PmState &S, u64 lo, u64 hi, u32 want, u64 *h_out, u32 *got);
+int pm_count(pfpb200_ctx *ctx, PmState &S, u64 klo, u64 khi, int has_lo, int has_hi, u64 *count);
+int pm_collect(pfpb200_ctx *ctx, PmState &S, int split);
+int pm_update(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h, int first, u64 *active);
+int pm_gather(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h);
+int pm_sort(pfpb200_ctx *ctx, PmState &S);
+int pm_sort_done(pfpb200_ctx *ctx, PmState &S);
+int pm_count_chars(pfpb200_ctx *ctx, PmState &S);
+int pm_fill(pfpb200_ctx *ctx, PmState &S);
+int pm_samples(pfpb200_ctx *ctx, PmState &S, int at_end, int prev, int next, u64 off);

@@ -80,6 +80,15 @@ class PfbwtResult(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k not in ("bwt", "sa", "ssa", "esa")}
 
 
+class PfbwtRank(C.Structure):
+    """include/pfpb200.h: pfpb200_pfbwt_rank (one rank of a sharded pfbwt call)."""
+    _fields_ = [("suffixes", C.c_uint64), ("chars", C.c_uint64), ("hard", C.c_uint64), ("peak_bytes", C.c_uint64),
+                ("ms_read", C.c_float), ("ms_sort", C.c_float), ("ms_emit", C.c_float), ("ms_write", C.c_float)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 @dataclass
 class BwtParseFiles:
     """.ilist / .bwlast / .bwsai as bytes (host copies)."""
@@ -121,7 +130,7 @@ SYMBOLS = ["pfpb200_create", "pfpb200_destroy", "pfpb200_set_stream", "pfpb200_p
            "pfpb200_dict_merge_finish",
            "pfpb200_shard_ranks_back", "pfpb200_multi_create", "pfpb200_multi_destroy", "pfpb200_multi_n_gpus",
            "pfpb200_multi_parse_host", "pfpb200_multi_parse_file", "pfpb200_multi_last_error",
-           "pfpb200_multi_phase_ms",
+           "pfpb200_multi_phase_ms", "pfpb200_multi_pfbwt_file", "pfpb200_multi_pfbwt_ranks",
            "pfpb200_check_dict_order",
            "pfpb200_bwtparse_device", "pfpb200_bwtparse_host", "pfpb200_bwtparse_file",
            "pfpb200_unparse_device", "pfpb200_unparse_file",
@@ -182,6 +191,10 @@ def load_library():
     L.pfpb200_multi_last_error.restype = C.c_char_p
     L.pfpb200_multi_phase_ms.argtypes = [vp, C.POINTER(C.c_float), C.c_int]
     L.pfpb200_multi_phase_ms.restype = C.c_int
+    L.pfpb200_multi_pfbwt_file.argtypes = [vp, C.c_char_p, u32, u32, C.POINTER(PfbwtResult)]
+    L.pfpb200_multi_pfbwt_file.restype = C.c_int
+    L.pfpb200_multi_pfbwt_ranks.argtypes = [vp, C.POINTER(PfbwtRank), C.c_int]
+    L.pfpb200_multi_pfbwt_ranks.restype = C.c_int
     _lib = L
     return L
 
@@ -492,6 +505,18 @@ class MultiScanner:
         o = Opts(w, p, _flags(sai, fasta, compress), nseg)
         self._check(self.L.pfpb200_multi_parse_file(self.h, os.fsencode(path), C.byref(o), C.byref(self.stats)))
         return self.stats.as_dict()
+
+    def pfbwt_file(self, basename, w=10, flags=0) -> dict:
+        """`pfbwt.x -w W [-S | -s -e] <basename>` sharded over the ranks: reads .dict .occ .ilist .bwlast
+        [.bwsai], writes the same .bwt [.sa | .ssa .esa] as Scanner.pfbwt_file.  Returns the summed counts,
+        the slowest rank's times and, under "ranks", each rank's suffixes, chars and times."""
+        r = PfbwtResult()
+        self._check(self.L.pfpb200_multi_pfbwt_file(self.h, os.fsencode(basename), w, flags, C.byref(r)))
+        d = r.as_dict()
+        buf = (PfbwtRank * len(self.gpu_ids))()
+        k = self.L.pfpb200_multi_pfbwt_ranks(self.h, buf, len(self.gpu_ids))
+        d["ranks"] = [buf[i].as_dict() for i in range(k)]
+        return d
 
     def phase_ms(self):
         """{phase: [ms of rank 0, rank 1, ...]} of the last parse."""

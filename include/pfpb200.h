@@ -381,6 +381,28 @@ int pfpb200_pfbwt_device(pfpb200_ctx *ctx, const uint8_t *d_dict, uint64_t dict_
 int pfpb200_pfbwt_file(pfpb200_ctx *ctx, const char *basename, uint32_t w, uint32_t flags,
                        pfpb200_pfbwt_result *res);
 
+/* ---- the last stage on several GPUs ---------------------------------------------------------------- *
+ * pfbwt over the ranks of a pfpb200_multi handle, for dictionaries of 4 GB and more: the same files as
+ * pfpb200_pfbwt_file, byte for byte, for every number of ranks.  Rank 0 reads the inputs and they
+ * travel peer to peer, so every rank holds the dictionary and the parse-side streams; the dictionary
+ * suffixes are partitioned by their first symbols, sorted by prefix doubling with the rank array
+ * spread over the GPUs (direct peer loads and stores: two different devices in the list need peer
+ * access), and every rank writes its contiguous piece of .bwt / .sa / .ssa / .esa into files rank 0
+ * created at their final sizes.  res: counts summed over the ranks, device pointers NULL, times the
+ * maximum over the ranks.  Limits: fewer than 2^32 suffixes per rank and fewer than 2^32 occurrences
+ * in one group of equal suffixes (PFPB200_E_LIMIT: list more GPUs), parse < 2^32-2 words. */
+int pfpb200_multi_pfbwt_file(pfpb200_multi *m, const char *basename, uint32_t w, uint32_t flags,
+                             pfpb200_pfbwt_result *res);
+typedef struct pfpb200_pfbwt_rank {
+    uint64_t suffixes;                       /* dictionary suffixes this rank sorted (its slice)     */
+    uint64_t chars;                          /* BWT chars (and SA values) it wrote                   */
+    uint64_t hard;                           /* of those, through the merge of the .ilist cursors    */
+    uint64_t peak_bytes;                     /* peak device memory of its context                    */
+    float ms_read, ms_sort, ms_emit, ms_write;   /* wall clock: inputs, suffix sort, emission, files */
+} pfpb200_pfbwt_rank;
+/* per-rank figures of the last pfpb200_multi_pfbwt_file call: fills up to cap entries, returns how many */
+int pfpb200_multi_pfbwt_ranks(const pfpb200_multi *m, pfpb200_pfbwt_rank *out, int cap);
+
 /* ---- the whole pipeline in one call --------------------------------------------------------------------- *
  * What `bigbwt <file> -w W -p P [-f] [-S | -s -e] [-k]` does with three processes and the files between
  * them (bigbwt:66-150): here the input streams into HBM, parse -> bwtparse -> pfbwt run there, and
