@@ -867,37 +867,10 @@ extern "C" int pfpb200_multi_parse_file(pfpb200_multi *m, const char *path, cons
 // barriers as the others; nobody frees memory a peer may still read before the last barrier.
 namespace {
 
-const char *const PB_EXT[5] = {"dict", "occ", "ilist", "bwlast", "bwsai"};
-const u64 PB_UNIT[5] = {1, 4, 4, 1, PFP_IBYTES};
-
-int pb_read_input(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count) {
-    char name[4096];
-    snprintf(name, sizeof(name), "%s.%s", base, PB_EXT[k]);
-    const int fd = open(name, O_RDONLY);
-    if (fd < 0) return pfp_fail(ctx, PFPB200_E_IO, "cannot open %s: %s", name, strerror(errno));
-    struct stat st;
-    if (fstat(fd, &st) != 0) { close(fd); return pfp_fail(ctx, PFPB200_E_IO, "cannot stat %s", name); }
-    const u64 bytes = (u64)st.st_size;
-    if (bytes % PB_UNIT[k] != 0) { close(fd); return pfp_fail(ctx, PFPB200_E_ARG, "invalid %s file", PB_EXT[k]); }
-    int rc = pfp_alloc(ctx, d, bytes, true);
-    if (rc == PFPB200_OK && bytes) rc = pfp_file_to_device(ctx, fd, 0, bytes, static_cast<u8 *>(*d));
-    close(fd);
-    *count = bytes / PB_UNIT[k];
-    return rc;
-}
-
 // rank 0: the input files into HBM, checked as pfpb200_pfbwt_file checks them
 int pb_inputs_rank0(pfpb200_multi *m, Rank &R) {
-    const bool want_sa = (m->pb_flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
     void *p[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    for (int k = 0; k < 4; k++) PFP_TRY(pb_read_input(R.ctx, m->pb_base, k, &p[k], &R.pb_n[k]));
-    if (R.pb_n[3] != R.pb_n[2])
-        return pfp_fail(R.ctx, PFPB200_E_ARG, ".bwlast holds %llu bytes, .ilist %llu entries",
-                        (unsigned long long)R.pb_n[3], (unsigned long long)R.pb_n[2]);
-    if (want_sa) {
-        PFP_TRY(pb_read_input(R.ctx, m->pb_base, 4, &p[4], &R.pb_n[4]));
-        if (R.pb_n[4] != R.pb_n[2]) return pfp_fail(R.ctx, PFPB200_E_ARG, "bwsa info read");
-    }
+    PFP_TRY(pb_read_inputs(R.ctx, m->pb_base, m->pb_flags, p, R.pb_n));
     const u64 N = R.pb_n[0], psize = R.pb_n[2];
     if (N <= 1 + (u64)m->pb_w) return pfp_fail(R.ctx, PFPB200_E_ARG, "invalid dictionary file");
     if (psize >= 0xFFFFFFFEull)
@@ -956,17 +929,13 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
         if (g == 0) run(pb_inputs_rank0(m, R));
         if (!agree()) break;
         if (g > 0) run(pb_inputs_peer(m, R));
-        S.d = (const u8 *)R.pb_in[0]; S.N = R.pb_n[0];
-        S.occ = (const u32 *)R.pb_in[1]; S.dwords = R.pb_n[1];
-        S.ilist = (const u32 *)R.pb_in[2]; S.psize = R.pb_n[2];
-        S.bwlast = (const u8 *)R.pb_in[3];
-        S.bwsai = want_sa ? (const u8 *)R.pb_in[4] : nullptr;
-        S.w = m->pb_w; S.flags = m->pb_flags;
-        if (ok()) run(pm_words(ctx, S));
+        S.in = PbInput{(const u8 *)R.pb_in[0], R.pb_n[0], (const u32 *)R.pb_in[1], R.pb_n[1], (const u32 *)R.pb_in[2],
+                       (const u8 *)R.pb_in[3], want_sa ? (const u8 *)R.pb_in[4] : nullptr, R.pb_n[2], m->pb_w, m->pb_flags};
+        if (ok()) run(pb_words(ctx, S.in, &S.wd));
         t_read = wall_sec();
         if (!agree()) break;
         // ---- 2. partition by first key: splitters from a sample of every rank's block of positions ----------
-        const u64 N = S.N, per = (N + (u64)G - 1) / (u64)G;
+        const u64 N = S.in.N, per = (N + (u64)G - 1) / (u64)G;
         R.n_sample = 0;
         {
             const u64 lo = std::min(N, per * (u64)g), hi = std::min(N, per * (u64)(g + 1));
@@ -995,14 +964,10 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
         S.base = 0;
         for (int q = 0; q < g; q++) S.base += m->r[q].pb.M0;
         if (ok()) run(pfp_alloc_t(ctx, &R.pb_rank, per));
-        int bn = 1;
-        while (bn < 64 && (N >> bn) != 0) bn++;
         if (ok()) {
             u64 mx = 0;                                      // one key layout for every rank: the largest share decides
             for (int q = 0; q < G; q++) mx = std::max(mx, m->r[q].pb.M0);
-            int b = 1;
-            while (b < 64 && (mx >> b) != 0) b++;
-            run(pm_collect(ctx, S, (m->split_key || b + bn + 1 > 64) ? 1 : 0));
+            run(pm_collect(ctx, S, (m->split_key || pb_bits(mx) + pb_bits(N) + 1 > 64) ? 1 : 0));
         }
         if (!agree()) break;
         // ---- 3. prefix doubling in lockstep -------------------------------------------------------------------
@@ -1012,7 +977,7 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
         ranks.per = per;
         bool alive = true;
         u32 rounds = 1;
-        for (u64 h = (u64)S.h0;; h *= 2, rounds++) {
+        for (u64 h = (u64)S.wd.h0;; h *= 2, rounds++) {
             u64 active = 0;
             if (ok()) run(pm_update(ctx, S, ranks, h, rounds == 1 ? 1 : 0, &active));   // stores changed ranks
             bool failed = false;
@@ -1036,20 +1001,18 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
         if (ok()) run(pm_sort_done(ctx, S));
         t_sort = wall_sec();
         // ---- 4. emission on my slice ------------------------------------------------------------------------
-        if (ok()) run(pm_count_chars(ctx, S));
+        if (ok()) run(pm_emit(ctx, S));
         if (!agree()) break;
         u64 off = 0, n_bwt = 0;
         for (int q = 0; q < G; q++) {
-            if (q < g) off += m->r[q].pb.chars;
-            n_bwt += m->r[q].pb.chars;
+            if (q < g) off += m->r[q].pb.em.chars;
+            n_bwt += m->r[q].pb.em.chars;
         }
-        if (ok()) run(pm_fill(ctx, S));
-        if (!agree()) break;
         int prev = -1, next = -1;                           // chars of the nearest non-empty pieces around mine
         for (int q = g - 1; q >= 0 && prev < 0; q--) prev = m->r[q].pb.c_last;
         for (int q = g + 1; q < G && next < 0; q++) next = m->r[q].pb.c_first;
-        if (ok() && (m->pb_flags & PFPB200_PFBWT_SSA)) run(pm_samples(ctx, S, 0, prev, next, off));
-        if (ok() && (m->pb_flags & PFPB200_PFBWT_ESA)) run(pm_samples(ctx, S, 1, prev, next, off));
+        if (ok() && (m->pb_flags & PFPB200_PFBWT_SSA)) run(pb_samples(ctx, S.em, 0, prev, next, off, false, &S.ssa, &S.n_ssa));
+        if (ok() && (m->pb_flags & PFPB200_PFBWT_ESA)) run(pb_samples(ctx, S.em, 1, prev, next, off, false, &S.esa, &S.n_esa));
         t_emit = wall_sec();
         if (!agree()) break;
         // ---- 5. files: created by rank 0 at their final sizes, every rank writes its piece ---------------------
@@ -1068,12 +1031,12 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
             if (bad) multi_fail(m, g, PFPB200_E_IO, m->io_err);
         }
         if (!agree()) break;
-        const u64 n = S.chars;
-        run(piece_to_file(R, fname("bwt"), off, S.bwt, n));
+        const u64 n = S.em.chars;
+        run(piece_to_file(R, fname("bwt"), off, S.em.bwt, n));
         if (ok() && (m->pb_flags & PFPB200_PFBWT_SA) && n) {
             // the .sa file has no entry for BWT position 0
-            if (off == 0) run(piece_to_file(R, fname("sa"), 0, S.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES));
-            else run(piece_to_file(R, fname("sa"), (off - 1) * PFP_IBYTES, S.sa5, n * PFP_IBYTES));
+            if (off == 0) run(piece_to_file(R, fname("sa"), 0, S.em.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES));
+            else run(piece_to_file(R, fname("sa"), (off - 1) * PFP_IBYTES, S.em.sa5, n * PFP_IBYTES));
         }
         if (ok() && S.n_ssa) run(piece_to_file(R, fname("ssa"), off_s * 2 * PFP_IBYTES, S.ssa, S.n_ssa * 2 * PFP_IBYTES));
         if (ok() && S.n_esa) run(piece_to_file(R, fname("esa"), off_e * 2 * PFP_IBYTES, S.esa, S.n_esa * 2 * PFP_IBYTES));
@@ -1081,8 +1044,8 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
     } while (0);
     cudaStreamSynchronize(ctx->stream);
     R.pb_stat.suffixes = S.M0;
-    R.pb_stat.chars = S.chars;
-    R.pb_stat.hard = S.n_hard;
+    R.pb_stat.chars = S.em.chars;
+    R.pb_stat.hard = S.em.n_hard;
     R.pb_stat.peak_bytes = ctx->arena.peak;
     R.pb_stat.ms_read = (float)(1e3 * (t_read - t0));
     R.pb_stat.ms_sort = (float)(1e3 * std::max(0.0, t_sort - t_read));
@@ -1102,9 +1065,8 @@ extern "C" int pfpb200_multi_pfbwt_file(pfpb200_multi *m, const char *basename, 
     if (!m || !basename || !res) return PFPB200_E_ARG;
     memset(res, 0, sizeof(*res));
     m->err[0] = 0;
-    if (w < 4) { snprintf(m->err, sizeof(m->err), "Windows size must be at least 4"); return PFPB200_E_ARG; }
-    if ((flags & PFPB200_PFBWT_SA) && (flags & (PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA))) {
-        snprintf(m->err, sizeof(m->err), "You can either require the sampled SA or the full SA, not both");
+    if (const char *e = pb_arg_error(w, flags)) {
+        snprintf(m->err, sizeof(m->err), "%s", e);
         return PFPB200_E_ARG;
     }
     for (int a = 0; a < m->n; a++)                          // the rank array is read and written across the GPUs

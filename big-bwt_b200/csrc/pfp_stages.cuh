@@ -133,8 +133,121 @@ int pfp_verify_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 
                      const DictArrays &D);
 
 // ---- the last stage (pfp_pfbwt.cu) and its sharded form (pfp_pfbwt_multi.cu) ---------------------------------
-// present[0..8): bit c set when byte value c occurs in d[0..N)
-int pfp_dict_alphabet(pfpb200_ctx *ctx, const u8 *d, u64 N, u32 *present);
+// pfp_pfbwt.cu holds what both paths compute the same way: the word structure and first-key coding,
+// the group heads of a doubling round, the emission and the sampled suffix array.  The two suffix
+// sorts stay apart; the emission reads a sort's output only through a slot reader (PbPackedSlots,
+// PbSplitSlots).
+constexpr int PB_T = 256;
+
+__device__ __forceinline__ bool pb_term(u8 c) { return c <= PFP_END_OF_WORD; }   // EndOfWord, EndOfDict
+
+// The ORDER-PRESERVING DENSE CODES of the byte values that occur in the dictionary (terminators 1,
+// then the text's alphabet from 2 up), bs bits each: a DNA dictionary has 7 values, 3 bits, and the
+// first round of a doubling already sorts by 21 symbols instead of 8.
+struct PbCodes { u8 code[256]; };
+
+// the first key of position t: its first h0 symbols as dense codes, cut behind the word's terminator
+// (zero padded); terminators get key 0 and sort in front.  code[]: PbCodes in shared memory
+__device__ __forceinline__ u64 pb_first_key(const u8 *__restrict__ d, u64 N, const u8 *code, int h0, int bs, u64 t) {
+    u64 k = 0;
+    bool live = !pb_term(d[t]);
+    for (int i = 0; i < h0; i++) {
+        u32 c = 0;
+        if (live) {
+            const u8 b = t + i < N ? d[t + i] : (u8)0;
+            c = code[b];
+            if (pb_term(b)) live = false;                            // the terminator itself is part of the key
+        }
+        k = (k << bs) | c;
+    }
+    return k;
+}
+
+static inline int pb_bits(u64 v) {
+    int b = 1;
+    while (b < 64 && (v >> b) != 0) b++;
+    return b;
+}
+
+__device__ __forceinline__ u64 pb_get5(const u8 *__restrict__ a, u64 i) {
+    u64 x = 0;
+#pragma unroll
+    for (int j = PFP_IBYTES - 1; j >= 0; j--) x = (x << 8) | a[i * PFP_IBYTES + j];
+    return x;
+}
+__device__ __forceinline__ void pb_put5(u8 *__restrict__ a, u64 i, u64 x) {
+#pragma unroll
+    for (int j = 0; j < PFP_IBYTES; j++) a[i * PFP_IBYTES + j] = (u8)(x >> (8 * j));
+}
+
+// launches a PB_T-thread kernel over n items, none when n = 0 (a rank of the sharded path may own nothing)
+#define PB_LAUNCH(ctx, n, kernel, ...)                                                          \
+    do {                                                                                        \
+        if ((n) > 0) {                                                                          \
+            kernel<<<pfp_blocks((n), PB_T), PB_T, 0, (ctx)->stream>>>(__VA_ARGS__);              \
+            PFP_LAUNCHED(ctx);                                                                  \
+        }                                                                                       \
+    } while (0)
+
+// group starts of a sorted key array, and head[group] = slot of its first member (escan: the scan of flag)
+__global__ void __launch_bounds__(PB_T) pb_gflags_k(const u64 *__restrict__ key, u64 M, u8 *__restrict__ flag);
+__global__ void __launch_bounds__(PB_T) pb_heads_k(const u8 *__restrict__ flag, const u32 *__restrict__ escan,
+                                                   const u32 *__restrict__ slot, u64 M, u32 *__restrict__ head);
+
+// the inputs of a pfbwt call: the dictionary and the parse-side streams (device pointers)
+struct PbInput {
+    const u8 *d = nullptr; u64 N = 0;
+    const u32 *occ = nullptr; u64 dwords = 0;
+    const u32 *ilist = nullptr; const u8 *bwlast = nullptr, *bwsai = nullptr; u64 psize = 0;
+    u32 w = 0, flags = 0;
+};
+
+// the word structure of the dictionary and the coding of the first key (pb_words)
+struct PbWords {
+    u32 *wid = nullptr;         // [N] word of every position (terminators before it)
+    u64 *wend = nullptr;        // [words + 1] position of every word's terminator
+    u32 *istart = nullptr;      // [words] first .ilist entry of every word, less one
+    PbCodes cd;
+    int bs = 0, h0 = 0;         // bits of a code, symbols in the first key
+};
+
+// slot k of the sorted dictionary suffixes -> its position and its group (the slot where the group
+// starts).  The one-GPU sort leaves (group << 32) | position in one u64, the sharded sort two arrays.
+struct PbPackedSlots {
+    const u64 *sa;
+    __device__ __forceinline__ u32 pos(u64 k) const { return (u32)sa[k]; }
+    __device__ __forceinline__ u32 grp(u64 k) const { return (u32)(sa[k] >> 32); }
+};
+struct PbSplitSlots {
+    const u64 *sa_pos;
+    const u32 *sa_grp;
+    __device__ __forceinline__ u64 pos(u64 k) const { return sa_pos[k]; }
+    __device__ __forceinline__ u32 grp(u64 k) const { return sa_grp[k]; }
+};
+
+// what the emission leaves: the BWT chars of the slots and, with -S / -s / -e, their suffix-array values
+struct PbEmit {
+    u8 *bwt = nullptr, *sa5 = nullptr;
+    u64 chars = 0, n_hard = 0, ngroups = 0;
+};
+
+// the argument checks of pfbwt.x: the message of the first one that fails, or null
+const char *pb_arg_error(u32 w, u32 flags);
+// .dict .occ .ilist .bwlast [.bwsai when flags want a suffix array] into held buffers (in[k], n[k] entries
+// of PB_UNIT[k] bytes), their sizes checked against each other
+constexpr u64 PB_UNIT[5] = {1, 4, 4, 1, PFP_IBYTES};
+int pb_read_inputs(pfpb200_ctx *ctx, const char *base, u32 flags, void *in[5], u64 n[5]);
+int pb_sync_read(pfpb200_ctx *ctx, int slot, int n);   // h_flags[slot, slot + n) <- d_flags, then synchronise
+int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W);
+// the BWT chars (and SA values) of n sorted slots; newgrp / gscan: scratch of n entries; held: the
+// outputs are held buffers recorded in ctx->pb_out[0..1], otherwise scratch
+template <class Slots>
+int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
+            PbEmit *E);
+// (BWT position + off, SA value) at the starts (at_end = 0) / ends of the runs of E's chars; prev / next:
+// the chars on either side of them (-1: none); held: the output is recorded in ctx->pb_out[2 + at_end]
+int pb_samples(pfpb200_ctx *ctx, const PbEmit &E, int at_end, int prev, int next, u64 off, bool held, u8 **out,
+               u64 *n_out);
 
 // the rank array of the sharded suffix sort, stored by position: block o = [o * per, (o + 1) * per)
 // lives on rank o; kernels load and store it through the peers' block pointers
@@ -145,14 +258,8 @@ struct PmRanks {
 
 // one rank's state of a sharded pfbwt call (pfpb200_multi_pfbwt_file)
 struct PmState {
-    // inputs: the whole dictionary and parse-side streams (device pointers valid on this rank)
-    const u8 *d = nullptr; u64 N = 0;
-    const u32 *occ = nullptr; u64 dwords = 0;
-    const u32 *ilist = nullptr; const u8 *bwlast = nullptr, *bwsai = nullptr; u64 psize = 0;
-    u32 w = 0, flags = 0;
-    // word structure and first-key coding
-    u8 *tflag = nullptr; u32 *wid = nullptr, *istart = nullptr; u64 *wend = nullptr;
-    u8 code[256]; int bs = 0, h0 = 0;
+    PbInput in;                                     // the whole dictionary and parse-side streams, on this rank
+    PbWords wd;
     // the owned first-key range and suffixes
     u64 rg_lo = 0, rg_hi = 0; int rg_has_lo = 0, rg_has_hi = 0;
     u64 M0 = 0, base = 0, M = 0, M2 = 0;
@@ -164,13 +271,11 @@ struct PmState {
     u8 *flag = nullptr, *keep = nullptr;
     u64 *sa_pos = nullptr; u32 *sa_grp = nullptr;  // per local slot
     // emission
-    uint2 *mrec = nullptr; u16 *mc = nullptr; u32 *cnt = nullptr, *gscan = nullptr; u8 *newgrp = nullptr;
-    u64 *off = nullptr; u64 ngroups = 0, chars = 0, n_hard = 0;
-    u8 *bwt = nullptr, *sa5 = nullptr, *ssa = nullptr, *esa = nullptr;
+    PbEmit em;
+    u8 *ssa = nullptr, *esa = nullptr;
     u64 n_ssa = 0, n_esa = 0;
     int c_first = -1, c_last = -1;                  // first / last char of the piece (-1: empty)
 };
-int pm_words(pfpb200_ctx *ctx, PmState &S);
 int pm_sample(pfpb200_ctx *ctx, PmState &S, u64 lo, u64 hi, u32 want, u64 *h_out, u32 *got);
 int pm_count(pfpb200_ctx *ctx, PmState &S, u64 klo, u64 khi, int has_lo, int has_hi, u64 *count);
 int pm_collect(pfpb200_ctx *ctx, PmState &S, int split);
@@ -178,6 +283,4 @@ int pm_update(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h, int first, 
 int pm_gather(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h);
 int pm_sort(pfpb200_ctx *ctx, PmState &S);
 int pm_sort_done(pfpb200_ctx *ctx, PmState &S);
-int pm_count_chars(pfpb200_ctx *ctx, PmState &S);
-int pm_fill(pfpb200_ctx *ctx, PmState &S);
-int pm_samples(pfpb200_ctx *ctx, PmState &S, int at_end, int prev, int next, u64 off);
+int pm_emit(pfpb200_ctx *ctx, PmState &S);
