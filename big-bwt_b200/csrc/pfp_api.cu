@@ -93,17 +93,10 @@ extern "C" int pfpb200_create(int device, pfpb200_ctx **out) {
     if (!ctx) return PFPB200_E_NOMEM;
     ctx->device = device;
     { const char *ev = getenv("PFPB200_LEGACY_K2"); ctx->legacy_k2 = ev && atoi(ev) != 0; }
-    { const char *ev = getenv("PFPB200_K1"); ctx->k1_mode = (ev && strcmp(ev, "rolling") == 0) ? 1 : (ev && strcmp(ev, "table") == 0) ? 2 : 0; }
+    { const char *ev = getenv("PFPB200_K1"); ctx->k1_rolling = ev && strcmp(ev, "rolling") == 0; }
     { const char *ev = getenv("PFPB200_TEST_WEAK_FP"); ctx->weak_fp = (ev && atoi(ev) != 0) ? 1u : 0u; }
-    { const char *ev = getenv("PFPB200_NO_SCAN_ALPHA"); ctx->no_scan_alpha = ev && atoi(ev) != 0; }
-    { const char *ev = getenv("PFPB200_RANK_FULL_SORT"); ctx->rank_full_sort = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_RANK_CHUNK_PASSES"); ctx->rank_chunk_passes = ev && atoi(ev) != 0; }
     { const char *ev = getenv("PFPB200_RANK_WARP_PASSES"); ctx->rank_warp_passes = ev && atoi(ev) != 0; }
-    { const char *ev = getenv("PFPB200_POOL_BY_WORD"); ctx->pool_by_word = ev && atoi(ev) != 0; }
-    { const char *ev = getenv("PFPB200_FUSE_K3"); ctx->fuse_k3 = ev && atoi(ev) != 0; }
-    { const char *ev = getenv("PFPB200_TABLE_SCALE"); if (ev && atof(ev) >= 1.2) ctx->table_scale = atof(ev); }
-    { const char *ev = getenv("PFPB200_K1_MIX"); ctx->k1_mix = ev ? atoi(ev) : 0; }
-    { const char *ev = getenv("PFPB200_K2_WINDOW"); ctx->k2_window = ev ? atoi(ev) : 0; }
     auto bail = [&](int code) { pfpb200_destroy(ctx); return code; };
     if (cudaSetDevice(device) != cudaSuccess) return bail(PFPB200_E_CUDA);
     cudaDeviceProp prop;
@@ -132,8 +125,7 @@ extern "C" int pfpb200_create(int device, pfpb200_ctx **out) {
         cudaEventCreateWithFlags(&ctx->ev_aux1, cudaEventDisableTiming) != cudaSuccess)
         return bail(PFPB200_E_CUDA);
     // per-device kernel attributes and constants of every stage (see pfp_common.cuh)
-    if (pfp_scan_init(ctx) || pfp_stream_init(ctx) || pfp_phrase_init(ctx) || pfp_prims_init(ctx) ||
-        pfp_rank_init(ctx))
+    if (pfp_scan_init(ctx) || pfp_stream_init(ctx) || pfp_prims_init(ctx) || pfp_rank_init(ctx))
         return bail(PFPB200_E_CUDA);
     *out = ctx;
     return PFPB200_OK;
@@ -150,7 +142,6 @@ extern "C" void pfpb200_destroy(pfpb200_ctx *ctx) {
     if (ctx->d_flags) cudaFree(ctx->d_flags);
     if (ctx->h_flags) cudaFreeHost(ctx->h_flags);
     if (ctx->d_keys) cudaFree(ctx->d_keys);
-    if (ctx->dna_table) cudaFree(ctx->dna_table);
     if (ctx->iv_etab) cudaFree(ctx->iv_etab);
     if (ctx->iv_xtab) cudaFree(ctx->iv_xtab);
     if (ctx->d_alpha) cudaFree(ctx->d_alpha);
@@ -259,17 +250,11 @@ static int parse_device_impl(pfpb200_ctx *ctx, const u8 *d_text, u64 n, const pf
         if (o->flags & PFPB200_F_SAI) PFP_TRY(pfp_alloc_t(ctx, &ph.sai, P * PFP_IBYTES, true));
         TextView tv{d_text, n, 0, (i64)n};
         DictArrays D;
-        const bool stream = pfp_stream_ok(sb, w) && !ctx->legacy_k2;
-        const bool fused = stream && ctx->fuse_k3;                      // K3 + pool inside the K2 pass (A/B)
-        if (fused) {
-            PFP_TRY(pfp_words_fused_stage(ctx, sb, tv, ph, P, -1, w, true, &D));
-        } else {
-            PFP_TRY(pfp_alloc_t(ctx, &ph.rec, P));
-            if (stream) PFP_TRY(pfp_stream_stage(ctx, sb, tv, ph, P, -1, w, true));
-            else {                                                      // any window size
-                PFP_TRY(pfp_scan_emit(ctx, sb, ends));
-                PFP_TRY(pfp_hash_stage(ctx, tv, ph, P, -1, w));
-            }
+        PFP_TRY(pfp_alloc_t(ctx, &ph.rec, P));
+        if (pfp_stream_ok(sb, w) && !ctx->legacy_k2) PFP_TRY(pfp_stream_stage(ctx, sb, tv, ph, P, -1, w, true));
+        else {                                                          // any window size
+            PFP_TRY(pfp_scan_emit(ctx, sb, ends));
+            PFP_TRY(pfp_hash_stage(ctx, tv, ph, P, -1, w));
         }
         PFP_TRY(pfp_scan_bits_free(ctx, &sb));
         tm.mark(ctx->stream);                                           // 2
@@ -290,12 +275,10 @@ static int parse_device_impl(pfpb200_ctx *ctx, const u8 *d_text, u64 n, const pf
             PFP_CUDA(ctx, cudaEventRecord(ctx->ev_copy, ctx->copy_stream));
             ctx->early_done = true;
         }
-        // K3 (when it did not run inside K2)
-        if (!fused) {
-            PFP_TRY(pfp_dedup_stage(ctx, ph, P, -1, w, &D));
-            PFP_TRY(pfp_free_now(ctx, ph.rec));
-            PFP_TRY(pfp_pool_stage(ctx, tv, ends, -1, w, &D));
-        }
+        // K3
+        PFP_TRY(pfp_dedup_stage(ctx, ph, P, -1, w, &D));
+        PFP_TRY(pfp_free_now(ctx, ph.rec));
+        PFP_TRY(pfp_pool_stage(ctx, tv, &D));
         if (o->flags & PFPB200_F_VERIFY) {
             PFP_TRY(pfp_uid_words(ctx, &D, P));
             PFP_TRY(pfp_verify_stage(ctx, tv, ends, -1, w, P, D));
@@ -303,7 +286,7 @@ static int parse_device_impl(pfpb200_ctx *ctx, const u8 *d_text, u64 n, const pf
         tm.mark(ctx->stream);                                           // 3
         // K4
         u32 *order = nullptr, rounds = 0;
-        PFP_TRY(pfp_rank_stage(ctx, D, &order, &rounds, ctx->alpha_valid && !ctx->no_scan_alpha));
+        PFP_TRY(pfp_rank_stage(ctx, D, &order, &rounds, ctx->alpha_valid));
         tm.mark(ctx->stream);                                           // 4
         u8 *dict = nullptr;
         u32 *occ = nullptr, *rank_of_uid = nullptr;
@@ -758,22 +741,17 @@ extern "C" int pfpb200_shard_words(pfpb200_ctx *ctx, int64_t first_start, pfpb20
         if (o.flags & PFPB200_F_SAI) PFP_TRY(pfp_alloc_t(ctx, &ph.sai, P * PFP_IBYTES, true));
         TextView tv{sh.d_buf, sh.n_buf, (i64)sh.buf_pos0, (i64)sh.n_global};
         DictArrays D;
-        const bool stream = pfp_stream_ok(ctx->sh.bits, w) && !ctx->legacy_k2;
-        const bool fused = stream && ctx->fuse_k3;
-        if (fused) {                       // K2 + K3 + pool in one pass; creators leave their fingerprints in rec
-            PFP_TRY(pfp_words_fused_stage(ctx, ctx->sh.bits, tv, ph, P, first_start, w, !ctx->sh.ends_emitted, &D));
-        } else {
-            if (stream) PFP_TRY(pfp_stream_stage(ctx, ctx->sh.bits, tv, ph, P, first_start, w, !ctx->sh.ends_emitted));
-            else PFP_TRY(pfp_hash_stage(ctx, tv, ph, P, first_start, w));
-            PFP_TRY(pfp_dedup_stage(ctx, ph, P, first_start, w, &D));
-            PFP_TRY(pfp_uid_words(ctx, &D, P));
-        }
+        if (pfp_stream_ok(ctx->sh.bits, w) && !ctx->legacy_k2)
+            PFP_TRY(pfp_stream_stage(ctx, ctx->sh.bits, tv, ph, P, first_start, w, !ctx->sh.ends_emitted));
+        else PFP_TRY(pfp_hash_stage(ctx, tv, ph, P, first_start, w));
+        PFP_TRY(pfp_dedup_stage(ctx, ph, P, first_start, w, &D));
+        PFP_TRY(pfp_uid_words(ctx, &D, P));
         u64 *wfpa = nullptr, *wfpb = nullptr;
         PFP_TRY(pfp_alloc_t(ctx, &wfpa, D.d));
         PFP_TRY(pfp_alloc_t(ctx, &wfpb, D.d));
         PFP_TRY(pfp_gather_word_fp(ctx, D, ph, wfpa, wfpb));
         PFP_TRY(pfp_free_now(ctx, ph.rec));
-        if (!fused) PFP_TRY(pfp_pool_stage(ctx, tv, ends, first_start, w, &D));
+        PFP_TRY(pfp_pool_stage(ctx, tv, &D));
         PFP_TRY(pfp_free_now(ctx, D.rep));
         if (o.flags & PFPB200_F_VERIFY) PFP_TRY(pfp_verify_stage(ctx, tv, ends, first_start, w, P, D));
         PFP_CUDA(ctx, cudaMemcpyAsync(ctx->h_flags, ctx->d_flags, sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));

@@ -62,30 +62,20 @@ struct pfpb200_ctx {
     cudaStream_t own_stream = nullptr;
     cudaStream_t stream = nullptr;
     u32 launches = 0;
-    int k1_mode = 0;               // PFPB200_K1=rolling: always the rolling-arithmetic scan kernel; =table: the 4^w-bit table form (A/B)
+    bool k1_rolling = false;       // PFPB200_K1=rolling: always the rolling-arithmetic scan kernel
     // byte values present in the text, as a by-product of the DNA form of K1 (8 x 32 bits): rows that
-    // pass the table path hold only A C G T, the others record their bytes.  Valid for the words of
+    // the interval form takes hold only A C G T, the others record their bytes.  Valid for the words of
     // a single-GPU parse; lets the ranking skip its own pass over the words' first bytes.
     u32 *d_alpha = nullptr;
     bool alpha_valid = false;
-    u32 *dna_table = nullptr;      // 4^w-bit trigger table of (dna_w, dna_p) for the DNA scan (w <= 10)
-    u32 dna_w = 0, dna_p = 0;
     void *iv_etab = nullptr;       // interval form of the DNA scan, tables of (iv_w, iv_p): 1024 x {a16 + 2, b16} (w <= 10)
     void *iv_xtab = nullptr;       //   or 256 x {f1 f0, f3 f2} (w <= 16); and the exact partial hashes {Ah, Bl} / {F0..F3}
     u32 iv_w = 0, iv_p = 0, iv_cthr = 0;
     int iv_skip = 0;               // > 0: the last scan found text that is not DNA, use the rolling kernel for this many calls
-    bool no_scan_alpha = false;      // PFPB200_NO_SCAN_ALPHA=1: the ranking finds the alphabet of the words itself (A/B)
-    bool rank_full_sort = false;     // PFPB200_RANK_FULL_SORT=1: radix-sort all 64 bits of the first key (A/B)
     bool rank_chunk_passes = false;  // PFPB200_RANK_CHUNK_PASSES=1: mid-size tie groups by chunk passes instead of LCP walks (A/B)
     bool rank_warp_passes = false;   // PFPB200_RANK_WARP_PASSES=1: tie groups of 2..32 words by warp chunk passes instead of LCP walks (A/B)
-    bool pool_by_word = false;       // PFPB200_POOL_BY_WORD=1: pool copy with eight lanes per word (A/B)
-    bool fuse_k3 = false;          // PFPB200_FUSE_K3=1: K3 + pool fused into the K2 pass (A/B; measured slower, see pfp_stream.cu)
-    double pool_ratio = 0.0;       // pool bytes / text bytes of the previous parse (pool sizing hint of the fused K2+K3)
     bool legacy_k2 = false;        // PFPB200_LEGACY_K2=1: per-phrase K2 kernels (A/B measurements)
-    double table_scale = 2.0;      // PFPB200_TABLE_SCALE: dictionary table slots per expected word (A/B)
     u32 weak_fp = 0;               // PFPB200_TEST_WEAK_FP=1 (tests): 2-bit fingerprints, so that PFPB200_F_VERIFY has collisions to catch
-    int k1_mix = 0;                // PFPB200_K1_MIX: every k-th row of the table scan by arithmetic (A/B)
-    int k2_window = 0;             // PFPB200_K2_WINDOW: shared-memory text window in phrase_hash_k (A/B)
     double dedup_ratio = 0.0;      // distinct words / phrases of the previous parse (table sizing hint)
     char err[512] = {0};
     std::vector<void *> scratch;   // freed at the end of every call
@@ -140,7 +130,6 @@ struct pfpb200_ctx {
 #define PFP_ERRBIT_LIMIT 2ull
 #define PFP_ERRBIT_INTERNAL 4ull
 #define PFP_ERRBIT_TABLE_FULL 8ull
-#define PFP_ERRBIT_POOL_FULL 16ull
 
 int pfp_fail(pfpb200_ctx *ctx, int code, const char *fmt, ...);
 
@@ -188,7 +177,6 @@ static inline int pfp_alloc_t(pfpb200_ctx *ctx, T **p, size_t count, bool held =
 // context's device -- so there is no process-wide "already done" state for host threads to race on.
 int pfp_scan_init(pfpb200_ctx *ctx);
 int pfp_stream_init(pfpb200_ctx *ctx);
-int pfp_phrase_init(pfpb200_ctx *ctx);
 int pfp_prims_init(pfpb200_ctx *ctx);
 int pfp_rank_init(pfpb200_ctx *ctx);
 

@@ -18,7 +18,6 @@
 #include "pfp_common.cuh"
 #include "pfp_stages.cuh"
 #include "pfp_fp.cuh"
-#include "pfp_table.cuh"
 #include <stdlib.h>
 
 // 16 bytes of a phrase at phrase offset o (multiple of 16), zero beyond the phrase end.
@@ -112,8 +111,6 @@ __global__ void phrase_records_k(TextView tv, const u64 *__restrict__ ends, u64 
 constexpr int PH_T = 256;
 constexpr int PH_WARPS = PH_T / 32;
 constexpr int PH_PER_BLOCK = PH_T;                   // one phrase per thread of a warp block
-constexpr int PH_WIN = 6144;                         // shared-memory text window per warp
-
 
 // A warp takes 32 consecutive phrases, flattens them into their 16-byte chunks and gives every
 // lane the same number of consecutive chunks (phrase lengths are geometric: giving lanes whole
@@ -126,18 +123,15 @@ __global__ void __launch_bounds__(PH_T) phrase_hash_k(TextView tv, PhraseArrays 
                                                       const u32 *__restrict__ keytab,
                                                       u32 *__restrict__ long_list,
                                                       u32 *__restrict__ long_count, u32 long_cap,
-                                                      u64 *__restrict__ flags, int use_window) {
+                                                      u64 *__restrict__ flags) {
     __shared__ __align__(16) u32 sk[NH_KEY_WORDS];
     __shared__ const u8 *s_ptr[PH_WARPS][32];
     __shared__ u32 s_len[PH_WARPS][32];
     __shared__ u32 s_pre[PH_WARPS][33];
     __shared__ unsigned long long s_acc[PH_WARPS][32][2];
-    extern __shared__ __align__(16) unsigned char ph_win[];     // PH_WARPS windows of PH_WIN bytes
     for (int i = threadIdx.x; i < NH_KEY_WORDS; i += PH_T) sk[i] = keytab[i];
     __syncthreads();
     const u32 lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-    unsigned char *win = ph_win + wp * PH_WIN;
-    const u8 *gend = tv.T + tv.n_buf;
     for (u64 j0 = ((u64)blockIdx.x * PH_WARPS + wp) * 32; j0 < P; j0 += (u64)gridDim.x * PH_PER_BLOCK) {
         const u64 j = j0 + lane;
         const bool valid = j < P;
@@ -162,28 +156,7 @@ __global__ void __launch_bounds__(PH_T) phrase_hash_k(TextView tv, PhraseArrays 
         const u32 nch = (mylen + 15) >> 4;
         const u32 incl = warp_incl_scan(nch);
         const u32 T = __shfl_sync(0xffffffffu, incl, 31);
-        // text window of the warp's phrases: one coalesced pass of 16-byte loads into shared
-        // memory, so that the per-lane chunk walks do not touch 32 cache lines per instruction
-        i64 wlo = mylen ? s0 - tv.pos0 : (i64)0x7fffffffffffffffLL;
-        i64 whi = mylen ? e - tv.pos0 + 1 : -1;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            wlo = min(wlo, __shfl_xor_sync(0xffffffffu, wlo, o));
-            whi = max(whi, __shfl_xor_sync(0xffffffffu, whi, o));
-        }
         const u8 *myptr = tv.T + (s0 - tv.pos0);
-        if (use_window && whi > wlo) {
-            const u8 *gbase = reinterpret_cast<const u8 *>(reinterpret_cast<uintptr_t>(tv.T + wlo) & ~(uintptr_t)15);
-            const u64 wbytes = (u64)((tv.T + whi) - gbase) + 24;    // + reach of the last 20-byte read
-            if (wbytes <= PH_WIN) {
-                for (u32 o = lane * 16; o < wbytes; o += 512) {
-                    uint4 v = make_uint4(0u, 0u, 0u, 0u);
-                    if (gbase + o < gend) v = __ldg(reinterpret_cast<const uint4 *>(gbase + o));
-                    *reinterpret_cast<uint4 *>(win + o) = v;
-                }
-                myptr = win + (myptr - gbase);
-            }
-        }
         s_ptr[wp][lane] = myptr;
         s_len[wp][lane] = mylen;
         s_pre[wp][lane] = incl - nch;
@@ -265,15 +238,14 @@ __global__ void __launch_bounds__(PH_T) phrase_hash_k(TextView tv, PhraseArrays 
 
 // Listed phrases (longer than one NH segment, touching the text borders, or left over by the
 // streaming pass): one warp per phrase, lanes stride over its 16-byte chunks; the chunks of
-// segment s enter the sum with weight FOLD^s (pfp_fp.cuh).
-__global__ void __launch_bounds__(PH_T) phrase_hash_long_k(TextView tv, PhraseArrays ph,
-                                                           i64 first_start, u32 w,
-                                                           const u32 *__restrict__ keytab,
-                                                           const u32 *__restrict__ long_list,
-                                                           const u32 *__restrict__ long_count, u32 long_cap,
-                                                           u64 *__restrict__ flags,
-                                                           PhraseFp *__restrict__ rec_compact /* non-null: record of
-                                                           the q-th listed phrase goes to rec_compact[q] */) {
+// segment s enter the sum with weight FOLD^s (pfp_fp.cuh).  Six CTAs per SM hold it at 40 registers
+// (48 resident warps); left to itself ptxas takes 46.
+__global__ void __launch_bounds__(PH_T, 6) phrase_hash_long_k(TextView tv, PhraseArrays ph,
+                                                              i64 first_start, u32 w,
+                                                              const u32 *__restrict__ keytab,
+                                                              const u32 *__restrict__ long_list,
+                                                              const u32 *__restrict__ long_count, u32 long_cap,
+                                                              u64 *__restrict__ flags) {
     __shared__ __align__(16) u32 sk[NH_KEY_WORDS];
     for (int i = threadIdx.x; i < NH_KEY_WORDS; i += PH_T) sk[i] = keytab[i];
     __syncthreads();
@@ -307,22 +279,58 @@ __global__ void __launch_bounds__(PH_T) phrase_hash_long_k(TextView tv, PhraseAr
         }
         if (lane == 0) {
             if (len > 0xFFFFFFFFull) atomicOr((unsigned long long *)&flags[0], PFP_ERRBIT_LIMIT);
-            if (rec_compact) store_rec(rec_compact, q, fa, fb);
-            else store_rec(ph.rec, j, fa, fb);
+            store_rec(ph.rec, j, fa, fb);
         }
     }
 }
 
-// ---- K3: dictionary table (slot layout and the probe loop: pfp_table.cuh) --------------------------------
+// ---- K3: dictionary table ---------------------------------------------------------------------------------
+// Open addressing, linear probing, 16-byte slots {key, val, check}; key 0 = empty.
+// A warp first groups its lanes by key (match.any) so that runs of identical phrases cost one
+// atomic per warp instead of 32.  `chk` is a 32-bit digest of the full 128-bit fingerprint and
+// the length, independent of the key: every phrase that lands in a slot must agree with it, or
+// the parse stops with PFPB200_E_COLLISION (the reference compares strings, newscan.cpp:282-286).
+// `val` is the word's occurrence count.
+struct __align__(16) DictSlot { u64 key; u32 val; u32 chk; };
+constexpr u32 TABLE_MAX_PROBES = 2048;
+
+__device__ __forceinline__ u32 check_of(const PhraseFp &r) {
+    u64 x = (r.fpa + 0x632BE59BD9B4E019ULL) * 0xD1342543DE82EF95ULL;
+    x ^= (rotl64(r.fpb, 23) + 0x2545F4914F6CDD1DULL) * 0xAF251AF3B0F025B5ULL;
+    x ^= x >> 29;
+    u32 c = (u32)(x ^ (x >> 32));
+    return c ? c : 1u;
+}
+
+// One probe sequence: a plain 16-byte load of the slot first -- on repetitive inputs nine phrases
+// in ten find their word already there and finish with one fire-and-forget add to its count --
+// and a CAS only on an empty slot.  The thread that wins the CAS is the word's creator.  Word ids
+// are not handed out here: table_insert_k leaves the slot in uid[] with a creator bit, and
+// table_compact_k numbers the words afterwards, in the order of their creators' records (one scan
+// over the records, no counter that every creator has to wait for).
+struct Probe { u64 slot; bool placed; bool creator; u32 seen_chk; };
+
+__device__ __forceinline__ Probe table_probe(DictSlot *__restrict__ tab, u64 cap, u64 slot, uint4 sv, u64 k) {
+    Probe r{slot, false, false, 0u};
+    u32 probes = 0;
+    for (;;) {
+        const u64 key = ((u64)sv.y << 32) | sv.x;
+        if (key == k) { r.placed = true; r.seen_chk = sv.w; break; }
+        if (key == 0ull) {
+            const u64 prev = atomicCAS((unsigned long long *)&tab[r.slot].key, 0ull, (unsigned long long)k);
+            if (prev == 0ull) { r.placed = true; r.creator = true; break; }
+            if (prev == k) { r.placed = true; break; }
+        }
+        if (++probes > TABLE_MAX_PROBES) break;               // table too small for this input
+        r.slot = (r.slot + 1 == cap) ? 0 : r.slot + 1;
+        sv = __ldcg(reinterpret_cast<const uint4 *>(tab + r.slot));
+    }
+    return r;
+}
+
 __global__ void table_init_k(DictSlot *__restrict__ tab, u64 cap) {
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < cap) *reinterpret_cast<uint4 *>(tab + i) = make_uint4(0u, 0u, 0u, 0u);
-}
-
-int pfp_table_init(pfpb200_ctx *ctx, DictSlot *tab, u64 cap) {
-    table_init_k<<<pfp_blocks(cap, 256), 256, 0, ctx->stream>>>(tab, cap);
-    PFP_LAUNCHED(ctx);
-    return PFPB200_OK;
 }
 
 constexpr int TI_T = 256;
@@ -555,22 +563,7 @@ static int table_words(pfpb200_ctx *ctx, const PhraseFp *rec, u64 n, DictSlot *t
     return PFPB200_OK;
 }
 
-// the few records of the fused K2 + K3 pass that met a slot whose creator had not stored the word id yet
-__global__ void table_pending_k(const DictSlot *__restrict__ tab, u64 P, u32 *__restrict__ uid,
-                                u32 *__restrict__ count) {
-    u64 j = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= P) return;
-    const u32 v = uid[j];
-    if (!(v & UID_PENDING)) return;
-    const u32 u = tab[v & ~UID_PENDING].val - 1;
-    uid[j] = u;
-    atomicAdd(&count[u], 1u);
-}
-
 // phrase pool: every distinct word once, zero padded to 8 bytes, 8-byte aligned
-constexpr int PC_GROUP = 8;                          // lanes per word
-constexpr int PC_PER_BLOCK = PH_T / PC_GROUP;
-
 // 8-byte word k of the phrase that starts at global position s0 and is len bytes long (zero
 // behind its end); special: the phrase touches a virtual border of the text
 __device__ __forceinline__ u64 phrase_word8(const TextView &tv, i64 s0, u64 len, u64 k, bool special) {
@@ -593,43 +586,11 @@ __device__ __forceinline__ u64 phrase_word8(const TextView &tv, i64 s0, u64 len,
     return v;
 }
 
-__global__ void __launch_bounds__(PH_T) pool_copy_k(TextView tv, const u64 *__restrict__ ends,
-                                                    i64 first_start, u32 w,
-                                                    const u32 *__restrict__ rep,
-                                                    const u32 *__restrict__ ulen,
-                                                    const u64 *__restrict__ uoff, u64 d,
-                                                    u64 *__restrict__ pool,
-                                                    const u32 *__restrict__ ulist /* null: words 0..d-1 */,
-                                                    const u32 *__restrict__ ucount, u64 pool_cap,
-                                                    const i64 *__restrict__ ustart /* null: from rep and ends */) {
-    const u32 li = threadIdx.x & (PC_GROUP - 1);
-    if (ulist) d = *ucount;
-    for (u64 x = (u64)blockIdx.x * PC_PER_BLOCK + (threadIdx.x / PC_GROUP); x < d;
-         x += (u64)gridDim.x * PC_PER_BLOCK) {
-        const u64 u = ulist ? ulist[x] : x;
-        const u64 len = ulen[u];
-        i64 s0, e;
-        if (ustart) {                              // noted by the word's creator: no walk through rep and ends
-            s0 = ustart[u];
-            e = s0 + (i64)len - 1;
-        } else {
-            const u64 j = rep[u];
-            e = (i64)ends[j];
-            s0 = (j == 0) ? first_start : (i64)ends[j - 1] - (i64)w + 1;
-        }
-        const bool special = (s0 < 0) || (e >= tv.n_global);
-        u64 nw = (len + 7) >> 3;
-        if (uoff[u] + nw > pool_cap) continue;                 // the caller sees PFP_ERRBIT_POOL_FULL and reruns
-        u64 *dst = pool + uoff[u];
-        for (u64 k = li; k < nw; k += PC_GROUP) dst[k] = phrase_word8(tv, s0, len, k, special);
-    }
-}
-
-// The same copy, organised by OUTPUT: the pool offsets ascend with the word id, so the 32 words of a
+// The copy is organised by OUTPUT: the pool offsets ascend with the word id, so the 32 words of a
 // warp fill one contiguous span of the pool; every lane takes consecutive 8-byte slots of that span
 // (coalesced stores, all lanes busy whatever the word lengths), finds the word a slot belongs to by
 // a binary search over the warp's 32 offsets (shuffles) and fetches its bytes from the text.
-// Measured against eight lanes per word (pool_copy_k): 0.65 -> see DESIGN (4 GB), half the instructions.
+// Eight lanes per word instead measured slower (DESIGN.md §3b).
 __global__ void __launch_bounds__(PH_T) pool_copy_span_k(TextView tv, const i64 *__restrict__ ustart,
                                                          const u32 *__restrict__ ulen,
                                                          const u64 *__restrict__ uoff, u64 d,
@@ -718,96 +679,19 @@ __global__ void __launch_bounds__(PH_T) verify_entries_k(u64 n, const u32 *__res
     }
 }
 
-// The few phrases the fused streaming pass leaves to the list kernel (the buffer's first phrase, a
-// final phrase at the virtual border, phrases open behind their tile or longer than a key
-// segment): one thread each, same table, same id / pool cursors.  A creator notes its word in
-// `created`, whose bytes pool_copy_k then fetches from the text.
-__global__ void table_insert_list_k(const PhraseFp *__restrict__ rec_small, const u32 *__restrict__ list,
-                                    const u32 *__restrict__ list_count, u32 list_cap,
-                                    DictSlot *__restrict__ tab, u64 cap, const u64 *__restrict__ ends,
-                                    i64 first_start, u32 w, u32 weak, u32 *__restrict__ uid,
-                                    u32 *__restrict__ rep, u32 *__restrict__ ulen, u32 *__restrict__ uwords,
-                                    u32 *__restrict__ count, u64 *__restrict__ uoff,
-                                    PhraseFp *__restrict__ rec_full, u32 *__restrict__ created,
-                                    u32 *__restrict__ created_count, u64 *__restrict__ flags) {
-    const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= min(*list_count, list_cap)) return;
-    const u64 j = list[i];
-    PhraseFp r = rec_small[i];
-    if (weak) { r.fpa &= 3ull; r.fpb = 0; }
-    const u64 k = sort_key_of(r.fpa, r.fpb);
-    const u32 chk = check_of(r);
-    const u64 s0 = __umul64hi(k, cap);
-    const Probe pr = table_probe(tab, cap, s0, __ldcg(reinterpret_cast<const uint4 *>(tab + s0)), k);
-    if (!pr.placed) { atomicOr((unsigned long long *)&flags[0], PFP_ERRBIT_TABLE_FULL); uid[j] = 0; return; }
-    u32 seen = pr.seen_chk;
-    if (pr.creator) {
-        const i64 st = j ? (i64)ends[j - 1] - (i64)w + 1 : first_start;
-        const u32 len = (u32)((i64)ends[j] - st + 1);
-        const u32 uw = (len + 7) >> 3;
-        const u32 u = (u32)atomicAdd((unsigned long long *)&flags[1], 1ull);
-        const u64 off = atomicAdd((unsigned long long *)&flags[7], (unsigned long long)uw);
-        atomicMax((unsigned long long *)&flags[2], (unsigned long long)len);
-        atomicAdd((unsigned long long *)&flags[3], (unsigned long long)len);
-        rep[u] = (u32)j; ulen[u] = len; uwords[u] = uw; uoff[u] = off;
-        tab[pr.slot].val = u + 1;
-        uid[j] = u;
-        atomicAdd(&count[u], 1u);
-        created[atomicAdd(created_count, 1u)] = u;
-        if (rec_full) store_rec(rec_full, j, r.fpa, r.fpb);
-    } else if (pr.seen_val) {
-        uid[j] = pr.seen_val - 1;
-        atomicAdd(&count[pr.seen_val - 1], 1u);
-    } else {
-        uid[j] = UID_PENDING | (u32)pr.slot;
-        atomicOr((unsigned long long *)&flags[6], 1ull);
-    }
-    if (seen == 0u) seen = atomicCAS(&tab[pr.slot].chk, 0u, chk);
-    if (seen != 0u && seen != chk) atomicOr((unsigned long long *)&flags[0], PFP_ERRBIT_COLLISION);
-}
-
-// insert the listed phrases (fingerprints in rec_small, list order) and copy the bytes of the words
-// they created into the pool
-int pfp_insert_list(pfpb200_ctx *ctx, const TextView &tv, const PhraseFp *rec_small, const u32 *list,
-                    const u32 *list_count, u64 list_cap, void *tab, u64 cap, const u64 *ends, i64 first_start,
-                    u32 w, const DictArrays &D, u64 pool_cap, PhraseFp *rec_full) {
-    u32 *created = nullptr;
-    PFP_TRY(pfp_alloc_t(ctx, &created, (size_t)list_cap + 1));
-    u32 *ccount = created + list_cap;
-    PFP_CUDA(ctx, cudaMemsetAsync(ccount, 0, sizeof(u32), ctx->stream));
-    const u32 lc = (u32)(list_cap < 0xFFFFFFFFull ? list_cap : 0xFFFFFFFFull);
-    table_insert_list_k<<<pfp_blocks(list_cap, 128), 128, 0, ctx->stream>>>(
-        rec_small, list, list_count, lc, (DictSlot *)tab, cap, ends, first_start, w, ctx->weak_fp, D.uid, D.rep, D.ulen,
-        D.uwords, D.count, D.uoff, rec_full, created, ccount, ctx->d_flags);
-    PFP_LAUNCHED(ctx);
-    u64 want = (list_cap + PC_PER_BLOCK - 1) / PC_PER_BLOCK;
-    u64 maxb = (u64)ctx->sm_count * 8;
-    pool_copy_k<<<(u32)(want < maxb ? (want ? want : 1) : maxb), PH_T, 0, ctx->stream>>>(
-        tv, ends, first_start, w, D.rep, D.ulen, D.uoff, 0, D.pool, created, ccount, pool_cap, nullptr);
-    PFP_LAUNCHED(ctx);
-    PFP_TRY(pfp_free_now(ctx, created));
-    return PFPB200_OK;
-}
-
-int pfp_table_pending(pfpb200_ctx *ctx, const void *tab, u64 P, u32 *uid, u32 *count) {
-    table_pending_k<<<pfp_blocks(P, 256), 256, 0, ctx->stream>>>((const DictSlot *)tab, P, uid, count);
-    PFP_LAUNCHED(ctx);
-    return PFPB200_OK;
-}
-
 // ------------------------------------------------------------------------------------------
 // host orchestration
 // ------------------------------------------------------------------------------------------
 // fingerprints of the phrases listed in long_list[0..*long_count): any length, any position
 int pfp_hash_list(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &ph, i64 first_start, u32 w,
-                  const u32 *long_list, const u32 *long_count, u64 max_count, PhraseFp *rec_compact) {
+                  const u32 *long_list, const u32 *long_count, u64 max_count) {
     u64 want = (max_count + PH_WARPS - 1) / PH_WARPS;
     u64 maxb = (u64)ctx->sm_count * 8;
     u32 nlb = (u32)(want < maxb ? want : maxb);
     if (nlb == 0) nlb = 1;
     phrase_hash_long_k<<<nlb, PH_T, 0, ctx->stream>>>(tv, ph, first_start, w, ctx->d_keys, long_list,
                                                       long_count, (u32)(max_count < 0xFFFFFFFFull ? max_count : 0xFFFFFFFFull),
-                                                      ctx->d_flags, rec_compact);
+                                                      ctx->d_flags);
     PFP_LAUNCHED(ctx);
     return PFPB200_OK;
 }
@@ -817,12 +701,6 @@ int pfp_records_range(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &
     if (j0 >= P) return PFPB200_OK;
     phrase_records_k<<<pfp_blocks(P - j0, 256), 256, 0, ctx->stream>>>(tv, ph.ends, j0, P, w, ph.last, ph.sai);
     PFP_LAUNCHED(ctx);
-    return PFPB200_OK;
-}
-
-int pfp_phrase_init(pfpb200_ctx *ctx) {
-    PFP_CUDA(ctx, cudaFuncSetAttribute(phrase_hash_k, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       PH_WARPS * PH_WIN));
     return PFPB200_OK;
 }
 
@@ -841,11 +719,10 @@ int pfp_hash_stage(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &ph,
     u64 maxb = (u64)ctx->sm_count * 32;
     u32 nb = (u32)(want < maxb ? want : maxb);
     if (nb == 0) nb = 1;
-    const int use_window = ctx->k2_window;   // measured: no gain on B200 once the atomics were gone
-    phrase_hash_k<<<nb, PH_T, use_window ? PH_WARPS * PH_WIN : 0, ctx->stream>>>(
-        tv, ph, P, first_start, w, ctx->d_keys, long_list, long_count, (u32)cap, ctx->d_flags, use_window);
+    phrase_hash_k<<<nb, PH_T, 0, ctx->stream>>>(tv, ph, P, first_start, w, ctx->d_keys, long_list, long_count,
+                                                (u32)cap, ctx->d_flags);
     PFP_LAUNCHED(ctx);
-    PFP_TRY(pfp_hash_list(ctx, tv, ph, first_start, w, long_list, long_count, cap, nullptr));
+    PFP_TRY(pfp_hash_list(ctx, tv, ph, first_start, w, long_list, long_count, cap));
     PFP_TRY(pfp_free_now(ctx, long_list));
     PFP_TRY(pfp_free_now(ctx, long_count));
     return PFPB200_OK;
@@ -870,7 +747,7 @@ int pfp_dedup_stage(pfpb200_ctx *ctx, const PhraseArrays &ph, u64 P, i64 first_s
     for (int attempt = 0;; attempt++) {
         double want = (double)P * 1.5;
         if (attempt == 0 && ctx->dedup_ratio > 0.0) {
-            double guess = ctx->dedup_ratio * (double)P * ctx->table_scale;
+            double guess = ctx->dedup_ratio * (double)P * 2.0;
             if (guess < want) want = guess;
         }
         cap = (u64)want + 1024;
@@ -914,8 +791,7 @@ int pfp_dedup_stage(pfpb200_ctx *ctx, const PhraseArrays &ph, u64 P, i64 first_s
 }
 
 // Builds the pool of distinct words.  One synchronisation (pool size, max / total word length).
-int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 first_start, u32 w,
-                   DictArrays *D) {
+int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, DictArrays *D) {
     u64 d = D->d;
     PFP_TRY(pfp_alloc_t(ctx, &D->uoff, d));
     PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, D->uwords, D->uoff, d, &ctx->d_flags[1]));
@@ -928,18 +804,10 @@ int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 fi
     D->max_len = (u32)ctx->h_flags[2];
     D->sum_len = ctx->h_flags[3];
     PFP_TRY(pfp_alloc_t(ctx, &D->pool, (size_t)D->pool_words));
-    u64 want = (d + PC_PER_BLOCK - 1) / PC_PER_BLOCK;
+    u64 want = (d + 32ull * PH_WARPS - 1) / (32ull * PH_WARPS);
     u64 maxb = (u64)ctx->sm_count * 32;
-    u32 nb = (u32)(want < maxb ? want : maxb);
-    if (nb == 0) nb = 1;
-    if (D->ustart && !ctx->pool_by_word) {
-        u64 wantw = (d + 32ull * PH_WARPS - 1) / (32ull * PH_WARPS);
-        pool_copy_span_k<<<(u32)(wantw < maxb ? (wantw ? wantw : 1) : maxb), PH_T, 0, ctx->stream>>>(
-            tv, D->ustart, D->ulen, D->uoff, d, D->pool);
-    } else {
-        pool_copy_k<<<nb, PH_T, 0, ctx->stream>>>(tv, ends, first_start, w, D->rep, D->ulen, D->uoff, d,
-                                                  D->pool, nullptr, nullptr, D->pool_words, D->ustart);
-    }
+    pool_copy_span_k<<<(u32)(want < maxb ? (want ? want : 1) : maxb), PH_T, 0, ctx->stream>>>(
+        tv, D->ustart, D->ulen, D->uoff, d, D->pool);
     PFP_LAUNCHED(ctx);
     return PFPB200_OK;
 }

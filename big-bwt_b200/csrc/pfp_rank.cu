@@ -1124,7 +1124,7 @@ int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bo
     int lg = 1;
     while (lg < 32 && (1ull << lg) < d) lg++;
     int sort_bits = (2 * lg + 2 + 7) / 8 * 8;
-    if (sort_bits > 64 || ctx->rank_full_sort) sort_bits = 64;
+    if (sort_bits > 64) sort_bits = 64;
     const int begin_bit = 64 - sort_bits;
     PFP_TRY(pfp_radix_sort_pairs(ctx, k0, v0, k1, v1, d, begin_bit, 64, &ks, &vs));
     rank_heads0_k<<<nbd, TB, 0, ctx->stream>>>(ks, d, am, (u32)begin_bit, head, depth);

@@ -166,17 +166,13 @@ __global__ void __launch_bounds__(K1_T) kr_scan_generic_k(const unsigned char *_
 }
 
 // ------------------------------------------------------------------------------------------------
-// K1a, DNA form (w <= 10).  For a window of w symbols from {A,C,G,T} the answer to "is this
-// window a trigger" is a function of 2w bits: a bit table of 4^w entries (128 KB for w = 10),
-// built once per (w, p) on the device from the SAME exact arithmetic, lives in shared memory.
-// One persistent CTA per SM; a warp takes 1 KB rows of the text, a lane 32 consecutive
-// positions: two coalesced 16-byte loads, 2-bit codes ((c >> 1) & 3: A=0 C=1 T=2 G=3) packed
-// four at a time with one multiply, the 9 symbols in front taken from the neighbour lane's
-// packed word by shuffle, and per position one funnel shift, one table word and one bit.
-// Exactness: every loaded byte is checked against the letter its code stands for (PRMT
-// decode + compare); a row with any other byte (N, lower case, text that is not DNA at all)
-// is redone by the same warp with the rolling arithmetic of kr_scan_k -- same trigger set for
-// every input, DNA or not.
+// K1a on DNA text: what the interval form (kr_scan_ivf_k) and its row kernel (kr_scan_rows_k)
+// share.  A warp takes 1 KB rows of the text, a lane 32 consecutive positions: two coalesced
+// 16-byte loads (kd_load_unit at the buffer's ends), 2-bit codes ((c >> 1) & 3: A=0 C=1 T=2 G=3)
+// packed four at a time with one multiply (dna_pack4 / dna_pack16).  Exactness: every loaded byte
+// is checked against the letter its code stands for (PRMT decode + compare); a row with any other
+// byte (N, lower case, text that is not DNA at all) is redone with the rolling arithmetic of
+// kr_scan_k (kd_row_by_arithmetic) -- same trigger set for every input, DNA or not.
 // ------------------------------------------------------------------------------------------------
 constexpr int KD_T = 1024;                    // threads per CTA (one CTA per SM)
 constexpr int KD_MAXW = 10;
@@ -184,26 +180,9 @@ constexpr u32 KD_LETTERS = 0x47544341u;       // code -> letter: 0 'A', 1 'C', 2
 
 // Powers of two kept in constant memory on purpose: a shift by a compile-time amount written as
 // a multiplication by an operand the compiler cannot see through is issued on the FMA pipe
-// (IMAD / IMAD.HI), which this kernel leaves idle, instead of the ALU pipe (SHF), which bounds it.
+// (IMAD / IMAD.HI), which has room, instead of the ALU pipe (SHF), which bounds these kernels.
 __constant__ u32 kd_pow2[33];
 __device__ __forceinline__ u32 shr_fma(u32 x, int s) { return s ? __umulhi(x, kd_pow2[32 - s]) : x; }
-// low 32 bits of (hi:lo) >> s, 0 < s < 32
-__device__ __forceinline__ u32 funnel_r_fma(u32 lo, u32 hi, int s) { return hi * kd_pow2[32 - s] + __umulhi(lo, kd_pow2[32 - s]); }
-
-__global__ void dna_table_k(pfp_scan_consts C, u32 *__restrict__ table, u32 nwords) {
-    const u32 wi = blockIdx.x * blockDim.x + threadIdx.x;
-    if (wi >= nwords) return;
-    u32 bits = 0;
-    for (u32 b = 0; b < 32; b++) {
-        const u32 idx = wi * 32 + b;          // symbol k of the window (k = 0 oldest) at bits [2k, 2k+2)
-        if (C.w < 16 && (idx >> (2 * C.w)) != 0) break;
-        u32 h = 0;
-        for (u32 k = 0; k < C.w; k++) h = pfp_push(h, (KD_LETTERS >> (8 * ((idx >> (2 * k)) & 3u))) & 255u);
-        if (pfp_is_trigger(h, C.pinv, C.pshift, C.plimit)) bits |= 1u << b;
-    }
-    table[wi] = bits;
-}
-
 // four text bytes -> their four 2-bit codes in bits 0..7 (first byte lowest); `bad` collects
 // every bit in which a byte differs from the letter of its code
 // returns a word whose TOP byte holds the four codes
@@ -229,8 +208,7 @@ __device__ __forceinline__ uint4 kd_load_unit(const uint4 *__restrict__ A, u64 q
     return make_uint4(0, 0, 0, 0);
 }
 
-// the byte values of a lane's 32 positions into the 256-bit set `alpha` (rows off the table path
-// only: kept out of line so that it costs the table path no registers)
+// the byte values of a lane's 32 positions into the 256-bit set `alpha` (kept out of line)
 __device__ __noinline__ void kd_note_alphabet(uint4 u0, uint4 u1, u64 q, u64 q_text0, u64 q_end, u32 lane,
                                                u32 *__restrict__ alpha) {
     const u32 xs[8] = {u0.x, u0.y, u0.z, u0.w, u1.x, u1.y, u1.z, u1.w};
@@ -252,9 +230,9 @@ __device__ __noinline__ void kd_note_alphabet(uint4 u0, uint4 u1, u64 q, u64 q_t
 // byte j (-16 <= j < 32) of {four words in front, eight words of the lane}
 #define KD_BYTE(wd, j) (__byte_perm((wd)[((j) + 16) >> 2], 0u, 0x4440u | (((j) + 16) & 3)))
 
-// A row that holds something besides A C G T (or that an A/B run gives to the arithmetic): the
-// trigger bits of the lane's 32 positions by the rolling arithmetic of kr_scan_k, exact for any
-// bytes; and, when the row is not pure A C G T, its byte values go into the alphabet set.
+// A row that holds something besides A C G T, or a clipped row at the buffer's ends: the trigger
+// bits of the lane's 32 positions by the rolling arithmetic of kr_scan_k, exact for any bytes; and,
+// when `note` is set, the row's byte values go into the alphabet set.
 template <int W>
 __device__ __noinline__ u32 kd_row_by_arithmetic(uint4 u0, uint4 u1, u32 lane, pfp_scan_consts C, u64 q, u64 q_text0,
                                                  u64 q_end, bool note, u32 *__restrict__ alpha) {
@@ -278,97 +256,12 @@ __device__ __noinline__ u32 kd_row_by_arithmetic(uint4 u0, uint4 u1, u32 lane, p
     return m;
 }
 
-// Rows overlap by one lane: row r covers the 32-position words 31r .. 31r+31 of the bit array,
-// lane 0 only supplies the symbols in front of lane 1 (its word belongs to lane 31 of row r-1).
-// Costs 1/32 of redundant work and removes every special case for "the bytes before my row".
-template <int W>
-__global__ void __launch_bounds__(KD_T, 1) kr_scan_dna_k(const uint4 *__restrict__ A, u64 q_end, u64 q_lo,
-                                                         u64 q_hi, pfp_scan_consts C,
-                                                         const u32 *__restrict__ table_g,
-                                                         u32 *__restrict__ mask32,
-                                                         u32 *__restrict__ tile_cnt, u64 nwords,
-                                                         u32 mix /* every mix-th row by arithmetic; 0: none */,
-                                                         u32 *__restrict__ alpha /* 256-bit set of the byte values seen */) {
-    extern __shared__ __align__(16) u32 tab[];
-    constexpr u32 TWORDS = ((1u << (2 * W)) + 31) / 32;
-    for (u32 i = threadIdx.x; i < TWORDS; i += KD_T) tab[i] = table_g[i];
-    __syncthreads();
-    const u32 lane = threadIdx.x & 31;
-    const u64 nrows = (nwords + 30) / 31;
-    const u64 wstride = (u64)gridDim.x * (KD_T / 32);
-    u64 row = (u64)blockIdx.x * (KD_T / 32) + (threadIdx.x >> 5);
-    if (row >= nrows) return;
-    const u64 q_full = q_end & ~(u64)15;               // whole 16-byte units end here
-    // software prefetch: the loads of the next row are in flight while this one is worked on
-    uint4 n0, n1;
-    {
-        const u64 q = (row * 31 + lane) * 32;
-        n0 = kd_load_unit(A, q_end, (i64)q);
-        n1 = kd_load_unit(A, q_end, (i64)q + 16);
-    }
-    for (; row < nrows; row += wstride) {
-        const uint4 u0 = n0, u1 = n1;
-        const u64 word = row * 31 + lane;               // my 32 positions = bit-array word `word`
-        const u64 q = word * 32;
-        const u64 nrow = row + wstride;
-        if (nrow < nrows) {
-            const u64 nq = (nrow * 31 + lane) * 32;
-            if ((nrow * 31 + 32) * 32 <= q_full) {      // interior row: no bounds to check
-                n0 = __ldg(A + (nq >> 4));
-                n1 = __ldg(A + (nq >> 4) + 1);
-            } else {
-                n0 = kd_load_unit(A, q_end, (i64)nq);
-                n1 = kd_load_unit(A, q_end, (i64)nq + 16);
-            }
-        }
-        u32 bad = 0;
-        const u32 S1 = dna_pack16(u0, bad), S2 = dna_pack16(u1, bad);
-        const u32 S0 = __shfl_up_sync(0xffffffffu, S2, 1);      // the 16 symbols in front of my run
-        u32 m = 0;
-        // mix > 0 gives every mix-th row to the arithmetic (table rows are bound by shared-memory
-        // bank conflicts, arithmetic rows by the ALU/FMA pipes).  Measured on B200, 4 GB, w=10:
-        // mix 0: 2.27 ms, 5: 2.68 ms, 3/6: 2.87 ms -- the slower rows only lengthen the tail. Off.
-        const bool by_table = !__any_sync(0xffffffffu, bad != 0) && !(mix && (row % mix) == mix - 1);
-        if (by_table) {
-            const u32 S[3] = {S0, S1, S2};
-#pragma unroll
-            for (int i = 0; i < 32; i++) {
-                const int b = 2 * (i + 16 - (W - 1));            // first stream bit of the window ending at i
-                const int k = b >> 5, sh = b & 31;
-                const int kh = (sh + 2 * W > 32) ? k + 1 : k;    // the window reaches into the next word
-                const u32 v = sh ? funnel_r_fma(S[k], S[kh], sh) : S[k];     // window in the low 2W bits
-                const u32 wd = *reinterpret_cast<const u32 *>(reinterpret_cast<const unsigned char *>(tab) +
-                                                              (shr_fma(v, 3) & (((1u << (2 * W)) - 1u) >> 5 << 2)));
-                m = __funnelshift_r(m, wd >> (v & 31), 1);        // bit i after 32 steps
-            }
-        } else {
-            // a row off the table path (warp-uniform, rare): out of line, so that it costs the table
-            // path neither registers nor instruction-cache lines
-            m = kd_row_by_arithmetic<W>(u0, u1, lane, C, q, q_lo >= (u64)(W - 1) ? q_lo - (u64)(W - 1) : 0, q_end,
-                                        __any_sync(0xffffffffu, bad != 0), alpha);
-        }
-        const bool mine = (lane != 0 || row == 0) && word < nwords;
-        if (q < q_lo || q + 32 > q_hi) m &= range_mask32(q, q_lo, q_hi);
-        if (!mine) m = 0;
-        if (mine) mask32[word] = m;
-        // per-tile counts: the words of a row lie in at most two tiles
-        const u32 c = __popc(m);
-        const u64 t0 = (row * 31 + 1) >> 10;
-        const bool in0 = (word >> 10) == t0 || lane == 0;
-        const u32 c0 = __reduce_add_sync(0xffffffffu, in0 ? c : 0u);
-        const u32 c1 = __reduce_add_sync(0xffffffffu, in0 ? 0u : c);
-        if (lane == 0) {
-            if (c0) atomicAdd(&tile_cnt[row == 0 ? 0 : t0], c0);
-            if (c1) atomicAdd(&tile_cnt[t0 + 1], c1);
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------------
 // K1a, interval form (w <= 10, p < PW) -- the default for DNA text since round 2.
 //
-// The bit-table form above pays 3.6 shared-memory wavefronts per position (32 random words in 32
-// banks).  This form needs ONE conflict-free wavefront, from two facts about the hash:
+// Round 1's form, a 4^w-bit trigger table in shared memory, paid 3.6 wavefronts per position (32
+// random words in 32 banks; DESIGN.md §3a).  This form needs ONE conflict-free wavefront, from two
+// facts about the hash:
 //  (1) it is LINEAR: H(window) = (Ah[hi] + Bl[lo]) mod PW, hi / lo = the codes of the w-5 older
 //      and the 5 newest symbols; and the hi block of the window ending at i IS the lo block of
 //      the window ending at i-5, so ONE table of 4^5 = 1024 entries, indexed by the 5-symbol block
@@ -385,7 +278,7 @@ __global__ void __launch_bounds__(KD_T, 1) kr_scan_dna_k(const uint4 *__restrict
 // Candidates (all triggers + 6e-5 of the positions for p = 100) are then decided EXACTLY from the
 // full 32-bit partial hashes {Ah, Bl} (a second, unreplicated 8 KB table) with the same
 // pfp_is_trigger() as everywhere else, so the trigger set is identical for every input; rows
-// holding anything besides A C G T go to the rolling arithmetic as in the bit-table form.
+// holding anything besides A C G T go to the rolling arithmetic (kr_scan_rows_k).
 // tests/test_arith.py::test_interval_form_* models both tables in numpy over all 4^10 windows.
 // ------------------------------------------------------------------------------------------------
 constexpr u32 KE_ENT = 1024;                                        // 5-symbol blocks
@@ -535,7 +428,10 @@ __device__ __forceinline__ u32 ke_row_bits(const u32 (&S)[3], const unsigned cha
 // The interior rows of the buffer (every position inside [q_lo, q_hi), whole 16-byte units): one
 // persistent 1024-thread CTA per SM, every warp walks a CONTIGUOUS run of rows (a running pointer
 // instead of 64-bit index arithmetic; the per-tile trigger counts are kept per lane and flushed
-// when the lane's word leaves its tile).  Rows overlap by one lane as in the bit-table form.
+// when the lane's word leaves its tile).  Rows overlap by one lane: row r covers the 32-position
+// words 31r .. 31r+31 of the bit array, lane 0 only supplies the symbols in front of lane 1 (its
+// word belongs to lane 31 of row r-1) -- 1/32 of redundant work, and no special case for "the
+// bytes before my row".
 // A row holding anything besides A C G T is not handled here: its number goes to `redo` and
 // kr_scan_rows_k does it by the rolling arithmetic -- this loop has no calls and no clipping.
 // BLK = 5: two blocks of 5 symbols (w <= 10); BLK = 4: four blocks of 4 symbols (11 <= w <= 16)
@@ -685,19 +581,6 @@ static void launch_scan(pfpb200_ctx *ctx, u32 ntiles, const uint4 *A, u64 q_end,
 #define K1_CASE(W) case W: launch_scan<W>(ctx, ntiles, A, q_end, q_lo, q_hi, C, mask, tile_cnt); break;
 
 template <int W>
-static cudaError_t launch_scan_dna(pfpb200_ctx *ctx, u32 ntiles, const uint4 *A, u64 q_end, u64 q_lo, u64 q_hi,
-                                   const pfp_scan_consts &C, uint4 *mask, u32 *tile_cnt) {
-    const size_t smem = (((size_t)1 << (2 * W)) + 31) / 32 * 4;
-    const u64 nwords = (u64)ntiles * (K1_TILE / 32);      // every word of every tile gets written
-    const int mix = ctx->k1_mix;
-    kr_scan_dna_k<W><<<ctx->sm_count, KD_T, smem, ctx->stream>>>(A, q_end, q_lo, q_hi, C, ctx->dna_table,
-                                                                reinterpret_cast<u32 *>(mask), tile_cnt, nwords,
-                                                                (u32)mix, ctx->d_alpha);
-    return cudaGetLastError();
-}
-#define KD_CASE(W) case W: le = launch_scan_dna<W>(ctx, ntiles, A, q_end, q_lo, q_hi, C, mask, tile_cnt); break;
-
-template <int W>
 static cudaError_t launch_scan_iv(pfpb200_ctx *ctx, u32 ntiles, const uint4 *A, u64 q_end, u64 q_lo, u64 q_hi,
                                   const pfp_scan_consts &C, uint4 *mask, u32 *tile_cnt, u32 *redo) {
     const u32 nwords = ntiles * (u32)(K1_TILE / 32);      // every word of every tile gets written
@@ -731,18 +614,9 @@ static cudaError_t launch_scan_iv(pfpb200_ctx *ctx, u32 ntiles, const uint4 *A, 
 }
 #define KE_CASE(W) case W: le = launch_scan_iv<W>(ctx, ntiles, A, q_end, q_lo, q_hi, C, mask, tile_cnt, redo); break;
 
-template <int W> static cudaError_t scan_attr() {
-    cudaError_t e = cudaFuncSetAttribute(kr_scan_k<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1_SMEM);
-    if (e == cudaSuccess && W <= KD_MAXW)
-        e = cudaFuncSetAttribute(kr_scan_dna_k<(W <= KD_MAXW ? W : KD_MAXW)>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)((((size_t)1 << (2 * (W <= KD_MAXW ? W : KD_MAXW))) + 31) / 32 * 4));
-    return e;
-}
-
 // dynamic shared memory limits of every scan kernel and the constant powers of two, on ctx's device
 int pfp_scan_init(pfpb200_ctx *ctx) {
-#define K1_ATTR(W) PFP_CUDA(ctx, scan_attr<W>());
+#define K1_ATTR(W) PFP_CUDA(ctx, cudaFuncSetAttribute(kr_scan_k<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1_SMEM));
     K1_ATTR(4) K1_ATTR(5) K1_ATTR(6) K1_ATTR(7) K1_ATTR(8) K1_ATTR(9) K1_ATTR(10)
     K1_ATTR(11) K1_ATTR(12) K1_ATTR(13) K1_ATTR(14) K1_ATTR(15) K1_ATTR(16)
     K1_ATTR(20) K1_ATTR(24) K1_ATTR(28) K1_ATTR(31) K1_ATTR(32)
@@ -753,18 +627,6 @@ int pfp_scan_init(pfpb200_ctx *ctx) {
     for (int i = 0; i < 32; i++) h[i] = 1u << i;
     h[32] = 0;
     PFP_CUDA(ctx, cudaMemcpyToSymbol(kd_pow2, h, sizeof(h), 0, cudaMemcpyHostToDevice));
-    return PFPB200_OK;
-}
-
-// the 4^w-bit trigger table of (w, p), cached in the context
-static int ensure_dna_table(pfpb200_ctx *ctx, const pfp_scan_consts &C) {
-    if (ctx->dna_table && ctx->dna_w == C.w && ctx->dna_p == C.p) return PFPB200_OK;
-    if (!ctx->dna_table) PFP_CUDA(ctx, cudaMalloc(&ctx->dna_table, ((size_t)1 << (2 * KD_MAXW)) / 8));
-    const u32 nwords = (u32)((((size_t)1 << (2 * C.w)) + 31) / 32);
-    dna_table_k<<<pfp_blocks(nwords, 256), 256, 0, ctx->stream>>>(C, ctx->dna_table, nwords);
-    PFP_LAUNCHED(ctx);
-    ctx->dna_w = C.w;
-    ctx->dna_p = C.p;
     return PFPB200_OK;
 }
 
@@ -842,42 +704,33 @@ int pfp_scan_bits(pfpb200_ctx *ctx, const u8 *d_buf, u64 n_buf, u64 buf_pos0, u6
     const cudaEvent_t e0 = evs[0], e1 = evs[1];
     // a text that is not DNA (most rows of the previous scan went to the arithmetic) is scanned by the
     // rolling kernel directly; the interval form is tried again every eighth call
-    const bool not_dna = ctx->k1_mode == 0 && ctx->iv_skip > 0 && ctx->iv_skip-- > 0;
-    // interval form (w <= 16): p must be invertible modulo PW and the threshold must leave the 16-bit range alone
-    const bool iv = w <= 16 && ctx->k1_mode == 0 && !not_dna && p >= 10 && p < PFP_PW &&
+    const bool not_dna = !ctx->k1_rolling && ctx->iv_skip > 0 && ctx->iv_skip-- > 0;
+    // interval form (w <= 16): p must be invertible modulo PW and the threshold must leave the 16-bit
+    // range alone; otherwise the rolling kernel
+    const bool iv = w <= 16 && !ctx->k1_rolling && !not_dna && p >= 10 && p < PFP_PW &&
                     (u64)ntiles * (K1_TILE / 32) < 0xFFFFFF00ull;
-    const bool dna = iv || (w <= (u32)KD_MAXW && ctx->k1_mode != 1 && !not_dna);
     u32 *redo = nullptr;                                   // rows the interval form hands to the arithmetic
     if (iv) {
         PFP_TRY(ensure_iv_tables(ctx, C));
         PFP_TRY(pfp_alloc_t(ctx, &redo, (size_t)ntiles * (K1_TILE / 32) / 31 + 2, false));
-    } else if (dna) {
-        PFP_TRY(ensure_dna_table(ctx, C));
     }
     PFP_CUDA(ctx, cudaEventRecord(e0, ctx->stream));
     ctx->alpha_valid = false;
-    if (dna) {
-        // the table form: bits and per-tile counts (added up by the warps) for every row
+    if (iv) {
+        // bits and per-tile counts (added up by the warps) for every row
         PFP_CUDA(ctx, cudaMemsetAsync(tile_cnt, 0, (size_t)ntiles * sizeof(u32), ctx->stream));
         PFP_CUDA(ctx, cudaMemsetAsync(ctx->d_alpha, 0, 8 * sizeof(u32), ctx->stream));
         ctx->alpha_valid = buf_pos0 == 0 && own_lo == 0;       // the whole text of a single-GPU parse
-        if (iv) PFP_CUDA(ctx, cudaMemsetAsync(&ctx->d_flags[3], 0, sizeof(u64), ctx->stream));
+        PFP_CUDA(ctx, cudaMemsetAsync(&ctx->d_flags[3], 0, sizeof(u64), ctx->stream));
         cudaError_t le = cudaSuccess;
-        if (iv) {
-            switch ((int)w) {
-                KE_CASE(4) KE_CASE(5) KE_CASE(6) KE_CASE(7) KE_CASE(8) KE_CASE(9) KE_CASE(10)
-                KE_CASE(11) KE_CASE(12) KE_CASE(13) KE_CASE(14) KE_CASE(15) KE_CASE(16)
-                default: le = cudaErrorInvalidValue;
-            }
-        } else {
-            switch ((int)w) {
-                KD_CASE(4) KD_CASE(5) KD_CASE(6) KD_CASE(7) KD_CASE(8) KD_CASE(9) KD_CASE(10)
-                default: le = cudaErrorInvalidValue;
-            }
+        switch ((int)w) {
+            KE_CASE(4) KE_CASE(5) KE_CASE(6) KE_CASE(7) KE_CASE(8) KE_CASE(9) KE_CASE(10)
+            KE_CASE(11) KE_CASE(12) KE_CASE(13) KE_CASE(14) KE_CASE(15) KE_CASE(16)
+            default: le = cudaErrorInvalidValue;
         }
         ctx->launches++;
         if (le != cudaSuccess)
-            return pfp_fail(ctx, PFPB200_E_CUDA, "%s launch: %s", iv ? "kr_scan_ivf_k / kr_scan_rows_k" : "kr_scan_dna_k", cudaGetErrorString(le));
+            return pfp_fail(ctx, PFPB200_E_CUDA, "kr_scan_ivf_k / kr_scan_rows_k launch: %s", cudaGetErrorString(le));
     } else {
         switch (w <= K1_MAXW_FAST ? (int)w : 0) {
             K1_CASE(4) K1_CASE(5) K1_CASE(6) K1_CASE(7) K1_CASE(8) K1_CASE(9) K1_CASE(10)

@@ -83,15 +83,7 @@ int pfp_scan_bits_free(pfpb200_ctx *ctx, ScanBits *sb);
 int pfp_hash_stage(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &ph, u64 P,
                    i64 first_start, u32 w);
 int pfp_hash_list(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &ph, i64 first_start, u32 w,
-                  const u32 *long_list, const u32 *long_count, u64 max_count, PhraseFp *rec_compact);
-int pfp_insert_list(pfpb200_ctx *ctx, const TextView &tv, const PhraseFp *rec_small, const u32 *list,
-                    const u32 *list_count, u64 list_cap, void *tab, u64 cap, const u64 *ends, i64 first_start,
-                    u32 w, const DictArrays &D, u64 pool_cap, PhraseFp *rec_full);
-int pfp_table_pending(pfpb200_ctx *ctx, const void *tab, u64 P, u32 *uid, u32 *count);
-// K2 + K3 + pool in one pass (the table insert fused into the streaming kernel); D is complete on
-// return.  ph.rec may be null (only sharded parsing keeps the creators' fingerprints).
-int pfp_words_fused_stage(pfpb200_ctx *ctx, const ScanBits &sb, const TextView &tv, const PhraseArrays &ph,
-                          u64 P, i64 first_start, u32 w, bool emit_ends, DictArrays *D);
+                  const u32 *long_list, const u32 *long_count, u64 max_count);
 int pfp_records_range(pfpb200_ctx *ctx, const TextView &tv, const PhraseArrays &ph, u64 j0, u64 P, u32 w);
 // K2 streaming: one pass over text + trigger bits writes ends (optional), .last, .sai and the
 // fingerprint records of all P phrases (ph.ends[P-1] must already hold a final virtual end, if any)
@@ -100,8 +92,7 @@ int pfp_stream_stage(pfpb200_ctx *ctx, const ScanBits &sb, const TextView &tv, c
                      u64 P, i64 first_start, u32 w, bool emit_ends);
 int pfp_dedup_stage(pfpb200_ctx *ctx, const PhraseArrays &ph, u64 P, i64 first_start, u32 w, DictArrays *D);
 int pfp_uid_words(pfpb200_ctx *ctx, DictArrays *D, u64 n);   // uid[0..n) -> word ids, if D->slot_of_word is set
-int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, const u64 *ends, i64 first_start, u32 w,
-                   DictArrays *D);
+int pfp_pool_stage(pfpb200_ctx *ctx, const TextView &tv, DictArrays *D);
 // Lexicographic order of the d pool words: order[i] = uid of the word of rank i+1.
 int pfp_rank_stage(pfpb200_ctx *ctx, DictArrays &D, u32 **order, u32 *rounds, bool alpha_from_scan = false);
 // .dict / .occ bytes and rank-per-uid from the order; outputs are `held` device buffers.

@@ -76,33 +76,6 @@ def test_divisibility_test(lib, p):
         assert bool(lib.t_trig(r, 10, p)) == (r % p == 0), (r, p)
 
 
-# ---- the table form of the scan (kr_scan_dna_k): its index layout and symbol coding, modelled in numpy ----
-def _dna_table(w, p):
-    """Bit idx of the table = "the window whose symbol k (k = 0 oldest) is code (idx >> 2k) & 3 is a
-    trigger", codes 0..3 = A C T G, i.e. (byte >> 1) & 3 -- what dna_table_k builds on the device."""
-    letters = np.array([65, 67, 84, 71], dtype=np.int64)
-    idx = np.arange(1 << (2 * w), dtype=np.int64)
-    h = np.zeros_like(idx)
-    for k in range(w):
-        h = (h * 256 + letters[(idx >> (2 * k)) & 3]) % PW
-    return (h % p) == 0
-
-
-@pytest.mark.parametrize("w,p", [(4, 10), (6, 50), (8, 16), (10, 100)])
-def test_table_form_of_the_scan_equals_the_rolling_hash(pkg, w, p):
-    from oracle import pfp_oracle as orc
-    text = pkg.synth.random_dna(200_000, 33 + w).numpy()
-    codes = (text.astype(np.int64) >> 1) & 3
-    assert np.array_equal(np.array([65, 67, 84, 71])[codes], text)       # the validity check of the kernel
-    table = _dna_table(w, p)
-    idx = np.zeros(text.size - w + 1, dtype=np.int64)
-    for k in range(w):                                                    # oldest symbol in the lowest bits
-        idx |= codes[k:text.size - w + 1 + k] << (2 * k)
-    got = np.flatnonzero(table[idx]) + (w - 1)
-    want = orc.triggers(text.tobytes(), w, p)
-    assert np.array_equal(got.astype(np.uint64), want)
-
-
 # ---- the interval form of the scan (kr_scan_iv_k): both tables modelled in numpy over ALL 4^10 windows ----
 def _interval_tables(w, p):
     """What dna_etab_k builds: per 5-symbol block x the exact partial hashes Ah (x as the w-5 older

@@ -60,9 +60,9 @@ def test_trigger_scan_vs_oracle(pkg, sc, w, p):
                                  (11, 100), (12, 50), (13, 1000), (14, 10), (15, 500), (16, 100), (16, 500), (16, 65536)])
 def test_interval_form_scan_vs_oracle_and_other_forms(pkg, w, p):
     """K1's interval form (kr_scan_ivf_k: two 5-symbol blocks for w <= 10, four 4-symbol blocks for
-    w <= 16) against the oracle and against the
-    bit-table and rolling forms, on DNA with rows that leave the table path (N runs, lower case,
-    a newline) and at misaligned starts.  p >= PW (last case) has no inverse: the library falls back."""
+    w <= 16) against the oracle and against the rolling form, on DNA with rows that leave the interval
+    form (N runs, lower case, a newline) and at misaligned starts.  p >= PW (the case (10, 3999999946))
+    has no inverse: the library falls back to the rolling form."""
     n = 700_000
     text = pkg.synth.random_dna(n, 77 + w).numpy().copy()
     text[100_000:103_000] = ord("N")
@@ -70,7 +70,7 @@ def test_interval_form_scan_vs_oracle_and_other_forms(pkg, w, p):
     text[500_000] = ord("\n")
     text[n - 5] = ord("N")
     want = orc.triggers(text.tobytes(), w, p)
-    for mode in ("", "table", "rolling"):
+    for mode in ("", "rolling"):
         old = os.environ.get("PFPB200_K1")
         if mode:
             os.environ["PFPB200_K1"] = mode
@@ -226,26 +226,6 @@ def test_rank_lcp_walks_on_large_families(pkg, w, p):
             os.environ.pop("PFPB200_RANK_CHUNK_PASSES", None)
         assert_same_files(s.parse_host(text, w, p), want, f"families w{w} p{p} chunk_passes={chunk_passes}")
         s.close()
-
-
-def test_fused_k3_equals_split_k3_64mb(pkg):
-    """The dictionary insert fused into the streaming K2 pass (PFPB200_FUSE_K3=1, an A/B path) against
-    K3 as its own kernels behind K2 (the default): same five streams, on a repetitive and on a
-    random text (the random one overflows the first pool / table guess and reruns the pass)."""
-    texts = [pkg.synth.pangenome_text(4_000_000, 16, 134).cuda(), pkg.synth.random_dna(48_000_000, 135, device="cuda")]
-    for t in texts:
-        res = []
-        for fuse in ("1", "0"):
-            os.environ["PFPB200_FUSE_K3"] = fuse
-            try:
-                s = pkg.pfp.Scanner(0)
-            finally:
-                os.environ.pop("PFPB200_FUSE_K3", None)
-            for _ in range(2):               # second parse: table and pool sized from the first
-                got = s.fetch(s.parse_device(t, 10, 100, sai=True))
-            res.append(got)
-            s.close()
-        assert_same_files(res[0], res[1], "fused vs split K3")
 
 
 @pytest.mark.parametrize("name", sorted(golden_dicz()))
