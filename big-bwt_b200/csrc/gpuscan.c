@@ -113,6 +113,13 @@ int main(int argc, char **argv) {
            st.ms_total, st.ms_scan, st.ms_emit, st.ms_hash, st.ms_dedup, st.ms_rank, st.rank_rounds,
            st.ms_dict, st.ms_remap, st.ms_h2d, st.ms_d2h, st.launches);
     printf("File read: %.3f s, file write: %.3f s\n", st.sec_read, st.sec_write);
+    if (ctx && verbose) {
+        uint64_t chunks = 0, peak = 0;
+        pfpb200_parse_plan(ctx, &chunks, &peak);
+        if (chunks) printf("Parse plan: streamed in %llu chunks, device peak %llu bytes\n",
+                           (unsigned long long)chunks, (unsigned long long)peak);
+        else printf("Parse plan: one-shot, device peak %llu bytes\n", (unsigned long long)peak);
+    }
     if (multi && verbose) {
         static const char *names[PFPB200_N_PHASES] = {"start", "h2d", "scan", "seams", "words", "splitters", "route",
                                                       "exchange", "merge", "ranks-back", "remap", "d2h"};

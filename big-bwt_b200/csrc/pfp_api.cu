@@ -479,11 +479,82 @@ static int cut_and_parse_device(pfpb200_ctx *ctx, const u8 *d_text, u64 n_text, 
 static int parse_file_impl(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, pfpb200_stats *stats,
                            bool write_files, pfpb200_outputs *dv_out);
 
+// Device bytes the one-shot parse_file takes per byte of input: the arena's high-water mark over the
+// file size, measured on a B200 at 1000 W (DESIGN.md §6b, profiles/r08_peaks.jsonl): config 2 (4 GB pan-genome, w 10 p 100) as plain
+// text ONESHOT_PEAK_PLAIN_C2, as 60-column FASTA ONESHOT_PEAK_FASTA_C2; config 4 (8 GB random ACGT,
+// nearly every phrase distinct) ONESHOT_PEAK_PLAIN_C4.  The estimate takes the larger plain figure, a
+// margin, and the fixed scratch of a parse (key table, flags, first slab); a smaller p has more
+// phrases per byte, and such a text may still end in PFPB200_E_NOMEM below the estimate, as before.
+constexpr double ONESHOT_PEAK_PLAIN_C2 = 1.749, ONESHOT_PEAK_FASTA_C2 = 1.985, ONESHOT_PEAK_PLAIN_C4 = 4.232;
+constexpr double ONESHOT_MARGIN = 1.15;
+constexpr u64 ONESHOT_FIXED = (u64)64 << 20;
+
+static u64 oneshot_estimate(u64 bytes, bool fasta) {
+    const double plain = ONESHOT_PEAK_PLAIN_C2 > ONESHOT_PEAK_PLAIN_C4 ? ONESHOT_PEAK_PLAIN_C2 : ONESHOT_PEAK_PLAIN_C4;
+    const double fa = ONESHOT_PEAK_FASTA_C2 * plain / ONESHOT_PEAK_PLAIN_C2;   // the raw bytes on top of the text
+    return (u64)((double)bytes * (fasta ? fa : plain) * ONESHOT_MARGIN) + ONESHOT_FIXED;
+}
+
+// Bytes of input the one-shot path holds: the file, or for gzip the text the host reader inflates
+// (the gzip trailer's size, mod 2^32: a lower bound for larger members)
+static u64 input_bytes(const char *path, bool fasta, bool *ok) {
+    struct stat sb;
+    *ok = stat(path, &sb) == 0;
+    if (!*ok) return 0;
+    u64 n = (u64)sb.st_size;
+    if (fasta && n >= 18) {
+        int fd = open(path, O_RDONLY);
+        if (fd >= 0) {
+            unsigned char mg[2] = {0, 0}, tr[4] = {0, 0, 0, 0};
+            if (pread(fd, mg, 2, 0) == 2 && mg[0] == 0x1f && mg[1] == 0x8b && pread(fd, tr, 4, (off_t)(n - 4)) == 4) {
+                const u64 isize = (u64)tr[0] | ((u64)tr[1] << 8) | ((u64)tr[2] << 16) | ((u64)tr[3] << 24);
+                if (isize > n) n = isize;
+            }
+            close(fd);
+        }
+    }
+    return n;
+}
+
 extern "C" int pfpb200_parse_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts,
                                   pfpb200_stats *stats) {
-    const int rc = parse_file_impl(ctx, path, opts, stats, true, nullptr);
-    if (ctx && rc == PFPB200_OK) pfp_release_held(ctx);
+    PFP_TRY(check_opts(ctx, opts));
+    if (!path) return pfp_fail(ctx, PFPB200_E_ARG, "null path");
+    ctx->plan_chunks = 0;
+    ctx->plan_peak = 0;
+    // Routing: the one-shot path for every input whose footprint fits the device memory available to
+    // the call (free memory plus what the context's arena holds unused); the streamed path otherwise.
+    // PFPB200_PARSE_BUDGET=<bytes> replaces that figure (tests: megabyte inputs take the streamed path).
+    PFP_TRY(begin_call(ctx));
+    u64 budget = 0;
+    const char *ev = getenv("PFPB200_PARSE_BUDGET");
+    if (ev && atoll(ev) > 0) budget = (u64)atoll(ev);
+    else {
+        size_t fr = 0, tot = 0;
+        PFP_CUDA(ctx, cudaMemGetInfo(&fr, &tot));
+        budget = (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
+    }
+    bool ok = false;
+    const u64 in = input_bytes(path, (opts->flags & PFPB200_F_FASTA) != 0, &ok);
+    int rc;
+    if (ok && oneshot_estimate(in, (opts->flags & PFPB200_F_FASTA) != 0) > budget) {
+        ctx->arena.peak = ctx->arena.in_use;
+        u64 chunks = 0;
+        rc = pfp_parse_file_streamed(ctx, path, opts, stats, budget, &chunks);
+        ctx->plan_chunks = chunks;
+    } else {
+        rc = parse_file_impl(ctx, path, opts, stats, true, nullptr);   // a missing file fails there
+    }
+    ctx->plan_peak = ctx->arena.peak;
+    if (rc == PFPB200_OK) pfp_release_held(ctx);
     return rc;
+}
+
+extern "C" int pfpb200_parse_plan(const pfpb200_ctx *ctx, uint64_t *chunks, uint64_t *peak_device_bytes) {
+    if (!ctx) return PFPB200_E_ARG;
+    if (chunks) *chunks = ctx->plan_chunks;
+    if (peak_device_bytes) *peak_device_bytes = ctx->plan_peak;
+    return PFPB200_OK;
 }
 
 // `bigbwt <file> -w W -p P [-f] [-S | -s -e]` in one call (bigbwt:66-150 runs newscan, bwtparse and
@@ -545,6 +616,7 @@ static int parse_file_impl(pfpb200_ctx *ctx, const char *path, const pfpb200_opt
         if (pread(fd, mg, 2, 0) == 2) gz = mg[0] == 0x1f && mg[1] == 0x8b;
     }
     PFP_TRY(begin_call(ctx));
+    ctx->arena.peak = ctx->arena.in_use;                       // pfpb200_parse_plan reports this call's peak
     pfpb200_outputs dv;
     memset(&dv, 0, sizeof(dv));
     double t1 = t0;

@@ -77,6 +77,7 @@ struct pfpb200_ctx {
     bool legacy_k2 = false;        // PFPB200_LEGACY_K2=1: per-phrase K2 kernels (A/B measurements)
     u32 weak_fp = 0;               // PFPB200_TEST_WEAK_FP=1 (tests): 2-bit fingerprints, so that PFPB200_F_VERIFY has collisions to catch
     double dedup_ratio = 0.0;      // distinct words / phrases of the previous parse (table sizing hint)
+    u64 plan_chunks = 0, plan_peak = 0;   // pfpb200_parse_plan: chunks (0: one-shot) and arena peak of the last parse_file
     char err[512] = {0};
     std::vector<void *> scratch;   // freed at the end of every call
     std::vector<void *> held;      // outputs: freed at the start of the next call / destroy

@@ -26,6 +26,16 @@ __device__ __forceinline__ u64 sort_key_of(u64 fa, u64 fb) {
     return k ? k : 0x9E3779B97F4A7C15ULL;
 }
 
+// 32-bit digest of the 128-bit fingerprint, independent of the table key: words that share a key
+// must agree on it (never 0: 0 marks a slot whose digest is not written yet)
+__device__ __forceinline__ u32 check_of(const PhraseFp &r) {
+    u64 x = (r.fpa + 0x632BE59BD9B4E019ULL) * 0xD1342543DE82EF95ULL;
+    x ^= (rotl64(r.fpb, 23) + 0x2545F4914F6CDD1DULL) * 0xAF251AF3B0F025B5ULL;
+    x ^= x >> 29;
+    u32 c = (u32)(x ^ (x >> 32));
+    return c ? c : 1u;
+}
+
 __device__ __forceinline__ void store_rec(PhraseFp *rec, u64 j, u64 fa, u64 fb) {
     *reinterpret_cast<uint4 *>(rec + j) = make_uint4((u32)fa, (u32)(fa >> 32), (u32)fb, (u32)(fb >> 32));
 }

@@ -182,6 +182,7 @@ int pfp_device_to_fd(pfpb200_ctx *ctx, int fd, u64 file_off, const void *d_src, 
 // runs to the end of its line; then lines are appended without their newline until a line starts
 // with '>', '@' or '+'.)
 enum : u32 { FS_H = 0, FS_S = 1, FS_L = 2 };
+static_assert(FS_L == PFP_FASTA_LINE_START, "the streamed parse starts a file in state L");
 
 // Summary of a run of bytes.  Up to its first newline a run behaves according to the state it is
 // entered in (all kept or all dropped); behind the first newline everything is fixed.
@@ -349,9 +350,9 @@ __device__ __forceinline__ FaSum64 fa_join64(const FaSum64 &a, const FaSum &b) {
     return r;
 }
 
-__global__ void __launch_bounds__(1024) fasta_scan_k(const FaSum *__restrict__ tsum, u32 ntiles,
+__global__ void __launch_bounds__(1024) fasta_scan_k(const FaSum *__restrict__ tsum, u32 ntiles, u32 start,
                                                      u32 *__restrict__ tstate, u64 *__restrict__ toff,
-                                                     u64 *__restrict__ total) {
+                                                     u64 *__restrict__ total, u32 *__restrict__ end_state) {
     __shared__ u32 s_state[1024];
     __shared__ u64 s_kept[1024];
     __shared__ FaSum64 s_sum[1024];
@@ -363,8 +364,8 @@ __global__ void __launch_bounds__(1024) fasta_scan_k(const FaSum *__restrict__ t
     for (u32 i = lo; i < hi; i++) acc = fa_join64(acc, tsum[i]);
     s_sum[t] = acc;
     __syncthreads();
-    if (t == 0) {                                  // chain the 1024 slices from the file start (state L)
-        u32 st = FS_L;
+    if (t == 0) {                                  // chain the 1024 slices from the entry state
+        u32 st = start;
         u64 kept = 0;
         for (u32 k = 0; k < 1024; k++) {
             const FaSum64 b = s_sum[k];
@@ -374,6 +375,7 @@ __global__ void __launch_bounds__(1024) fasta_scan_k(const FaSum *__restrict__ t
             st = fa_out64(b.head, b.flags, st);
         }
         *total = kept;
+        *end_state = st;
     }
     __syncthreads();
     u32 st = s_state[t];
@@ -450,8 +452,11 @@ __global__ void fasta_first_byte_k(const u8 *__restrict__ f, u32 *__restrict__ f
 // d_file[0..n) (FASTA bytes in HBM) -> *d_text, *n_text.  *d_text non-null on entry: the caller's
 // buffer (>= n + 16 bytes) is filled; else an arena buffer of ctx (held or scratch).
 // *supported = 0: the file needs the host reader, nothing was produced.
+// state: null = d_file is the whole file.  Otherwise d_file is a piece of it: *state holds the
+// automaton state in front of it (FS_L at the file start) and receives the state behind it, and the
+// leading '>' is required only of the piece that starts the file.
 int pfp_fasta_device(pfpb200_ctx *ctx, const u8 *d_file, u64 n, u8 **d_text, u64 *n_text, int *supported,
-                     bool held) {
+                     bool held, u32 *state, bool file_start) {
     u8 *const user_out = *d_text;
     *d_text = nullptr;
     *n_text = 0;
@@ -469,11 +474,13 @@ int pfp_fasta_device(pfpb200_ctx *ctx, const u8 *d_file, u64 n, u8 **d_text, u64
     PFP_TRY(pfp_alloc_t(ctx, &flags, 4));
     total = reinterpret_cast<u64 *>(flags + 2);
     PFP_CUDA(ctx, cudaMemsetAsync(flags, 0, 4 * sizeof(u32), ctx->stream));
-    fasta_first_byte_k<<<1, 1, 0, ctx->stream>>>(d_file, flags);
-    PFP_LAUNCHED(ctx);
+    if (file_start) {
+        fasta_first_byte_k<<<1, 1, 0, ctx->stream>>>(d_file, flags);
+        PFP_LAUNCHED(ctx);
+    }
     fasta_sum_k<<<ntiles, K0_T, 0, ctx->stream>>>(d_file, n, tsum, flags);
     PFP_LAUNCHED(ctx);
-    fasta_scan_k<<<1, 1024, 0, ctx->stream>>>(tsum, ntiles, tstate, toff, total);
+    fasta_scan_k<<<1, 1024, 0, ctx->stream>>>(tsum, ntiles, state ? *state : (u32)FS_L, tstate, toff, total, flags + 1);
     PFP_LAUNCHED(ctx);
     u32 h[4];
     PFP_CUDA(ctx, cudaMemcpyAsync(h, flags, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
@@ -491,7 +498,7 @@ int pfp_fasta_device(pfpb200_ctx *ctx, const u8 *d_file, u64 n, u8 **d_text, u64
         PFP_CUDA(ctx, cudaMemcpyAsync(h, flags, sizeof(u32), cudaMemcpyDeviceToHost, ctx->stream));
         PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         if (h[0] & K0_BAD) { *supported = 0; if (!user_out) PFP_TRY(pfp_free_now(ctx, out)); }
-        else { *d_text = out; *n_text = kept; }
+        else { *d_text = out; *n_text = kept; if (state) *state = h[1]; }
     }
     PFP_TRY(pfp_free_now(ctx, tsum));
     PFP_TRY(pfp_free_now(ctx, tstate));

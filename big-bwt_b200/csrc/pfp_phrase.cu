@@ -294,14 +294,6 @@ __global__ void __launch_bounds__(PH_T, 6) phrase_hash_long_k(TextView tv, Phras
 struct __align__(16) DictSlot { u64 key; u32 val; u32 chk; };
 constexpr u32 TABLE_MAX_PROBES = 2048;
 
-__device__ __forceinline__ u32 check_of(const PhraseFp &r) {
-    u64 x = (r.fpa + 0x632BE59BD9B4E019ULL) * 0xD1342543DE82EF95ULL;
-    x ^= (rotl64(r.fpb, 23) + 0x2545F4914F6CDD1DULL) * 0xAF251AF3B0F025B5ULL;
-    x ^= x >> 29;
-    u32 c = (u32)(x ^ (x >> 32));
-    return c ? c : 1u;
-}
-
 // One probe sequence: a plain 16-byte load of the slot first -- on repetitive inputs nine phrases
 // in ten find their word already there and finish with one fire-and-forget add to its count --
 // and a CAS only on an empty slot.  The thread that wins the CAS is the word's creator.  Word ids

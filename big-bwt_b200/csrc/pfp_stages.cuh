@@ -108,9 +108,16 @@ int pfp_file_to_device(pfpb200_ctx *ctx, int fd, u64 off, u64 bytes, u8 *d_dst);
 int pfp_device_to_file(pfpb200_ctx *ctx, const char *name, const void *d_src, u64 bytes);
 int pfp_device_to_fd(pfpb200_ctx *ctx, int fd, u64 file_off, const void *d_src, u64 bytes, const char *name);
 void pfp_io_destroy(pfpb200_ctx *ctx);
-// FASTA bytes in HBM -> the text T of `-f` mode (kseq.h:177-218); *supported = 0: host reader needed
+// FASTA bytes in HBM -> the text T of `-f` mode (kseq.h:177-218); *supported = 0: host reader needed.
+constexpr u32 PFP_FASTA_LINE_START = 2;   // state of the K0 line automaton at the start of a file
+// state / file_start: a piece of a file streamed in order (the automaton state carried across pieces)
 int pfp_fasta_device(pfpb200_ctx *ctx, const u8 *d_file, u64 n, u8 **d_text, u64 *n_text, int *supported,
-                     bool held);
+                     bool held, u32 *state = nullptr, bool file_start = true);
+
+// ---- the streamed parse of a file larger than the device (pfp_chunked.cu) -------------------------------------
+// pfpb200_parse_file in chunks of budget / 8 new bytes against one dictionary; *chunks = how many
+int pfp_parse_file_streamed(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, pfpb200_stats *stats,
+                            u64 budget, u64 *chunks);
 
 // ---- sharded parsing building blocks ------------------------------------------------------------------------
 int pfp_gather_word_fp(pfpb200_ctx *ctx, const DictArrays &D, const PhraseArrays &ph, u64 *wfpa,

@@ -120,7 +120,7 @@ class PfpFiles:
 _lib = None
 
 SYMBOLS = ["pfpb200_create", "pfpb200_destroy", "pfpb200_set_stream", "pfpb200_parse_device",
-           "pfpb200_parse_host", "pfpb200_parse_file", "pfpb200_fasta_extract", "pfpb200_fasta_extract_device",
+           "pfpb200_parse_host", "pfpb200_parse_file", "pfpb200_parse_plan", "pfpb200_fasta_extract", "pfpb200_fasta_extract_device",
            "pfpb200_read_input",
            "pfpb200_free_host",
            "pfpb200_scan_triggers", "pfpb200_memcpy_d2h", "pfpb200_strerror",
@@ -159,6 +159,8 @@ def load_library():
     L.pfpb200_parse_host.restype = C.c_int
     L.pfpb200_parse_file.argtypes = [vp, C.c_char_p, C.POINTER(Opts), C.POINTER(Stats)]
     L.pfpb200_parse_file.restype = C.c_int
+    L.pfpb200_parse_plan.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
+    L.pfpb200_parse_plan.restype = C.c_int
     L.pfpb200_fasta_extract.argtypes = [vp, u64, vp, C.POINTER(C.c_int)]
     L.pfpb200_fasta_extract.restype = u64
     L.pfpb200_scan_triggers.argtypes = [vp, vp, u64, u64, u64, u64, u32, u32, C.POINTER(vp),
@@ -314,10 +316,20 @@ class Scanner:
         return out
 
     # -- file in, files out: what `bigbwt` runs -------------------------------------------------------
-    def parse_file(self, path, w=10, p=100, sai=False, fasta=False, compress=False, nseg=0) -> dict:
-        o = Opts(w, p, _flags(sai, fasta, compress), nseg)
+    def parse_file(self, path, w=10, p=100, sai=False, fasta=False, compress=False, nseg=0, verify=False) -> dict:
+        """Writes <path>.dict|.dicz .occ .parse .last [.sai]; returns the stats and, under "chunks" and
+        "peak_device_bytes", how the call ran (chunks 0: one-shot; see pfpb200_parse_plan)."""
+        o = Opts(w, p, _flags(sai, fasta, compress, verify=verify), nseg)
         self._check(self.L.pfpb200_parse_file(self.h, os.fsencode(path), C.byref(o), C.byref(self.stats)))
-        return self.stats.as_dict()
+        d = self.stats.as_dict()
+        d["chunks"], d["peak_device_bytes"] = self.parse_plan()
+        return d
+
+    def parse_plan(self):
+        """(chunks, peak device bytes) of the last parse_file call; chunks 0: the one-shot path."""
+        c, pk = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.L.pfpb200_parse_plan(self.h, C.byref(c), C.byref(pk)))
+        return c.value, pk.value
 
     # -- the stage after the parse: bwtparse (bwtparse.c) ---------------------------------------------
     def bwtparse_device(self, parse_ptr: int, n: int, last_ptr: int, sai_ptr: int | None = None) -> BwtParseResult:

@@ -31,7 +31,9 @@ extern "C" {
                                     613-617), a phrase > 2^32-1 bytes, or >= 2^31-2 phrases on ONE
                                     GPU (the reference allows 2^32-2 phrases, bigbwt:110-114; here
                                     bit 31 of the per-phrase word id marks ids still being created,
-                                    so a text with more phrases needs two or more shards)        */
+                                    so a text with more phrases needs two or more shards, or the
+                                    chunks of a streamed pfpb200_parse_file, where the limit applies
+                                    per chunk and the total may reach 2^32-2)                    */
 #define PFPB200_E_COLLISION  -6  /* fingerprint collision detected (newscan.cpp:282-286)         */
 #define PFPB200_E_INTERNAL   -7  /* an invariant of the pipeline was violated                    */
 
@@ -123,6 +125,18 @@ int pfpb200_parse_host(pfpb200_ctx *ctx, const uint8_t *text, uint64_t n_text,
  * back into the files the same way. */
 int pfpb200_parse_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts,
                        pfpb200_stats *stats);
+
+/* How the last pfpb200_parse_file call ran.  An input whose one-shot footprint (about 1.5 to 4 device
+ * bytes per input byte, DESIGN.md §6b) exceeds the device memory available to the call is parsed in
+ * chunks instead: the text streams through HBM against one dictionary that lives across the chunks,
+ * .parse is written as global word ids and rewritten with ranks at the end, like the reference's
+ * .parse_old and remapParse (newscan.cpp:443-466).  The outputs are the same bytes; the text is then
+ * bounded by the disk, the dictionary (as the reference's std::map by RAM) by one GPU.  The per-GPU
+ * limit of 2^31-2 phrases applies per chunk, so a streamed parse reaches the reference's 2^32-2.
+ * PFPB200_PARSE_BUDGET=<bytes> in the environment replaces the available-memory figure (routing and
+ * chunk size: budget / 8 new bytes per chunk).  *chunks = 0 for the one-shot path; *peak_device_bytes
+ * = the high-water mark of the context's device arena during the call. */
+int pfpb200_parse_plan(const pfpb200_ctx *ctx, uint64_t *chunks, uint64_t *peak_device_bytes);
 
 /* kseq-equivalent FASTA/FASTQ extraction + toupper + validity cut (kseq.h:177-218,
  * newscan.cpp:338-349), host side.  `out` must hold n bytes; returns text length and sets
