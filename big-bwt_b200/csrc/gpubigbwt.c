@@ -161,6 +161,11 @@ int main(int argc, char **argv) {
     printf("GPU: parse %.3f ms, bwtparse %.3f ms (%u rounds), pfbwt %.3f ms (suffix sort %.3f in %u rounds, BWT%s %.3f)\n",
            st.ms_total, bp.ms_total, bp.rounds, r.ms_total, r.ms_sa, r.rounds, flags ? " + SA" : "", r.ms_fill);
     printf("File read: %.3f s; stages after the parse + file write: %.3f s\n", st.sec_read, st.sec_write);
+    uint64_t chunks = 0, windows = 0, parse_peak = 0, pfbwt_peak = 0;
+    pfpb200_parse_plan(ctx, &chunks, &parse_peak);
+    pfpb200_pfbwt_plan(ctx, &windows, &pfbwt_peak);
+    printf("Plan: parse %llu chunks (0: in one piece), peak %.3f GB; pfbwt %llu windows, peak %.3f GB\n",
+           (unsigned long long)chunks, (double)parse_peak * 1e-9, (unsigned long long)windows, (double)pfbwt_peak * 1e-9);
     printf("==== Elapsed time: %.3f wall clock seconds\n",
            (double)(t1.tv_sec - t0.tv_sec) + 1e-9 * (double)(t1.tv_nsec - t0.tv_nsec));
     pfpb200_destroy(ctx);

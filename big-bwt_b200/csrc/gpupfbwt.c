@@ -94,6 +94,12 @@ int main(int argc, char **argv) {
     printf("Hard bwt chars: %llu\n", (unsigned long long)r.hard);
     printf("GPU pfbwt: %.3f ms (dictionary suffix sort %.3f in %u doubling rounds, BWT%s %.3f), %u kernel launches\n",
            r.ms_total, r.ms_sa, r.rounds, flags ? " + SA" : "", r.ms_fill, r.launches);
+    if (ctx) {
+        uint64_t windows = 0, peak = 0;
+        pfpb200_pfbwt_plan(ctx, &windows, &peak);
+        printf("Plan: %llu output windows (1: in one piece), device peak %.3f GB\n", (unsigned long long)windows,
+               (double)peak * 1e-9);
+    }
     if (multi) {
         pfpb200_pfbwt_rank pr[PFPB200_MAX_RANKS];
         int k = pfpb200_multi_pfbwt_ranks(multi, pr, PFPB200_MAX_RANKS);

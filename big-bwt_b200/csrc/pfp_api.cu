@@ -516,28 +516,35 @@ static u64 input_bytes(const char *path, bool fasta, bool *ok) {
     return n;
 }
 
+// Routing of a file parse: the one-shot path for every input whose footprint fits the device memory
+// available to the call (free memory plus what the context's arena holds unused); the streamed path
+// otherwise.  PFPB200_PARSE_BUDGET=<bytes> replaces that figure (tests: megabyte inputs take the streamed path).
+static int parse_route(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, bool *streamed, u64 *budget) {
+    PFP_TRY(begin_call(ctx));
+    const char *ev = getenv("PFPB200_PARSE_BUDGET");
+    if (ev && atoll(ev) > 0) *budget = (u64)atoll(ev);
+    else {
+        size_t fr = 0, tot = 0;
+        PFP_CUDA(ctx, cudaMemGetInfo(&fr, &tot));
+        *budget = (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
+    }
+    bool ok = false;
+    const u64 in = input_bytes(path, (opts->flags & PFPB200_F_FASTA) != 0, &ok);
+    *streamed = ok && oneshot_estimate(in, (opts->flags & PFPB200_F_FASTA) != 0) > *budget;
+    return PFPB200_OK;
+}
+
 extern "C" int pfpb200_parse_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts,
                                   pfpb200_stats *stats) {
     PFP_TRY(check_opts(ctx, opts));
     if (!path) return pfp_fail(ctx, PFPB200_E_ARG, "null path");
     ctx->plan_chunks = 0;
     ctx->plan_peak = 0;
-    // Routing: the one-shot path for every input whose footprint fits the device memory available to
-    // the call (free memory plus what the context's arena holds unused); the streamed path otherwise.
-    // PFPB200_PARSE_BUDGET=<bytes> replaces that figure (tests: megabyte inputs take the streamed path).
-    PFP_TRY(begin_call(ctx));
+    bool streamed = false;
     u64 budget = 0;
-    const char *ev = getenv("PFPB200_PARSE_BUDGET");
-    if (ev && atoll(ev) > 0) budget = (u64)atoll(ev);
-    else {
-        size_t fr = 0, tot = 0;
-        PFP_CUDA(ctx, cudaMemGetInfo(&fr, &tot));
-        budget = (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
-    }
-    bool ok = false;
-    const u64 in = input_bytes(path, (opts->flags & PFPB200_F_FASTA) != 0, &ok);
+    PFP_TRY(parse_route(ctx, path, opts, &streamed, &budget));
     int rc;
-    if (ok && oneshot_estimate(in, (opts->flags & PFPB200_F_FASTA) != 0) > budget) {
+    if (streamed) {
         ctx->arena.peak = ctx->arena.in_use;
         u64 chunks = 0;
         rc = pfp_parse_file_streamed(ctx, path, opts, stats, budget, &chunks);
@@ -558,44 +565,78 @@ extern "C" int pfpb200_parse_plan(const pfpb200_ctx *ctx, uint64_t *chunks, uint
 }
 
 // `bigbwt <file> -w W -p P [-f] [-S | -s -e]` in one call (bigbwt:66-150 runs newscan, bwtparse and
-// pfbwt as three processes that hand each other files): the input streams into HBM, the three stages
-// run there, and only <path>.bwt (and .sa / .ssa / .esa) are written -- with keep_files != 0 also the
-// intermediate files the reference leaves behind with `bigbwt -k`.
+// pfbwt as three processes that hand each other files).  An input that fits the device streams into HBM,
+// the three stages run there, and only <path>.bwt (and .sa / .ssa / .esa) are written -- with keep_files
+// != 0 also the intermediate files the reference leaves behind with `bigbwt -k`.  An input that does not
+// fit (the rule of pfpb200_parse_file) goes through the files as the reference's stages do: the streamed
+// parse writes them, bwtparse reads them, and pfbwt reads .dict / .occ and takes the parse's BWT from
+// HBM.  Either way pfbwt writes its outputs in windows when they do not fit (DESIGN.md §6c).
 extern "C" int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, uint32_t pfbwt_flags,
                                    int keep_files, pfpb200_stats *stats, pfpb200_bwtparse_result *bp_out,
                                    pfpb200_pfbwt_result *res) {
     if (!ctx || !opts || !res) return PFPB200_E_ARG;
     if (opts->flags & PFPB200_F_COMPRESS) return pfp_fail(ctx, PFPB200_E_ARG, "bigbwt: -c stops after the parse, use pfpb200_parse_file");
+    PFP_TRY(check_opts(ctx, opts));
+    if (!path) return pfp_fail(ctx, PFPB200_E_ARG, "null path");
     pfpb200_opts o = *opts;
     o.flags |= PFPB200_F_SAI;                                  // the later stages take .sai whenever a suffix array is wanted
     o.nseg = 0;
+    ctx->plan_chunks = ctx->plan_peak = 0;
+    ctx->pb_windows = ctx->pb_peak = 0;
+    bool streamed = false;
+    u64 budget = 0;
+    PFP_TRY(parse_route(ctx, path, &o, &streamed, &budget));
     pfpb200_stats st;
-    pfpb200_outputs dv;
-    PFP_TRY(parse_file_impl(ctx, path, &o, &st, keep_files != 0, &dv));
-    if (stats) *stats = st;
-    const double t0 = wall_sec();
     pfpb200_bwtparse_result bp;
-    PFP_TRY(pfpb200_bwtparse_device(ctx, dv.parse, dv.n_phrases, dv.last, dv.sai, &bp));
-    if (bp_out) *bp_out = bp;
-    PFP_TRY(pfpb200_pfbwt_device(ctx, dv.dict, dv.dict_bytes, dv.occ, dv.n_distinct, bp.ilist, bp.bwlast, bp.bwsai,
-                                 bp.n_out, o.w, pfbwt_flags, res));
     char name[4096];
-    auto put = [&](const char *ext, const void *p, u64 bytes) -> int {
-        snprintf(name, sizeof(name), "%s.%s", path, ext);
-        return pfp_device_to_file(ctx, name, p, bytes);
-    };
-    if (keep_files) {
-        PFP_TRY(put("ilist", bp.ilist, bp.n_out * 4));
-        PFP_TRY(put("bwlast", bp.bwlast, bp.n_out));
-        PFP_TRY(put("bwsai", bp.bwsai, bp.n_out * PFP_IBYTES));
+    auto fname = [&](const char *ext) { snprintf(name, sizeof(name), "%s.%s", path, ext); return name; };
+    auto put = [&](const char *ext, const void *p, u64 bytes) -> int { return pfp_device_to_file(ctx, fname(ext), p, bytes); };
+    int rc = PFPB200_OK;
+    double t0 = 0;
+    PbInput in;
+    in.w = o.w;
+    in.flags = pfbwt_flags;
+    if (!streamed) {
+        pfpb200_outputs dv;
+        PFP_TRY(parse_file_impl(ctx, path, &o, &st, keep_files != 0, &dv));
+        ctx->plan_peak = ctx->arena.peak;
+        t0 = wall_sec();
+        PFP_TRY(pfpb200_bwtparse_device(ctx, dv.parse, dv.n_phrases, dv.last, dv.sai, &bp));
+        if (keep_files) {
+            PFP_TRY(put("ilist", bp.ilist, bp.n_out * 4));
+            PFP_TRY(put("bwlast", bp.bwlast, bp.n_out));
+            PFP_TRY(put("bwsai", bp.bwsai, bp.n_out * PFP_IBYTES));
+        }
+        in.d = dv.dict; in.N = dv.dict_bytes; in.occ = dv.occ; in.dwords = dv.n_distinct;
+    } else {
+        ctx->arena.peak = ctx->arena.in_use;
+        u64 chunks = 0;
+        rc = pfp_parse_file_streamed(ctx, path, &o, &st, budget, &chunks);
+        ctx->plan_chunks = chunks;
+        ctx->plan_peak = ctx->arena.peak;
+        pfp_release_scratch(ctx);                              // the parse's buffers go before the later stages
+        pfp_release_held(ctx);
+        t0 = wall_sec();
+        if (rc == PFPB200_OK) rc = pfpb200_bwtparse_file(ctx, path, 1, 0, &bp);
+        void *f[2] = {nullptr, nullptr};
+        u64 n[2] = {0, 0};
+        for (int k = 0; k < 2 && rc == PFPB200_OK; k++) rc = pb_read_file(ctx, path, k, &f[k], &n[k]);
+        in.d = static_cast<u8 *>(f[0]); in.N = n[0]; in.occ = static_cast<u32 *>(f[1]); in.dwords = n[1];
     }
-    PFP_TRY(put("bwt", res->bwt, res->n_bwt));
-    if (pfbwt_flags & PFPB200_PFBWT_SA) PFP_TRY(put("sa", res->sa, res->n_sa * PFP_IBYTES));
-    if (pfbwt_flags & PFPB200_PFBWT_SSA) PFP_TRY(put("ssa", res->ssa, res->n_ssa * 2 * PFP_IBYTES));
-    if (pfbwt_flags & PFPB200_PFBWT_ESA) PFP_TRY(put("esa", res->esa, res->n_esa * 2 * PFP_IBYTES));
-    if (stats) stats->sec_write += (float)(wall_sec() - t0);     // (includes the two later stages: they are milliseconds to a second)
+    if (rc == PFPB200_OK) {
+        if (stats) *stats = st;
+        if (bp_out) *bp_out = bp;
+        in.ilist = bp.ilist; in.bwlast = bp.bwlast; in.bwsai = bp.bwsai; in.psize = bp.n_out;
+        ctx->arena.peak = ctx->arena.in_use;                   // pfpb200_pfbwt_plan reports the pfbwt step's peak
+        rc = pb_to_files(ctx, in, path, res);
+    }
+    if (streamed && !keep_files) {                             // as `bigbwt` without -k
+        static const char *const inter[] = {"dict", "occ", "parse", "last", "sai", "ilist", "bwlast", "bwsai"};
+        for (const char *ext : inter) unlink(fname(ext));
+    }
+    if (rc == PFPB200_OK && stats) stats->sec_write += (float)(wall_sec() - t0);   // (includes the two later stages)
     pfp_release_scratch(ctx);
-    return PFPB200_OK;
+    return rc;
 }
 
 static int parse_file_impl(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, pfpb200_stats *stats,

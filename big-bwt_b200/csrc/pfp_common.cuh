@@ -78,6 +78,7 @@ struct pfpb200_ctx {
     u32 weak_fp = 0;               // PFPB200_TEST_WEAK_FP=1 (tests): 2-bit fingerprints, so that PFPB200_F_VERIFY has collisions to catch
     double dedup_ratio = 0.0;      // distinct words / phrases of the previous parse (table sizing hint)
     u64 plan_chunks = 0, plan_peak = 0;   // pfpb200_parse_plan: chunks (0: one-shot) and arena peak of the last parse_file
+    u64 pb_windows = 0, pb_peak = 0;      // pfpb200_pfbwt_plan: output windows and arena peak of the last pfbwt file call
     char err[512] = {0};
     std::vector<void *> scratch;   // freed at the end of every call
     std::vector<void *> held;      // outputs: freed at the start of the next call / destroy

@@ -33,11 +33,30 @@
 #include "pfp_stages.cuh"
 #include <errno.h>
 #include <fcntl.h>
+#include <stdlib.h>
 #include <sys/stat.h>
 #include <unistd.h>
 
 constexpr u64 PB_BATCH = (u64)1 << 30;          // occurrences sorted at once in the hard groups
 constexpr u32 PB_BIG = 512;                     // easy members with more occurrences get a CTA instead of a thread
+
+// Device bytes that the output of c BWT chars with at most h hard occurrences takes, from the allocations
+// of pb_window and pb_samples: per char its byte and, with -S / -s / -e, its 5-byte SA value; then, one
+// after the other, the merge of the hard occurrences (u64 key and u32 value, twice for the sort's
+// ping-pong: 24, and the sort's digit histograms, 256 u32 per 2048 pairs: 0.5; at most one batch of
+// PB_BATCH at a time) and, with -s / -e, the run samples (u32 flag and u64 scan: 12, and at most one
+// 10-byte sample per char).  One byte per char on top covers the easy members' CTA list (4 B per 512
+// chars) and the scans' tile sums.  A window holds at most min(c, h) hard occurrences.
+constexpr u64 PB_MERGE_BYTES = 2 * (8 + 4) + 1;
+constexpr u64 PB_SAMPLE_BYTES = 4 + 8 + 2 * PFP_IBYTES;
+static u64 pb_out_bytes(u64 c, u64 h, u32 flags) {
+    const bool want_sa = (flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
+    const bool samples = (flags & (PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
+    u64 m = h < c ? h : c;
+    if (m > PB_BATCH) m = PB_BATCH;
+    const u64 merge = PB_MERGE_BYTES * m, sample = samples ? PB_SAMPLE_BYTES * c : 0;
+    return c * (2 + (want_sa ? PFP_IBYTES : 0)) + (merge > sample ? merge : sample);
+}
 
 __global__ void __launch_bounds__(PB_T) pb_flags_k(const u8 *__restrict__ d, u64 N, u8 *__restrict__ flag) {
     const u64 t = (u64)blockIdx.x * PB_T + threadIdx.x;
@@ -219,14 +238,15 @@ __global__ void __launch_bounds__(PB_T) pb_hard_k(const u32 *__restrict__ cnt, c
     hcnt[k] = (!alone && (want_sa || mixed[g])) ? cnt[k] : 0u;
 }
 
-// members that need no merge: a whole word (chars from .bwlast, :155-203), or one char for all
+// members that need no merge: a whole word (chars from .bwlast, :155-203), or one char for all; slots
+// [ka, kb) of a window whose chars start at BWT position base
 __global__ void __launch_bounds__(PB_T) pb_easy_k(PbView v, const u32 *__restrict__ cnt, const u32 *__restrict__ hcnt,
                                                   const u64 *__restrict__ off, const u32 *__restrict__ ilist,
                                                   const u8 *__restrict__ bwlast, const u8 *__restrict__ bwsai,
-                                                  u8 *__restrict__ bwt, u8 *__restrict__ sa5, u32 *__restrict__ big,
-                                                  u32 *__restrict__ big_n, u32 big_cap) {
-    const u64 k = (u64)blockIdx.x * PB_T + threadIdx.x;
-    if (k >= v.N || cnt[k] == 0 || hcnt[k] != 0) return;
+                                                  u64 ka, u64 kb, u64 base, u8 *__restrict__ bwt, u8 *__restrict__ sa5,
+                                                  u32 *__restrict__ big, u32 *__restrict__ big_n, u32 big_cap) {
+    const u64 k = ka + (u64)blockIdx.x * PB_T + threadIdx.x;
+    if (k >= kb || cnt[k] == 0 || hcnt[k] != 0) return;
     u32 word, len; bool full; u8 c;
     pb_member(v, k, word, len, full, c);
     const u32 n = cnt[k];
@@ -235,7 +255,7 @@ __global__ void __launch_bounds__(PB_T) pb_easy_k(PbView v, const u32 *__restric
         if (i < big_cap) big[i] = (u32)k;
         return;
     }
-    const u64 o = off[k];
+    const u64 o = off[k] - base;
     const u32 is = v.istart[word] + 1u;                              // ilist[0] is the end symbol's entry (:376-383)
     for (u32 j = 0; j < n; j++) {
         const u32 ip = (full || sa5) ? ilist[is + j] : 0u;
@@ -249,7 +269,7 @@ __global__ void __launch_bounds__(PB_T) pb_easy_k(PbView v, const u32 *__restric
 __global__ void __launch_bounds__(PB_T) pb_easy_big_k(PbView v, const u32 *__restrict__ big, const u32 *__restrict__ big_n,
                                                       u32 big_cap, const u32 *__restrict__ cnt, const u64 *__restrict__ off,
                                                       const u32 *__restrict__ ilist, const u8 *__restrict__ bwlast,
-                                                      const u8 *__restrict__ bwsai, u8 *__restrict__ bwt,
+                                                      const u8 *__restrict__ bwsai, u64 base, u8 *__restrict__ bwt,
                                                       u8 *__restrict__ sa5) {
     const u32 nbig = min(*big_n, big_cap);
     for (u32 b = blockIdx.x; b < nbig; b += gridDim.x) {
@@ -257,7 +277,7 @@ __global__ void __launch_bounds__(PB_T) pb_easy_big_k(PbView v, const u32 *__res
         u32 word, len; bool full; u8 c;
         pb_member(v, k, word, len, full, c);
         const u32 n = cnt[k];
-        const u64 o = off[k];
+        const u64 o = off[k] - base;
         const u32 is = v.istart[word] + 1u;
         for (u32 j = threadIdx.x; j < n; j += PB_T) {
             const u32 ip = (full || sa5) ? ilist[is + j] : 0u;
@@ -284,44 +304,47 @@ __global__ void __launch_bounds__(PB_T) pb_gen_k(PbView v, const u32 *__restrict
     }
 }
 
+// the sorted occurrences of a batch to their BWT positions, less the window's first position base
 __global__ void __launch_bounds__(PB_T) pb_scatter_k(PbView v, const u64 *__restrict__ key, const u32 *__restrict__ val,
                                                      u64 ne, u64 e0, u32 g0, const u32 *__restrict__ first,
                                                      const u64 *__restrict__ off, const u64 *__restrict__ hoff,
-                                                     const u8 *__restrict__ bwsai, u8 *__restrict__ bwt,
+                                                     const u8 *__restrict__ bwsai, u64 base, u8 *__restrict__ bwt,
                                                      u8 *__restrict__ sa5) {
     const u64 e = (u64)blockIdx.x * PB_T + threadIdx.x;
     if (e >= ne) return;
     const u64 kk = key[e];
     const u32 k = val[e], f = first[(u32)(kk >> 32) + g0];
-    const u64 pos = off[f] + (e0 + e - hoff[f]);
+    const u64 pos = off[f] - base + (e0 + e - hoff[f]);
     u32 word, len; bool full; u8 c;
     pb_member(v, k, word, len, full, c);
     bwt[pos] = c;
     if (sa5) pb_put5(sa5, pos, pb_get5(bwsai, (u32)kk) - len);
 }
 
-// the next batch of hard groups: out = {kb, hoff[kb], group of slot ka, groups in [ka, kb)} with [ka, kb) =
-// as many whole groups as fit into `cap` occurrences, at least one (hoff[0..N] is non-decreasing)
-__global__ void pb_batch_k(const u64 *__restrict__ hoff, const u32 *__restrict__ gscan, const u8 *__restrict__ newgrp,
-                           const u32 *__restrict__ first, u64 ngroups, u64 ka, u64 N, u64 cap, u64 *__restrict__ out) {
-    const u64 target = hoff[ka] + cap;
-    u64 kb = N;
-    if (hoff[N] > target) {
-        u64 a = ka, b = N;                                       // first index with hoff > target
+// The next run of whole groups of slots [ka, end) (end: a group start or the last slot + 1) that fits
+// into `cap` items of a scan acc[0..end] (non-decreasing): the hard occurrences of a merge batch (hoff),
+// or the chars of a window (off).  out = {kb, acc[kb], group of slot ka, groups in [ka, kb)}, at least one
+// group: a group larger than cap is taken whole.
+__global__ void pb_batch_k(const u64 *__restrict__ acc, const u32 *__restrict__ gscan, const u8 *__restrict__ newgrp,
+                           const u32 *__restrict__ first, u64 ngroups, u64 ka, u64 end, u64 cap, u64 *__restrict__ out) {
+    const u64 target = acc[ka] + cap;
+    u64 kb = end;
+    if (acc[end] > target) {
+        u64 a = ka, b = end;                                     // first index with acc > target
         while (a < b) {
             const u64 m = (a + b) >> 1;
-            if (hoff[m] <= target) a = m + 1; else b = m;
+            if (acc[m] <= target) a = m + 1; else b = m;
         }
-        const u64 kl = a - 1;                                    // >= ka: hoff[ka] <= target
+        const u64 kl = a - 1;                                    // >= ka: acc[ka] <= target
         const u64 g = gscan[kl] + newgrp[kl] - 1u;
         kb = first[g];
-        if (kb <= ka) kb = g + 1 < ngroups ? first[g + 1] : N;   // one group larger than the batch: take it whole
+        if (kb <= ka) kb = g + 1 < ngroups ? first[g + 1] : end;   // one group larger than cap: take it whole
     }
     const u64 ga = gscan[ka] + newgrp[ka] - 1u;
     out[0] = kb;
-    out[1] = hoff[kb];
+    out[1] = acc[kb];
     out[2] = ga;
-    out[3] = kb < N ? gscan[kb] + newgrp[kb] - 1u - ga : ngroups - ga;
+    out[3] = gscan[kb - 1] + newgrp[kb - 1] - ga;                // kb > ka
 }
 
 // sampled suffix array: flag[i] = 1 at the first (start) / last (end) position of every run of the BWT;
@@ -352,7 +375,7 @@ const char *pb_arg_error(u32 w, u32 flags) {
     return nullptr;
 }
 
-static int pb_read_file(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count) {
+int pb_read_file(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count) {
     static const char *const ext[5] = {"dict", "occ", "ilist", "bwlast", "bwsai"};
     char name[4096];
     snprintf(name, sizeof(name), "%s.%s", base, ext[k]);
@@ -424,39 +447,66 @@ int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W) {
     return PFPB200_OK;
 }
 
-// count -> scans -> first / mixed / hard -> easy / easy-big -> hard batches
+// the plan over all n slots: count -> scans -> first / mixed / hard
 template <class Slots>
-int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
-            PbEmit *E) {
+int pb_plan(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, u8 *newgrp, u32 *gscan, PbPlan *P) {
     const bool want_sa = (in.flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
-    uint2 *mrec = nullptr;
-    u16 *mc = nullptr;
-    u32 *cnt = nullptr, *hcnt = nullptr, *first = nullptr;
-    u8 *mixed = nullptr;
-    u64 *off = nullptr, *hoff = nullptr;
-    PFP_TRY(pfp_alloc_t(ctx, &mrec, n));
-    PFP_TRY(pfp_alloc_t(ctx, &mc, n));
-    PFP_TRY(pfp_alloc_t(ctx, &cnt, n));
-    PFP_TRY(pfp_alloc_t(ctx, &hcnt, n));
-    PFP_TRY(pfp_alloc_t(ctx, &off, n + 1));
-    PFP_TRY(pfp_alloc_t(ctx, &hoff, n + 1));
-    const PbView V{in.d, W.wid, in.occ, W.istart, W.wend, mrec, mc, n, in.w};
-    // ---- ranges of the BWT, easy members ----
-    PB_LAUNCH(ctx, n, pb_count_k<Slots>, V, sl, cnt, newgrp);
+    P->n = n;
+    P->newgrp = newgrp;
+    P->gscan = gscan;
+    PFP_TRY(pfp_alloc_t(ctx, &P->mrec, n));
+    PFP_TRY(pfp_alloc_t(ctx, &P->mc, n));
+    PFP_TRY(pfp_alloc_t(ctx, &P->cnt, n));
+    PFP_TRY(pfp_alloc_t(ctx, &P->hcnt, n));
+    PFP_TRY(pfp_alloc_t(ctx, &P->off, n + 1));
+    PFP_TRY(pfp_alloc_t(ctx, &P->hoff, n + 1));
+    const PbView V{in.d, W.wid, in.occ, W.istart, W.wend, P->mrec, P->mc, n, in.w};
+    PB_LAUNCH(ctx, n, pb_count_k<Slots>, V, sl, P->cnt, newgrp);
     PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, newgrp, gscan, n, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
-    PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, cnt, off, n, &ctx->d_flags[2]));
+    PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, P->cnt, P->off, n, &ctx->d_flags[2]));
+    PFP_CUDA(ctx, cudaMemcpyAsync(&P->off[n], &ctx->d_flags[2], sizeof(u64), cudaMemcpyDeviceToDevice, ctx->stream));
     PFP_TRY(pb_sync_read(ctx, 1, 2));
-    const u64 ngroups = E->ngroups = (u32)ctx->h_flags[1], chars = E->chars = ctx->h_flags[2];
-    PFP_TRY(pfp_alloc_t(ctx, &first, ngroups + 1));
-    PFP_TRY(pfp_alloc_t(ctx, &mixed, ngroups + 1));
-    PFP_CUDA(ctx, cudaMemsetAsync(mixed, 0, ngroups + 1, ctx->stream));
-    PB_LAUNCH(ctx, n, pb_first_k, newgrp, gscan, n, first);
-    PB_LAUNCH(ctx, n, pb_mixed_k, V, newgrp, gscan, first, mixed);
-    PB_LAUNCH(ctx, n, pb_hard_k, cnt, newgrp, gscan, mixed, n, want_sa ? 1 : 0, hcnt);
-    PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, hcnt, hoff, n, &ctx->d_flags[3]));
-    PFP_CUDA(ctx, cudaMemcpyAsync(&hoff[n], &ctx->d_flags[3], sizeof(u64), cudaMemcpyDeviceToDevice, ctx->stream));
+    const u64 ngroups = P->ngroups = (u32)ctx->h_flags[1];
+    P->chars = ctx->h_flags[2];
+    PFP_TRY(pfp_alloc_t(ctx, &P->first, ngroups + 1));
+    PFP_TRY(pfp_alloc_t(ctx, &P->mixed, ngroups + 1));
+    PFP_CUDA(ctx, cudaMemsetAsync(P->mixed, 0, ngroups + 1, ctx->stream));
+    PB_LAUNCH(ctx, n, pb_first_k, newgrp, gscan, n, P->first);
+    PB_LAUNCH(ctx, n, pb_mixed_k, V, newgrp, gscan, P->first, P->mixed);
+    PB_LAUNCH(ctx, n, pb_hard_k, P->cnt, newgrp, gscan, P->mixed, n, want_sa ? 1 : 0, P->hcnt);
+    PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, P->hcnt, P->hoff, n, &ctx->d_flags[3]));
+    PFP_CUDA(ctx, cudaMemcpyAsync(&P->hoff[n], &ctx->d_flags[3], sizeof(u64), cudaMemcpyDeviceToDevice, ctx->stream));
     PFP_TRY(pb_sync_read(ctx, 3, 1));
-    const u64 n_hard = E->n_hard = ctx->h_flags[3];
+    P->n_hard = ctx->h_flags[3];
+    return PFPB200_OK;
+}
+int pb_window_end(pfpb200_ctx *ctx, const PbPlan &P, u64 ka, u64 cap, u64 *kb, u64 *chars_end) {
+    pb_batch_k<<<1, 1, 0, ctx->stream>>>(P.off, P.gscan, P.newgrp, P.first, P.ngroups, ka, P.n, cap, &ctx->d_flags[12]);
+    PFP_LAUNCHED(ctx);
+    PFP_TRY(pb_sync_read(ctx, 12, 2));
+    *kb = ctx->h_flags[12];
+    *chars_end = ctx->h_flags[13];
+    return PFPB200_OK;
+}
+
+// easy / easy-big -> hard batches, over the slots [ka, kb) of one window
+int pb_window(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 ka, u64 kb, u64 hcap,
+              bool held, PbEmit *E) {
+    const bool want_sa = (in.flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
+    const PbView V{in.d, W.wid, in.occ, W.istart, W.wend, P.mrec, P.mc, P.n, in.w};
+    // the window's first and last char and hard occurrence
+    u64 *h = &ctx->h_flags[12];
+    PFP_CUDA(ctx, cudaMemcpyAsync(&h[0], &P.off[ka], sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+    PFP_CUDA(ctx, cudaMemcpyAsync(&h[1], &P.off[kb], sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+    PFP_CUDA(ctx, cudaMemcpyAsync(&h[2], &P.hoff[ka], sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+    PFP_CUDA(ctx, cudaMemcpyAsync(&h[3], &P.hoff[kb], sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
+    PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const u64 base = h[0], chars = h[1] - h[0], e_end = h[3];
+    u64 ea = h[2];
+    E->base = base;
+    E->chars = chars;
+    E->n_hard = e_end - ea;
+    E->ngroups = P.ngroups;
     PFP_TRY(pfp_alloc_t(ctx, &E->bwt, chars, held));
     if (held) ctx->pb_out[0] = E->bwt;
     if (want_sa) {
@@ -469,24 +519,26 @@ int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64
     u32 *big = nullptr, *big_n = reinterpret_cast<u32 *>(&ctx->d_flags[6]);
     PFP_TRY(pfp_alloc_t(ctx, &big, big_cap));
     PFP_CUDA(ctx, cudaMemsetAsync(&ctx->d_flags[6], 0, sizeof(u64), ctx->stream));
-    PB_LAUNCH(ctx, n, pb_easy_k, V, cnt, hcnt, off, in.ilist, in.bwlast, in.bwsai, bwt, sa5, big, big_n, big_cap);
-    if (n) {
-        pb_easy_big_k<<<ctx->sm_count * 8, PB_T, 0, ctx->stream>>>(V, big, big_n, big_cap, cnt, off, in.ilist, in.bwlast,
-                                                                   in.bwsai, bwt, sa5);
+    PB_LAUNCH(ctx, kb - ka, pb_easy_k, V, P.cnt, P.hcnt, P.off, in.ilist, in.bwlast, in.bwsai, ka, kb, base, bwt, sa5, big,
+              big_n, big_cap);
+    if (kb > ka) {
+        pb_easy_big_k<<<ctx->sm_count * 8, PB_T, 0, ctx->stream>>>(V, big, big_n, big_cap, P.cnt, P.off, in.ilist,
+                                                                   in.bwlast, in.bwsai, base, bwt, sa5);
         PFP_LAUNCHED(ctx);
     }
     // ---- hard members: the merge of the ilist cursors as a sort, in batches ----
-    if (n_hard) {
-        const u64 cap = n_hard < PB_BATCH ? n_hard : PB_BATCH;
+    if (E->n_hard) {
+        const u64 lim = hcap < PB_BATCH ? hcap : PB_BATCH;
+        const u64 cap = lim ? lim : 1;
         u64 *hk0 = nullptr, *hk1 = nullptr;
         u32 *hv0 = nullptr, *hv1 = nullptr;
-        u64 ka = 0, ea = 0;                                    // (a single group may exceed the batch: the buffers grow)
+        u64 k = ka;                                            // (a single group may exceed the batch: the buffers grow)
         u64 buf = 0;
-        while (ka < n && ea < n_hard) {
-            pb_batch_k<<<1, 1, 0, ctx->stream>>>(hoff, gscan, newgrp, first, ngroups, ka, n, cap, &ctx->d_flags[4]);
+        while (k < kb && ea < e_end) {
+            pb_batch_k<<<1, 1, 0, ctx->stream>>>(P.hoff, P.gscan, P.newgrp, P.first, P.ngroups, k, kb, cap, &ctx->d_flags[4]);
             PFP_LAUNCHED(ctx);
             PFP_TRY(pb_sync_read(ctx, 4, 4));
-            const u64 kb = ctx->h_flags[4], eb = ctx->h_flags[5], ng = ctx->h_flags[7];
+            const u64 k2 = ctx->h_flags[4], eb = ctx->h_flags[5], ng = ctx->h_flags[7];
             const u32 g0 = (u32)ctx->h_flags[6];
             const u64 ne = eb - ea;
             if (ne >= 0xFFFFFFFEull) return pfp_fail(ctx, PFPB200_E_LIMIT, "pfbwt: one group of equal suffixes with 2^32 occurrences");
@@ -494,24 +546,37 @@ int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64
                 if (ne > buf) {
                     if (hk0) { PFP_TRY(pfp_free_now(ctx, hk0)); PFP_TRY(pfp_free_now(ctx, hk1)); PFP_TRY(pfp_free_now(ctx, hv0)); PFP_TRY(pfp_free_now(ctx, hv1)); }
                     buf = ne > cap ? ne : cap;
+                    if (buf > E->n_hard) buf = E->n_hard;
                     PFP_TRY(pfp_alloc_t(ctx, &hk0, buf));
                     PFP_TRY(pfp_alloc_t(ctx, &hk1, buf));
                     PFP_TRY(pfp_alloc_t(ctx, &hv0, buf));
                     PFP_TRY(pfp_alloc_t(ctx, &hv1, buf));
                 }
-                pb_gen_k<<<pfp_blocks(kb - ka, PB_T), PB_T, 0, ctx->stream>>>(V, hcnt, hoff, gscan, newgrp, in.ilist, ka, kb, ea, g0, hk0, hv0);
+                pb_gen_k<<<pfp_blocks(k2 - k, PB_T), PB_T, 0, ctx->stream>>>(V, P.hcnt, P.hoff, P.gscan, P.newgrp, in.ilist, k, k2, ea, g0, hk0, hv0);
                 PFP_LAUNCHED(ctx);
                 u64 *sk = nullptr;
                 u32 *sv = nullptr;
                 PFP_TRY(pfp_radix_sort_pairs(ctx, hk0, hv0, hk1, hv1, ne, 0, 32 + pb_bits(ng), &sk, &sv));
-                pb_scatter_k<<<pfp_blocks(ne, PB_T), PB_T, 0, ctx->stream>>>(V, sk, sv, ne, ea, g0, first, off, hoff, in.bwsai, bwt, sa5);
+                pb_scatter_k<<<pfp_blocks(ne, PB_T), PB_T, 0, ctx->stream>>>(V, sk, sv, ne, ea, g0, P.first, P.off, P.hoff,
+                                                                             in.bwsai, base, bwt, sa5);
                 PFP_LAUNCHED(ctx);
             }
-            ka = kb;
+            k = k2;
             ea = eb;
         }
+        PFP_TRY(pfp_free_now(ctx, hk0)); PFP_TRY(pfp_free_now(ctx, hk1));
+        PFP_TRY(pfp_free_now(ctx, hv0)); PFP_TRY(pfp_free_now(ctx, hv1));
     }
+    PFP_TRY(pfp_free_now(ctx, big));
     return PFPB200_OK;
+}
+
+template <class Slots>
+int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
+            PbEmit *E) {
+    PbPlan P;
+    PFP_TRY(pb_plan(ctx, in, W, sl, n, newgrp, gscan, &P));
+    return pb_window(ctx, in, W, P, 0, n, P.n_hard, held, E);
 }
 template int pb_emit<PbSplitSlots>(pfpb200_ctx *, const PbInput &, const PbWords &, PbSplitSlots, u64, bool, u8 *, u32 *,
                                    PbEmit *);
@@ -556,7 +621,132 @@ static void pb_drop_own_outputs(pfpb200_ctx *ctx) {
     pfp_release_scratch(ctx);
 }
 
-static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, pfpb200_pfbwt_result *res) {
+// The device memory the outputs of a file call may take once its plan is done: PFPB200_PFBWT_BUDGET=<bytes>,
+// or the free memory plus what the context's arena holds unused (as pfpb200_parse_file counts it).
+static int pb_budget(pfpb200_ctx *ctx, u64 *budget) {
+    const char *ev = getenv("PFPB200_PFBWT_BUDGET");
+    if (ev && atoll(ev) > 0) {
+        *budget = (u64)atoll(ev);
+        return PFPB200_OK;
+    }
+    size_t fr = 0, tot = 0;
+    PFP_CUDA(ctx, cudaMemGetInfo(&fr, &tot));
+    *budget = (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
+    return PFPB200_OK;
+}
+
+// appends host bytes to an output file at file_off
+static int pb_put_host(pfpb200_ctx *ctx, int fd, u64 file_off, const u8 *p, u64 bytes, const char *name) {
+    u64 done = 0;
+    while (done < bytes) {
+        const ssize_t r = pwrite(fd, p + done, bytes - done, (off_t)(file_off + done));
+        if (r <= 0) return pfp_fail(ctx, PFPB200_E_IO, "%s: write error: %s", name, strerror(errno));
+        done += (u64)r;
+    }
+    return PFPB200_OK;
+}
+
+// The outputs of a plan in windows of whole groups of at most cap chars (DESIGN.md §6c): each window's
+// chars and SA values go to <base>.bwt / .sa at their offsets, its run samples are appended to
+// <base>.ssa / .esa.  Samples across a window border: a window's first char knows the char in front of
+// it (-s); the last run end of a window (-e) waits on the host until the next window's first char shows
+// whether the run goes on.
+struct PbOutFiles {
+    int fd[4] = {-1, -1, -1, -1};              // bwt, sa, ssa, esa
+    char name[4][4096];
+    ~PbOutFiles() {
+        for (int i = 0; i < 4; i++)
+            if (fd[i] >= 0) close(fd[i]);
+    }
+};
+static int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 cap,
+                            const char *base, pfpb200_pfbwt_result *res, u64 *windows) {
+    static const char *const ext[4] = {"bwt", "sa", "ssa", "esa"};
+    const u32 want[4] = {0, PFPB200_PFBWT_SA, PFPB200_PFBWT_SSA, PFPB200_PFBWT_ESA};   // .bwt always
+    const u64 size[4] = {P.chars, (P.chars - 1) * PFP_IBYTES, 0, 0};   // .sa: no entry for BWT position 0
+    PbOutFiles F;
+    for (int i = 0; i < 4; i++) {
+        if (want[i] && !(in.flags & want[i])) continue;
+        snprintf(F.name[i], sizeof(F.name[i]), "%s.%s", base, ext[i]);
+        F.fd[i] = open(F.name[i], O_WRONLY | O_CREAT | O_TRUNC, 0666);
+        if (F.fd[i] < 0) return pfp_fail(ctx, PFPB200_E_IO, "%s: %s", F.name[i], strerror(errno));
+        if (size[i] && ftruncate(F.fd[i], (off_t)size[i]) != 0)
+            return pfp_fail(ctx, PFPB200_E_IO, "%s: %s", F.name[i], strerror(errno));
+    }
+    const u64 S2 = 2 * PFP_IBYTES;                            // one sample: (BWT position, SA value)
+    u64 ka = 0, n_s = 0, n_e = 0;
+    int prev = -1;                                           // last char of the windows so far (-1: none yet)
+    bool pending = false;                                    // the last run end so far, not yet written
+    u8 pend[2 * PFP_IBYTES];
+    *windows = 0;
+    while (ka < P.n) {
+        u64 kb = 0, cend = 0;
+        PFP_TRY(pb_window_end(ctx, P, ka, cap, &kb, &cend));
+        PbEmit E;
+        PFP_TRY(pb_window(ctx, in, W, P, ka, kb, cap, false, &E));
+        ++*windows;
+        const u64 n = E.chars;
+        if (n) {
+            u8 *cf = reinterpret_cast<u8 *>(&ctx->h_flags[9]), *cl = reinterpret_cast<u8 *>(&ctx->h_flags[10]);
+            PFP_CUDA(ctx, cudaMemcpyAsync(cf, E.bwt, 1, cudaMemcpyDeviceToHost, ctx->stream));
+            PFP_CUDA(ctx, cudaMemcpyAsync(cl, E.bwt + n - 1, 1, cudaMemcpyDeviceToHost, ctx->stream));
+            PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            const int c_first = *cf, c_last = *cl;
+            PFP_TRY(pfp_device_to_fd(ctx, F.fd[0], E.base, E.bwt, n, F.name[0]));
+            if (F.fd[1] >= 0) {
+                if (E.base == 0) PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], 0, E.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES, F.name[1]));
+                else PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], (E.base - 1) * PFP_IBYTES, E.sa5, n * PFP_IBYTES, F.name[1]));
+            }
+            u8 *out = nullptr;
+            u64 m = 0;
+            if (F.fd[2] >= 0) {
+                PFP_TRY(pb_samples(ctx, E, 0, prev, -1, E.base, false, &out, &m));
+                PFP_TRY(pfp_device_to_fd(ctx, F.fd[2], n_s * S2, out, m * S2, F.name[2]));
+                PFP_TRY(pfp_free_now(ctx, out));
+                n_s += m;
+            }
+            if (F.fd[3] >= 0) {
+                if (pending && c_first != prev) {
+                    PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
+                    n_e++;
+                }
+                // with no char behind the window its last position ends a run: m >= 1, the last one pending
+                PFP_TRY(pb_samples(ctx, E, 1, -1, -1, E.base, false, &out, &m));
+                PFP_TRY(pfp_device_to_fd(ctx, F.fd[3], n_e * S2, out, (m - 1) * S2, F.name[3]));
+                PFP_CUDA(ctx, cudaMemcpyAsync(pend, out + (m - 1) * S2, S2, cudaMemcpyDeviceToHost, ctx->stream));
+                PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+                PFP_TRY(pfp_free_now(ctx, out));
+                n_e += m - 1;
+                pending = true;
+            }
+            prev = c_last;
+        }
+        PFP_TRY(pfp_free_now(ctx, E.bwt));
+        PFP_TRY(pfp_free_now(ctx, E.sa5));
+        ka = kb;
+    }
+    if (pending) {
+        PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
+        n_e++;
+    }
+    for (int i = 0; i < 4; i++) {
+        const int fd = F.fd[i];
+        F.fd[i] = -1;
+        if (fd >= 0 && close(fd) != 0) return pfp_fail(ctx, PFPB200_E_IO, "%s: write error: %s", F.name[i], strerror(errno));
+    }
+    res->n_bwt = P.chars;
+    if (in.flags & PFPB200_PFBWT_SA) res->n_sa = P.chars - 1;
+    res->n_ssa = n_s;
+    res->n_esa = n_e;
+    return PFPB200_OK;
+}
+
+// out_base == null: the outputs stay in HBM, held by the context (pfpb200_pfbwt_device).  Otherwise they
+// are meant for the files <out_base>.*: held as well when they fit the device memory the call has once its
+// plan is done (the caller writes them), written here window by window when they do not (res->bwt ...
+// stay null).  *windows: windows the output took.
+static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, const char *out_base, pfpb200_pfbwt_result *res,
+                             u64 *windows) {
     memset(res, 0, sizeof(*res));
     const u64 N = in.N, dwords = in.dwords, psize = in.psize;
     const u32 w = in.w, flags = in.flags;
@@ -637,25 +827,45 @@ static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, pfpb200_pfbwt_
     PFP_CUDA(ctx, cudaEventRecord(evs[1], ctx->stream));
     // ---- 3. emission --------------------------------------------------------------------------------------------
     PFP_TRY(pfp_free_now(ctx, rank));                        // the ranks travel with the suffix array from here on
-    PbEmit E;
-    PFP_TRY(pb_emit(ctx, in, W, PbPackedSlots{sa}, N, true, flag, escan, &E));
-    // ---- 4. sampled suffix array: the entries at the starts / ends of the runs ----------------------------------------
-    u8 *ssa = nullptr, *esa = nullptr;
-    u64 n_ssa = 0, n_esa = 0;
-    if (flags & PFPB200_PFBWT_SSA) PFP_TRY(pb_samples(ctx, E, 0, -1, -1, 0, true, &ssa, &n_ssa));
-    if (flags & PFPB200_PFBWT_ESA) PFP_TRY(pb_samples(ctx, E, 1, -1, -1, 0, true, &esa, &n_esa));
+    PbPlan P;
+    PFP_TRY(pb_plan(ctx, in, W, PbPackedSlots{sa}, N, flag, escan, &P));
+    u64 cap = P.chars;
+    if (out_base) {              // one window when the whole output fits, else windows of the most chars that fit
+        u64 budget = 0;
+        PFP_TRY(pb_budget(ctx, &budget));
+        if (pb_out_bytes(P.chars, P.n_hard, flags) > budget) {
+            u64 lo = 0, hi = P.chars;                        // pb_out_bytes grows with c: the largest c that fits
+            while (lo < hi) {
+                const u64 mid = lo + (hi - lo + 1) / 2;
+                if (pb_out_bytes(mid, P.n_hard, flags) <= budget) lo = mid; else hi = mid - 1;
+            }
+            cap = lo;                                        // < P.chars; 0: one group per window
+        }
+    }
+    *windows = 1;
+    if (cap < P.chars) {
+        PFP_TRY(pb_write_windows(ctx, in, W, P, cap, out_base, res, windows));
+    } else {
+        PbEmit E;
+        PFP_TRY(pb_window(ctx, in, W, P, 0, N, P.n_hard, true, &E));
+        // ---- 4. sampled suffix array: the entries at the starts / ends of the runs ------------------------------------
+        u8 *ssa = nullptr, *esa = nullptr;
+        u64 n_ssa = 0, n_esa = 0;
+        if (flags & PFPB200_PFBWT_SSA) PFP_TRY(pb_samples(ctx, E, 0, -1, -1, 0, true, &ssa, &n_ssa));
+        if (flags & PFPB200_PFBWT_ESA) PFP_TRY(pb_samples(ctx, E, 1, -1, -1, 0, true, &esa, &n_esa));
+        res->bwt = E.bwt;
+        res->n_bwt = E.chars;
+        if (flags & PFPB200_PFBWT_SA) {                      // the .sa file has no entry for the first BWT char (:157-163)
+            res->sa = E.sa5 + PFP_IBYTES;
+            res->n_sa = E.chars - 1;
+        }
+        res->ssa = ssa; res->n_ssa = n_ssa;
+        res->esa = esa; res->n_esa = n_esa;
+    }
     PFP_CUDA(ctx, cudaEventRecord(evs[2], ctx->stream));
     PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    res->bwt = E.bwt;
-    res->n_bwt = E.chars;
-    if (flags & PFPB200_PFBWT_SA) {                          // the .sa file has no entry for the first BWT char (:157-163)
-        res->sa = E.sa5 + PFP_IBYTES;
-        res->n_sa = E.chars - 1;
-    }
-    res->ssa = ssa; res->n_ssa = n_ssa;
-    res->esa = esa; res->n_esa = n_esa;
     res->dict_bytes = N; res->dict_words = dwords; res->parse_size = psize;
-    res->easy = E.chars - E.n_hard; res->hard = E.n_hard;
+    res->easy = P.chars - P.n_hard; res->hard = P.n_hard;
     res->rounds = rounds;
     res->launches = ctx->launches - launches0;
     cudaEventElapsedTime(&res->ms_sa, evs[0], evs[1]);
@@ -664,17 +874,48 @@ static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, pfpb200_pfbwt_
     return PFPB200_OK;
 }
 
+// entry of the device and file calls: the outputs of the previous call go, the flags are cleared
+static int pb_begin(pfpb200_ctx *ctx) {
+    PFP_CUDA(ctx, cudaSetDevice(ctx->device));
+    pb_drop_own_outputs(ctx);
+    ctx->err[0] = 0;
+    PFP_CUDA(ctx, cudaMemsetAsync(ctx->d_flags, 0, 8 * sizeof(u64), ctx->stream));
+    return PFPB200_OK;
+}
+
 extern "C" int pfpb200_pfbwt_device(pfpb200_ctx *ctx, const uint8_t *d_dict, uint64_t dict_bytes, const uint32_t *d_occ,
                                     uint64_t n_words, const uint32_t *d_ilist, const uint8_t *d_bwlast,
                                     const uint8_t *d_bwsai, uint64_t parse_size, uint32_t w, uint32_t flags,
                                     pfpb200_pfbwt_result *res) {
     if (!ctx || !d_dict || !d_occ || !d_ilist || !d_bwlast || !res) return PFPB200_E_ARG;
-    PFP_CUDA(ctx, cudaSetDevice(ctx->device));
-    pb_drop_own_outputs(ctx);
-    ctx->err[0] = 0;
-    PFP_CUDA(ctx, cudaMemsetAsync(ctx->d_flags, 0, 8 * sizeof(u64), ctx->stream));
+    PFP_TRY(pb_begin(ctx));
     const PbInput in{d_dict, dict_bytes, d_occ, n_words, d_ilist, d_bwlast, d_bwsai, parse_size, w, flags};
-    const int rc = pfbwt_device_impl(ctx, in, res);
+    u64 windows = 0;
+    const int rc = pfbwt_device_impl(ctx, in, nullptr, res, &windows);
+    pfp_release_scratch(ctx);
+    return rc;
+}
+
+// the inputs (device pointers) -> <base>.bwt [.sa | .ssa .esa]: in one window when they fit, else in windows;
+// the plan of the call for pfpb200_pfbwt_plan
+int pb_to_files(pfpb200_ctx *ctx, const PbInput &in, const char *base, pfpb200_pfbwt_result *res) {
+    PFP_TRY(pb_begin(ctx));
+    u64 windows = 0;
+    int rc = pfbwt_device_impl(ctx, in, base, res, &windows);
+    char name[4096];
+    auto put = [&](const char *ext, const void *p, u64 bytes) {
+        if (rc != PFPB200_OK) return;
+        snprintf(name, sizeof(name), "%s.%s", base, ext);
+        rc = pfp_device_to_file(ctx, name, p, bytes);
+    };
+    if (rc == PFPB200_OK && res->bwt) {                           // held: the one-window run
+        put("bwt", res->bwt, res->n_bwt);
+        if (in.flags & PFPB200_PFBWT_SA) put("sa", res->sa, res->n_sa * PFP_IBYTES);
+        if (in.flags & PFPB200_PFBWT_SSA) put("ssa", res->ssa, res->n_ssa * 2 * PFP_IBYTES);
+        if (in.flags & PFPB200_PFBWT_ESA) put("esa", res->esa, res->n_esa * 2 * PFP_IBYTES);
+    }
+    ctx->pb_windows = windows;
+    ctx->pb_peak = ctx->arena.peak;
     pfp_release_scratch(ctx);
     return rc;
 }
@@ -687,22 +928,19 @@ extern "C" int pfpb200_pfbwt_file(pfpb200_ctx *ctx, const char *basename, uint32
     pfp_release_scratch(ctx);
     pfp_release_held(ctx);
     ctx->err[0] = 0;
+    ctx->pb_windows = ctx->pb_peak = 0;
+    ctx->arena.peak = ctx->arena.in_use;                              // pfpb200_pfbwt_plan reports this call's peak
     void *in[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     u64 n[5] = {0, 0, 0, 0, 0};
     PFP_TRY(pb_read_inputs(ctx, basename, flags, in, n));
-    int rc = pfpb200_pfbwt_device(ctx, static_cast<u8 *>(in[0]), n[0], static_cast<u32 *>(in[1]), n[1],
-                                  static_cast<u32 *>(in[2]), static_cast<u8 *>(in[3]), static_cast<u8 *>(in[4]), n[2], w,
-                                  flags, res);
-    char name[4096];
-    auto put = [&](const char *ext, const void *p, u64 bytes) {
-        if (rc != PFPB200_OK) return;
-        snprintf(name, sizeof(name), "%s.%s", basename, ext);
-        rc = pfp_device_to_file(ctx, name, p, bytes);
-    };
-    put("bwt", res->bwt, res->n_bwt);
-    if (flags & PFPB200_PFBWT_SA) put("sa", res->sa, res->n_sa * PFP_IBYTES);
-    if (flags & PFPB200_PFBWT_SSA) put("ssa", res->ssa, res->n_ssa * 2 * PFP_IBYTES);
-    if (flags & PFPB200_PFBWT_ESA) put("esa", res->esa, res->n_esa * 2 * PFP_IBYTES);
-    pfp_release_scratch(ctx);
-    return rc;
+    const PbInput pin{static_cast<u8 *>(in[0]), n[0], static_cast<u32 *>(in[1]), n[1], static_cast<u32 *>(in[2]),
+                      static_cast<u8 *>(in[3]), static_cast<u8 *>(in[4]), n[2], w, flags};
+    return pb_to_files(ctx, pin, basename, res);
+}
+
+extern "C" int pfpb200_pfbwt_plan(const pfpb200_ctx *ctx, uint64_t *windows, uint64_t *peak_device_bytes) {
+    if (!ctx) return PFPB200_E_ARG;
+    if (windows) *windows = ctx->pb_windows;
+    if (peak_device_bytes) *peak_device_bytes = ctx->pb_peak;
+    return PFPB200_OK;
 }

@@ -223,25 +223,57 @@ struct PbSplitSlots {
     __device__ __forceinline__ u32 grp(u64 k) const { return sa_grp[k]; }
 };
 
-// what the emission leaves: the BWT chars of the slots and, with -S / -s / -e, their suffix-array values
+// what the emission leaves: the BWT chars of the slots (of one window: chars [base, base + chars) of the
+// slice) and, with -S / -s / -e, their suffix-array values
 struct PbEmit {
     u8 *bwt = nullptr, *sa5 = nullptr;
-    u64 chars = 0, n_hard = 0, ngroups = 0;
+    u64 chars = 0, n_hard = 0, ngroups = 0, base = 0;
 };
+
+// The plan of the emission over all n slots (pb_plan): per slot its member record, occurrences, and
+// the start of its range in the BWT (off) and in the hard merge (hoff); per group its first slot and
+// whether its chars are mixed.  Every group owns one contiguous range of the BWT, so the output can be
+// produced for any run of whole groups [ka, kb) on its own: chars [off[ka], off[kb]) (pb_window).
+struct PbPlan {
+    uint2 *mrec = nullptr;      // [n] {word, suffix length}
+    u16 *mc = nullptr;          // [n] char in front | whole word << 8 | counts << 9
+    u32 *cnt = nullptr, *hcnt = nullptr;   // [n] occurrences, of them to merge
+    u64 *off = nullptr, *hoff = nullptr;   // [n + 1] exclusive scans of cnt / hcnt
+    u32 *first = nullptr;       // [ngroups + 1] first slot of every group
+    u8 *mixed = nullptr;        // [ngroups + 1]
+    u8 *newgrp = nullptr;       // [n] caller's scratch
+    u32 *gscan = nullptr;       // [n] caller's scratch: groups before the slot
+    u64 n = 0, ngroups = 0, chars = 0, n_hard = 0;
+};
+
 
 // the argument checks of pfbwt.x: the message of the first one that fails, or null
 const char *pb_arg_error(u32 w, u32 flags);
 // .dict .occ .ilist .bwlast [.bwsai when flags want a suffix array] into held buffers (in[k], n[k] entries
 // of PB_UNIT[k] bytes), their sizes checked against each other
 constexpr u64 PB_UNIT[5] = {1, 4, 4, 1, PFP_IBYTES};
+int pb_read_file(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count);   // one of them
 int pb_read_inputs(pfpb200_ctx *ctx, const char *base, u32 flags, void *in[5], u64 n[5]);
 int pb_sync_read(pfpb200_ctx *ctx, int slot, int n);   // h_flags[slot, slot + n) <- d_flags, then synchronise
 int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W);
-// the BWT chars (and SA values) of n sorted slots; newgrp / gscan: scratch of n entries; held: the
-// outputs are held buffers recorded in ctx->pb_out[0..1], otherwise scratch
+// the plan of the emission over n sorted slots; newgrp / gscan: scratch of n entries
+template <class Slots>
+int pb_plan(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, u8 *newgrp, u32 *gscan, PbPlan *P);
+// the end of the window of whole groups that starts at slot ka and holds at most cap chars (at least
+// one group: a larger group gets a window of its own); *chars_end = off[*kb]
+int pb_window_end(pfpb200_ctx *ctx, const PbPlan &P, u64 ka, u64 cap, u64 *kb, u64 *chars_end);
+// the BWT chars (and SA values) of the slots [ka, kb), a run of whole groups, into buffers of the window:
+// E->bwt[0, E->chars) = chars [off[ka], off[kb]); hard merge batches of at most min(PB_BATCH, hcap)
+// occurrences; held: the outputs are held buffers recorded in ctx->pb_out[0..1], otherwise scratch
+int pb_window(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 ka, u64 kb, u64 hcap,
+              bool held, PbEmit *E);
+// pb_plan and one window over all n slots
 template <class Slots>
 int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
             PbEmit *E);
+// pfpb200_pfbwt_file from the inputs in HBM: the outputs to <base>.bwt [.sa | .ssa .esa], in windows when they
+// do not fit the device memory left once the plan is done; records the plan for pfpb200_pfbwt_plan
+int pb_to_files(pfpb200_ctx *ctx, const PbInput &in, const char *base, pfpb200_pfbwt_result *res);
 // (BWT position + off, SA value) at the starts (at_end = 0) / ends of the runs of E's chars; prev / next:
 // the chars on either side of them (-1: none); held: the output is recorded in ctx->pb_out[2 + at_end]
 int pb_samples(pfpb200_ctx *ctx, const PbEmit &E, int at_end, int prev, int next, u64 off, bool held, u8 **out,

@@ -134,7 +134,7 @@ SYMBOLS = ["pfpb200_create", "pfpb200_destroy", "pfpb200_set_stream", "pfpb200_p
            "pfpb200_check_dict_order",
            "pfpb200_bwtparse_device", "pfpb200_bwtparse_host", "pfpb200_bwtparse_file",
            "pfpb200_unparse_device", "pfpb200_unparse_file",
-           "pfpb200_pfbwt_device", "pfpb200_pfbwt_file", "pfpb200_bigbwt_file",
+           "pfpb200_pfbwt_device", "pfpb200_pfbwt_file", "pfpb200_pfbwt_plan", "pfpb200_bigbwt_file",
            "pfpb200_launch_count", "pfpb200_last_error", "pfpb200_abi_version"]
 
 
@@ -161,6 +161,8 @@ def load_library():
     L.pfpb200_parse_file.restype = C.c_int
     L.pfpb200_parse_plan.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
     L.pfpb200_parse_plan.restype = C.c_int
+    L.pfpb200_pfbwt_plan.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
+    L.pfpb200_pfbwt_plan.restype = C.c_int
     L.pfpb200_fasta_extract.argtypes = [vp, u64, vp, C.POINTER(C.c_int)]
     L.pfpb200_fasta_extract.restype = u64
     L.pfpb200_scan_triggers.argtypes = [vp, vp, u64, u64, u64, u64, u32, u32, C.POINTER(vp),
@@ -376,14 +378,26 @@ class Scanner:
         return r
 
     def pfbwt_file(self, basename, w=10, flags=0) -> dict:
+        """Writes <basename>.bwt (+ .sa / .ssa / .esa); returns the result and, under "windows" and
+        "peak_device_bytes", how the outputs were written (windows 1: in one piece; see pfpb200_pfbwt_plan)."""
         self.L.pfpb200_pfbwt_file.argtypes = [C.c_void_p, C.c_char_p, C.c_uint32, C.c_uint32, C.POINTER(PfbwtResult)]
         self.L.pfpb200_pfbwt_file.restype = C.c_int
         r = PfbwtResult()
         self._check(self.L.pfpb200_pfbwt_file(self.h, os.fsencode(basename), w, flags, C.byref(r)))
-        return r.as_dict()
+        d = r.as_dict()
+        d["windows"], d["peak_device_bytes"] = self.pfbwt_plan()
+        return d
+
+    def pfbwt_plan(self):
+        """(windows, peak device bytes) of the pfbwt step of the last pfbwt_file / bigbwt_file call."""
+        n, pk = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.L.pfpb200_pfbwt_plan(self.h, C.byref(n), C.byref(pk)))
+        return n.value, pk.value
 
     def bigbwt_file(self, path, w=10, p=100, fasta=False, flags=0, keep=False) -> dict:
-        """The whole pipeline for a file: <path>.bwt (+ .sa / .ssa / .esa) written, stages in HBM."""
+        """The whole pipeline for a file: <path>.bwt (+ .sa / .ssa / .esa) written, stages in HBM, or through
+        the files for a text larger than the device.  The plans of the parse ("chunks") and of pfbwt
+        ("windows"), each with its "peak_device_bytes", are in the "parse" and "pfbwt" entries."""
         self.L.pfpb200_bigbwt_file.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(Opts), C.c_uint32, C.c_int,
                                                C.POINTER(Stats), C.POINTER(BwtParseResult), C.POINTER(PfbwtResult)]
         self.L.pfpb200_bigbwt_file.restype = C.c_int
@@ -391,7 +405,10 @@ class Scanner:
         bp, r = BwtParseResult(), PfbwtResult()
         self._check(self.L.pfpb200_bigbwt_file(self.h, os.fsencode(path), C.byref(o), flags, 1 if keep else 0,
                                                C.byref(self.stats), C.byref(bp), C.byref(r)))
-        return {"parse": self.stats.as_dict(), "bwtparse": bp.as_dict(), "pfbwt": r.as_dict()}
+        d = {"parse": self.stats.as_dict(), "bwtparse": bp.as_dict(), "pfbwt": r.as_dict()}
+        d["parse"]["chunks"], d["parse"]["peak_device_bytes"] = self.parse_plan()
+        d["pfbwt"]["windows"], d["pfbwt"]["peak_device_bytes"] = self.pfbwt_plan()
+        return d
 
     def bwt_of_text(self, text, w=10, p=100, flags=0):
         """The whole pipeline on one context, nothing leaves HBM in between: parse -> bwtparse -> pfbwt.

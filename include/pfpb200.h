@@ -391,9 +391,20 @@ int pfpb200_pfbwt_device(pfpb200_ctx *ctx, const uint8_t *d_dict, uint64_t dict_
                          uint64_t n_words, const uint32_t *d_ilist, const uint8_t *d_bwlast,
                          const uint8_t *d_bwsai /* NULL without SA flags */, uint64_t parse_size /* n_phrases + 1 */,
                          uint32_t w, uint32_t flags, pfpb200_pfbwt_result *res);
-/* `pfbwt.x -w W [-S | -s -e] <basename>`: reads .dict .occ .ilist .bwlast [.bwsai], writes .bwt [.sa | .ssa .esa] */
+/* `pfbwt.x -w W [-S | -s -e] <basename>`: reads .dict .occ .ilist .bwlast [.bwsai], writes .bwt [.sa | .ssa .esa].
+ * Once the suffix sort and the plan of the output are done, the outputs are held in HBM and written
+ * as a whole when they fit the device memory left to the call (free memory plus what the context's
+ * arena holds unused); res then carries device pointers, as pfpb200_pfbwt_device's does.  Otherwise
+ * they are produced in windows of whole groups of equal dictionary suffixes, each written to the files
+ * at its offset, and res carries counts and times with NULL device pointers.  The peak then depends on
+ * the dictionary, not on the text.  PFPB200_PFBWT_BUDGET=<bytes> in the environment replaces the
+ * available-memory figure (windows of the most chars whose output fits it). */
 int pfpb200_pfbwt_file(pfpb200_ctx *ctx, const char *basename, uint32_t w, uint32_t flags,
                        pfpb200_pfbwt_result *res);
+/* How the last pfpb200_pfbwt_file / pfpb200_bigbwt_file call wrote its outputs: *windows (1: in one
+ * piece from HBM) and *peak_device_bytes, the high-water mark of the context's device arena during the
+ * pfbwt step.  NULL outputs are skipped; ctx NULL: PFPB200_E_ARG. */
+int pfpb200_pfbwt_plan(const pfpb200_ctx *ctx, uint64_t *windows, uint64_t *peak_device_bytes);
 
 /* ---- the last stage on several GPUs ---------------------------------------------------------------- *
  * pfbwt over the ranks of a pfpb200_multi handle, for dictionaries of 4 GB and more: the same files as
@@ -421,7 +432,12 @@ int pfpb200_multi_pfbwt_ranks(const pfpb200_multi *m, pfpb200_pfbwt_rank *out, i
  * What `bigbwt <file> -w W -p P [-f] [-S | -s -e] [-k]` does with three processes and the files between
  * them (bigbwt:66-150): here the input streams into HBM, parse -> bwtparse -> pfbwt run there, and
  * <path>.bwt (and .sa / .ssa / .esa per pfbwt_flags) are written; keep_files != 0 (`-k`) also writes
- * the intermediate .dict .occ .parse .last .sai .ilist .bwlast .bwsai.  stats / bp may be NULL. */
+ * the intermediate .dict .occ .parse .last .sai .ilist .bwlast .bwsai.  stats / bp may be NULL (bp's
+ * device pointers stay valid until the next call).  A text that does not fit the device (the routing of
+ * pfpb200_parse_file, PFPB200_PARSE_BUDGET) takes the files: the streamed parse writes them, bwtparse
+ * reads them, pfbwt reads .dict / .occ, and without keep_files they are deleted at the end.  pfbwt
+ * writes as pfpb200_pfbwt_file does, in windows when its outputs do not fit (res then carries no
+ * device pointers).  pfpb200_parse_plan and pfpb200_pfbwt_plan report the two steps' plans. */
 int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, uint32_t pfbwt_flags,
                         int keep_files, pfpb200_stats *stats, pfpb200_bwtparse_result *bp,
                         pfpb200_pfbwt_result *res);
