@@ -80,6 +80,11 @@ static int multi_bigbwt(const char *path, const pfpb200_opts *opts, unsigned fla
             printf("GPU %d (rank %d): pfbwt %llu suffixes, %llu chars, sort %.3f ms, emit %.3f ms, write %.3f ms\n",
                    devices[g], g, (unsigned long long)pr[g].suffixes, (unsigned long long)pr[g].chars, pr[g].ms_sort,
                    pr[g].ms_emit, pr[g].ms_write);
+        uint64_t wn[PFPB200_MAX_RANKS];
+        k = pfpb200_multi_pfbwt_windows(multi, wn, PFPB200_MAX_RANKS);
+        printf("Plan: output windows per rank:");
+        for (int g = 0; g < k; g++) printf("%s%llu", g ? "," : " ", (unsigned long long)wn[g]);
+        printf("\n");
     }
     if (!keep) {
         char name[4096];

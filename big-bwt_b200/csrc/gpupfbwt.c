@@ -108,6 +108,11 @@ int main(int argc, char **argv) {
                    "write %.3f ms, peak %.3f GB\n", devices[g], g, (unsigned long long)pr[g].suffixes,
                    (unsigned long long)pr[g].chars, (unsigned long long)pr[g].hard, pr[g].ms_read, pr[g].ms_sort,
                    pr[g].ms_emit, pr[g].ms_write, (double)pr[g].peak_bytes * 1e-9);
+        uint64_t wn[PFPB200_MAX_RANKS];
+        k = pfpb200_multi_pfbwt_windows(multi, wn, PFPB200_MAX_RANKS);
+        printf("Plan: output windows per rank:");
+        for (int g = 0; g < k; g++) printf("%s%llu", g ? "," : " ", (unsigned long long)wn[g]);
+        printf("\n");
     }
     printf("==== Elapsed time: %.0f wall clock seconds\n", difftime(time(NULL), start));
     pfpb200_destroy(ctx);

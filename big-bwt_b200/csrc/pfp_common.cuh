@@ -167,6 +167,7 @@ void pfp_release_scratch(pfpb200_ctx *ctx);
 void pfp_release_held(pfpb200_ctx *ctx);
 void pfp_arena_destroy(pfpb200_ctx *ctx);
 int pfp_arena_consolidate(pfpb200_ctx *ctx);
+void pfp_arena_trim(pfpb200_ctx *ctx);   // slabs with nothing in use go back to the driver
 void pfp_arena_reserve(pfpb200_ctx *ctx, size_t bytes);
 
 template <typename T>

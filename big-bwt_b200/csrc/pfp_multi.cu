@@ -115,6 +115,7 @@ struct Rank {
     u64 *pb_rank = nullptr;               // my block of the rank array
     pfpb200_pfbwt_rank pb_stat;
     u32 pb_rounds = 0;
+    u64 pb_windows = 0, pb_ssa = 0, pb_esa = 0;   // output windows, run samples after the stitching
 };
 
 }  // namespace
@@ -906,10 +907,12 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
     auto agree = [&]() { bool f; m->bar.sum(0, !ok(), &f); return !f; };    // a barrier: true when no rank has failed
     auto run = [&](int rc) { if (rc != PFPB200_OK) multi_fail(m, g, rc, pfpb200_last_error(ctx)); };
     const double t0 = wall_sec();
-    double t_read = t0, t_sort = t0, t_emit = t0, t_write = t0;
+    double t_read = t0, t_sort = t0, t_plan = t0, t_write = t0;
+    char part[2][4096] = {{0}, {0}};                        // my part files of .ssa / .esa (empty: none)
     const u32 launches0 = ctx->launches;
     memset(&R.pb_stat, 0, sizeof(R.pb_stat));
     R.pb_rounds = 0;
+    R.pb_windows = R.pb_ssa = R.pb_esa = 0;
     R.pb_rank = nullptr;
     S = PmState();
     pfp_release_scratch(ctx);
@@ -1000,57 +1003,112 @@ void pfbwt_rank_main(pfpb200_multi *m, int g) {
         if (!alive) break;
         if (ok()) run(pm_sort_done(ctx, S));
         t_sort = wall_sec();
-        // ---- 4. emission on my slice ------------------------------------------------------------------------
-        if (ok()) run(pm_emit(ctx, S));
+        // ---- 4. the plan of my slice: once every rank has one, every offset is known ---------------------------
+        if (ok()) run(pm_plan(ctx, S));
+        pfp_arena_trim(ctx);                                // the sort's memory goes back for the others' windows
+        t_plan = wall_sec();
         if (!agree()) break;
+        const u32 flags = m->pb_flags;
         u64 off = 0, n_bwt = 0;
+        int share = 0;                                      // ranks listed on my device
         for (int q = 0; q < G; q++) {
-            if (q < g) off += m->r[q].pb.em.chars;
-            n_bwt += m->r[q].pb.em.chars;
+            if (q < g) off += m->r[q].pb.plan.chars;
+            n_bwt += m->r[q].pb.plan.chars;
+            share += m->r[q].device == R.device ? 1 : 0;
         }
-        int prev = -1, next = -1;                           // chars of the nearest non-empty pieces around mine
-        for (int q = g - 1; q >= 0 && prev < 0; q--) prev = m->r[q].pb.c_last;
-        for (int q = g + 1; q < G && next < 0; q++) next = m->r[q].pb.c_first;
-        if (ok() && (m->pb_flags & PFPB200_PFBWT_SSA)) run(pb_samples(ctx, S.em, 0, prev, next, off, false, &S.ssa, &S.n_ssa));
-        if (ok() && (m->pb_flags & PFPB200_PFBWT_ESA)) run(pb_samples(ctx, S.em, 1, prev, next, off, false, &S.esa, &S.n_esa));
-        t_emit = wall_sec();
-        if (!agree()) break;
-        // ---- 5. files: created by rank 0 at their final sizes, every rank writes its piece ---------------------
-        u64 off_s = 0, off_e = 0, tot_s = 0, tot_e = 0;
-        for (int q = 0; q < G; q++) {
-            if (q < g) { off_s += m->r[q].pb.n_ssa; off_e += m->r[q].pb.n_esa; }
-            tot_s += m->r[q].pb.n_ssa; tot_e += m->r[q].pb.n_esa;
-        }
+        u64 budget = 0;                                     // read now: the other ranks' plans are allocated and
+                                                            // their sorts' slabs released
+        run(pb_budget(ctx, share, &budget));
+        const u64 cap = pb_window_chars(S.plan, flags, budget);
+        // ---- 5. files: rank 0 creates them, every rank writes its piece in windows ----------------------------
         char name[4096];
         auto fname = [&](const char *ext) { snprintf(name, sizeof(name), "%s.%s", m->pb_base, ext); return name; };
         if (g == 0) {
             int bad = create_sized(m, fname("bwt"), n_bwt);
-            if (!bad && (m->pb_flags & PFPB200_PFBWT_SA)) bad = create_sized(m, fname("sa"), (n_bwt - 1) * PFP_IBYTES);
-            if (!bad && (m->pb_flags & PFPB200_PFBWT_SSA)) bad = create_sized(m, fname("ssa"), tot_s * 2 * PFP_IBYTES);
-            if (!bad && (m->pb_flags & PFPB200_PFBWT_ESA)) bad = create_sized(m, fname("esa"), tot_e * 2 * PFP_IBYTES);
+            if (!bad && (flags & PFPB200_PFBWT_SA)) bad = create_sized(m, fname("sa"), (n_bwt - 1) * PFP_IBYTES);
+            if (!bad && (flags & PFPB200_PFBWT_SSA)) bad = create_sized(m, fname("ssa"), 0);
+            if (!bad && (flags & PFPB200_PFBWT_ESA)) bad = create_sized(m, fname("esa"), 0);
             if (bad) multi_fail(m, g, PFPB200_E_IO, m->io_err);
         }
         if (!agree()) break;
-        const u64 n = S.em.chars;
-        run(piece_to_file(R, fname("bwt"), off, S.em.bwt, n));
-        if (ok() && (m->pb_flags & PFPB200_PFBWT_SA) && n) {
-            // the .sa file has no entry for BWT position 0
-            if (off == 0) run(piece_to_file(R, fname("sa"), 0, S.em.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES));
-            else run(piece_to_file(R, fname("sa"), (off - 1) * PFP_IBYTES, S.em.sa5, n * PFP_IBYTES));
+        // ranks sharing the device take their window's memory in one piece now that all have read their
+        // budgets, before any of them allocates a window
+        if (share > 1 && S.plan.n) pfp_arena_reserve(ctx, ctx->arena.total + pb_window_bytes(S.plan, flags, cap));
+        {
+            PbOutFiles F;
+            static const char *const ext[4] = {"bwt", "sa", "ssa", "esa"};
+            const u32 want[4] = {0, PFPB200_PFBWT_SA, PFPB200_PFBWT_SSA, PFPB200_PFBWT_ESA};
+            for (int i = 0; i < 4 && ok() && S.plan.n; i++) {   // a rank that owns nothing writes nothing
+                if (want[i] && !(flags & want[i])) continue;
+                if (i < 2) {
+                    snprintf(F.name[i], sizeof(F.name[i]), "%s.%s", m->pb_base, ext[i]);
+                    F.fd[i] = open(F.name[i], O_WRONLY);
+                } else {                                    // the run samples go to a part file of my own first
+                    snprintf(part[i - 2], sizeof(part[i - 2]), "%s.%s.%d", m->pb_base, ext[i], g);
+                    snprintf(F.name[i], sizeof(F.name[i]), "%s", part[i - 2]);
+                    F.fd[i] = open(F.name[i], O_RDWR | O_CREAT | O_TRUNC, 0666);
+                    if (F.fd[i] < 0) part[i - 2][0] = 0;
+                }
+                if (F.fd[i] < 0) run(pfp_fail(ctx, PFPB200_E_IO, "%s: %s", F.name[i], strerror(errno)));
+            }
+            if (ok() && S.plan.n) run(pb_write_windows(ctx, S.in, S.wd, S.plan, cap, F, off, &S.piece));
+            R.pb_windows = S.piece.windows;
+            for (int i = 0; i < 2; i++) {
+                const int fd = F.fd[i];
+                F.fd[i] = -1;
+                if (fd >= 0 && close(fd) != 0 && ok())
+                    run(pfp_fail(ctx, PFPB200_E_IO, "%s: write error: %s", F.name[i], strerror(errno)));
+            }
+            if (!agree()) break;
+            // ---- 6. run samples across the rank borders: a piece's first -s record goes when the previous
+            // non-empty piece ends with the same char, its last -e record when the next one starts with it
+            const u64 S2 = 2 * PFP_IBYTES;
+            u64 ns[PFPB200_MAX_RANKS], ne[PFPB200_MAX_RANKS], drop_s[PFPB200_MAX_RANKS], off_s = 0, off_e = 0;
+            for (int q = 0, prev = -1; q < G; q++) {
+                const PbPiece &pq = m->r[q].pb.piece;
+                drop_s[q] = (flags & PFPB200_PFBWT_SSA) && pq.c_first >= 0 && pq.c_first == prev ? 1 : 0;
+                ns[q] = pq.n_ssa - drop_s[q];
+                if (pq.c_last >= 0) prev = pq.c_last;
+            }
+            for (int q = G - 1, next = -1; q >= 0; q--) {
+                const PbPiece &pq = m->r[q].pb.piece;
+                ne[q] = pq.n_esa - ((flags & PFPB200_PFBWT_ESA) && pq.c_last >= 0 && pq.c_last == next ? 1 : 0);
+                if (pq.c_first >= 0) next = pq.c_first;
+            }
+            for (int q = 0; q < g; q++) { off_s += ns[q]; off_e += ne[q]; }
+            R.pb_ssa = ns[g];
+            R.pb_esa = ne[g];
+            const u64 from[2] = {drop_s[g] * S2, 0}, bytes[2] = {ns[g] * S2, ne[g] * S2}, to[2] = {off_s * S2, off_e * S2};
+            std::vector<u8> buf;
+            for (int i = 0; i < 2 && ok(); i++) {
+                if (F.fd[2 + i] < 0 || bytes[i] == 0) continue;
+                buf.resize((size_t)std::min<u64>(bytes[i], (u64)64 << 20));
+                const int fd = open(fname(ext[2 + i]), O_WRONLY);
+                if (fd < 0) { run(pfp_fail(ctx, PFPB200_E_IO, "%s: %s", name, strerror(errno))); break; }
+                for (u64 done = 0; done < bytes[i] && ok();) {
+                    const u64 k = std::min<u64>(bytes[i] - done, buf.size());
+                    const ssize_t r = pread(F.fd[2 + i], buf.data(), k, (off_t)(from[i] + done));
+                    if (r != (ssize_t)k) run(pfp_fail(ctx, PFPB200_E_IO, "%s: read error", F.name[2 + i]));
+                    else run(pb_put_host(ctx, fd, to[i] + done, buf.data(), k, name));
+                    done += k;
+                }
+                if (close(fd) != 0 && ok()) run(pfp_fail(ctx, PFPB200_E_IO, "%s: write error: %s", name, strerror(errno)));
+            }
         }
-        if (ok() && S.n_ssa) run(piece_to_file(R, fname("ssa"), off_s * 2 * PFP_IBYTES, S.ssa, S.n_ssa * 2 * PFP_IBYTES));
-        if (ok() && S.n_esa) run(piece_to_file(R, fname("esa"), off_e * 2 * PFP_IBYTES, S.esa, S.n_esa * 2 * PFP_IBYTES));
         t_write = wall_sec();
     } while (0);
     cudaStreamSynchronize(ctx->stream);
+    for (int i = 0; i < 2; i++)                             // the part files go, whatever happened
+        if (part[i][0]) unlink(part[i]);
     R.pb_stat.suffixes = S.M0;
-    R.pb_stat.chars = S.em.chars;
-    R.pb_stat.hard = S.em.n_hard;
+    R.pb_stat.chars = S.plan.chars;
+    R.pb_stat.hard = S.plan.n_hard;
     R.pb_stat.peak_bytes = ctx->arena.peak;
     R.pb_stat.ms_read = (float)(1e3 * (t_read - t0));
     R.pb_stat.ms_sort = (float)(1e3 * std::max(0.0, t_sort - t_read));
-    R.pb_stat.ms_emit = (float)(1e3 * std::max(0.0, t_emit - t_sort));
-    R.pb_stat.ms_write = (float)(1e3 * std::max(0.0, t_write - t_emit));
+    // the plan and the windows' device work; the files, the barriers between them and the stitching
+    R.pb_stat.ms_emit = (float)(1e3 * std::max(0.0, t_plan - t_sort) + S.piece.ms_emit);
+    R.pb_stat.ms_write = (float)std::max(0.0, 1e3 * std::max(0.0, t_write - t_plan) - S.piece.ms_emit);
     R.launches = ctx->launches - launches0;
     m->bar.wait();                                          // no peer reads my memory any more
     pfp_release_scratch(ctx);
@@ -1097,8 +1155,8 @@ extern "C" int pfpb200_multi_pfbwt_file(pfpb200_multi *m, const char *basename, 
     for (const Rank &R : m->r) {
         const pfpb200_pfbwt_rank &s = R.pb_stat;
         res->n_bwt += s.chars;
-        res->n_ssa += R.pb.n_ssa;
-        res->n_esa += R.pb.n_esa;
+        res->n_ssa += R.pb_ssa;
+        res->n_esa += R.pb_esa;
         res->hard += s.hard;
         res->launches += R.launches;
         res->ms_sa = std::max(res->ms_sa, s.ms_sort);
@@ -1118,5 +1176,12 @@ extern "C" int pfpb200_multi_pfbwt_ranks(const pfpb200_multi *m, pfpb200_pfbwt_r
     if (!m || !out) return PFPB200_E_ARG;
     int k = 0;
     for (; k < m->n && k < cap; k++) out[k] = m->r[k].pb_stat;
+    return k;
+}
+
+extern "C" int pfpb200_multi_pfbwt_windows(const pfpb200_multi *m, uint64_t *windows, int cap) {
+    if (!m || !windows) return PFPB200_E_ARG;
+    int k = 0;
+    for (; k < m->n && k < cap; k++) windows[k] = m->r[k].pb_windows;
     return k;
 }

@@ -25,16 +25,19 @@
 // Outputs are byte-identical to pfbwtNT.x (.bwt, .sa, .ssa, .esa): tests/test_pfbwt_gpu.py.
 //
 // Steps 1, 3 and 4 serve the sharded path too (pfp_pfbwt_multi.cu, pfp_multi.cu): the input reader
-// and argument checks, the word structure (pb_words), the group heads of a doubling round, the
-// emission on a slice of sorted slots (pb_emit) and the run samples (pb_samples).  The emission reads
-// the sort's output only through a slot reader.  Step 2 is this file's own: 32-bit packed ranks and
-// positions, N < 2^32 - 16; the sharded sort partitions the suffixes and keeps 64-bit ranks.
+// and argument checks, the word structure (pb_words: word ends, no per-position array), the group heads
+// of a doubling round, the plan of the emission on a slice of sorted slots (pb_plan), its windows written
+// to the files (pb_write_windows) and the run samples (pb_samples).  The emission reads the sort's output
+// only through a slot reader.  Step 2 is this file's own: 32-bit packed ranks and positions, N < 2^32 - 16,
+// and the word of every position (pb_word_ids); the sharded sort partitions the suffixes, keeps 64-bit
+// ranks and finds the words of its own suffixes in the word ends.
 #include "pfp_common.cuh"
 #include "pfp_stages.cuh"
 #include <errno.h>
 #include <fcntl.h>
 #include <stdlib.h>
 #include <sys/stat.h>
+#include <time.h>
 #include <unistd.h>
 
 constexpr u64 PB_BATCH = (u64)1 << 30;          // occurrences sorted at once in the hard groups
@@ -63,11 +66,12 @@ __global__ void __launch_bounds__(PB_T) pb_flags_k(const u8 *__restrict__ d, u64
     if (t < N) flag[t] = pb_term(d[t]) ? 1 : 0;
 }
 
-// wend[k] = position of the k-th terminator; wid[t] = terminators before t = the word of position t
-__global__ void __launch_bounds__(PB_T) pb_wend_k(const u8 *__restrict__ flag, const u32 *__restrict__ wid, u64 N,
-                                                  u64 *__restrict__ wend) {
+// wend[k] = position of the k-th terminator, over the chunk [c0, c0 + n) whose first terminator is
+// number k0; scan[t] = terminators of the chunk before t
+__global__ void __launch_bounds__(PB_T) pb_wend_k(const u8 *__restrict__ flag, const u32 *__restrict__ scan, u64 n,
+                                                  u64 c0, u64 k0, u64 *__restrict__ wend) {
     const u64 t = (u64)blockIdx.x * PB_T + threadIdx.x;
-    if (t < N && flag[t]) wend[wid[t]] = t;
+    if (t < n && flag[t]) wend[k0 + scan[t]] = c0 + t;
 }
 
 __global__ void __launch_bounds__(PB_T) pb_alpha_k(const u8 *__restrict__ d, u64 N, u32 *__restrict__ present) {
@@ -168,7 +172,7 @@ __global__ void __launch_bounds__(PB_T) pb_compact_k(const u8 *__restrict__ keep
 // ---- the walk over the sorted suffixes (both paths) -----------------------------------------------
 struct PbView {
     const u8 *d;
-    const u32 *wid, *occ, *istart;
+    const u32 *occ, *istart;
     const u64 *wend;
     uint2 *mrec;                // per slot, written by pb_count_k: {word, suffix length}
     u16 *mc;                    // per slot: char in front | whole word << 8 | counts << 9
@@ -194,7 +198,7 @@ __global__ void __launch_bounds__(PB_T) pb_count_k(PbView v, Slots sl, u32 *__re
     newgrp[k] = (k == 0 || sl.grp(k) != sl.grp(k - 1)) ? 1 : 0;
     u32 word = 0, len = 0, n = 0, m = 0;
     if (!pb_term(v.d[s])) {
-        word = v.wid[s];
+        word = sl.word(k);
         len = (u32)(v.wend[word] - s);
         if (len > v.w) {                                             // pfbwt.cpp:152
             const bool full = s == 0 || v.d[s - 1] == PFP_END_OF_WORD;   // :154
@@ -411,26 +415,35 @@ int pb_sync_read(pfpb200_ctx *ctx, int slot, int n) {
     return PFPB200_OK;
 }
 
-// terminator flags -> word of every position and word ends; .occ -> first .ilist entry of every word;
-// the dictionary's alphabet -> dense codes, symbols per 64-bit first key
+// terminator flags -> word ends, chunk by chunk; .occ -> first .ilist entry of every word; the
+// dictionary's alphabet -> dense codes, symbols per 64-bit first key
 int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W) {
-    const u64 N = in.N;
-    u8 *flag = nullptr;
-    PFP_TRY(pfp_alloc_t(ctx, &flag, N));
-    PFP_TRY(pfp_alloc_t(ctx, &W->wid, N));
+    const u64 N = in.N, chunk = N < PB_CHUNK ? N : PB_CHUNK;
     PFP_TRY(pfp_alloc_t(ctx, &W->wend, in.dwords + 2));
     PFP_TRY(pfp_alloc_t(ctx, &W->istart, in.dwords + 1));
-    PB_LAUNCH(ctx, N, pb_flags_k, in.d, N, flag);
-    PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, flag, W->wid, N, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
-    PFP_TRY(pfp_exclusive_scan_u32(ctx, in.occ, W->istart, in.dwords, reinterpret_cast<u32 *>(&ctx->d_flags[2])));
-    PFP_TRY(pb_sync_read(ctx, 1, 2));
-    if ((u32)ctx->h_flags[1] != in.dwords + 1)                        // get_num_words(), :360, + the final EndOfDict
-        return pfp_fail(ctx, PFPB200_E_ARG, "the dictionary holds %u words, .occ %llu", (u32)ctx->h_flags[1] - 1,
+    u8 *flag = nullptr;
+    u32 *scan = nullptr;
+    PFP_TRY(pfp_alloc_t(ctx, &flag, chunk));
+    PFP_TRY(pfp_alloc_t(ctx, &scan, chunk));
+    u64 words = 0;                                                    // terminators before the chunk
+    for (u64 c0 = 0; c0 < N; c0 += chunk) {
+        const u64 n = N - c0 < chunk ? N - c0 : chunk;
+        PB_LAUNCH(ctx, n, pb_flags_k, in.d + c0, n, flag);
+        PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, flag, scan, n, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
+        PFP_TRY(pb_sync_read(ctx, 1, 1));
+        const u64 nt = (u32)ctx->h_flags[1];
+        if (words + nt <= in.dwords + 1) PB_LAUNCH(ctx, n, pb_wend_k, flag, scan, n, c0, words, W->wend);
+        words += nt;                                                  // (too many: reported below)
+    }
+    PFP_TRY(pfp_free_now(ctx, flag));
+    PFP_TRY(pfp_free_now(ctx, scan));
+    if (words != in.dwords + 1)                                       // get_num_words(), :360, + the final EndOfDict
+        return pfp_fail(ctx, PFPB200_E_ARG, "the dictionary holds %u words, .occ %llu", (u32)words - 1,
                         (unsigned long long)in.dwords);
+    PFP_TRY(pfp_exclusive_scan_u32(ctx, in.occ, W->istart, in.dwords, reinterpret_cast<u32 *>(&ctx->d_flags[2])));
+    PFP_TRY(pb_sync_read(ctx, 2, 1));
     if ((u64)(u32)ctx->h_flags[2] + 1 != in.psize)                    // assert(last==psize), :384
         return pfp_fail(ctx, PFPB200_E_ARG, "sum of .occ + 1 != size of .ilist");
-    PB_LAUNCH(ctx, N, pb_wend_k, flag, W->wid, N, W->wend);
-    PFP_TRY(pfp_free_now(ctx, flag));
     u32 *present = reinterpret_cast<u32 *>(&ctx->d_flags[8]);       // 8 x 32 bits = slots 8..11
     PFP_CUDA(ctx, cudaMemsetAsync(present, 0, 8 * sizeof(u32), ctx->stream));
     pb_alpha_k<<<ctx->sm_count * 8, PB_T, 0, ctx->stream>>>(in.d, N, present);
@@ -447,6 +460,16 @@ int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W) {
     return PFPB200_OK;
 }
 
+// wid[t] = terminators before t = the word of position t (N < 2^32 - 16 on the one-GPU path)
+int pb_word_ids(pfpb200_ctx *ctx, const PbInput &in, PbWords *W) {
+    u8 *flag = nullptr;
+    PFP_TRY(pfp_alloc_t(ctx, &flag, in.N));
+    PFP_TRY(pfp_alloc_t(ctx, &W->wid, in.N));
+    PB_LAUNCH(ctx, in.N, pb_flags_k, in.d, in.N, flag);
+    PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, flag, W->wid, in.N, nullptr));
+    return pfp_free_now(ctx, flag);
+}
+
 // the plan over all n slots: count -> scans -> first / mixed / hard
 template <class Slots>
 int pb_plan(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, u8 *newgrp, u32 *gscan, PbPlan *P) {
@@ -460,7 +483,7 @@ int pb_plan(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64
     PFP_TRY(pfp_alloc_t(ctx, &P->hcnt, n));
     PFP_TRY(pfp_alloc_t(ctx, &P->off, n + 1));
     PFP_TRY(pfp_alloc_t(ctx, &P->hoff, n + 1));
-    const PbView V{in.d, W.wid, in.occ, W.istart, W.wend, P->mrec, P->mc, n, in.w};
+    const PbView V{in.d, in.occ, W.istart, W.wend, P->mrec, P->mc, n, in.w};
     PB_LAUNCH(ctx, n, pb_count_k<Slots>, V, sl, P->cnt, newgrp);
     PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, newgrp, gscan, n, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
     PFP_TRY(pfp_exclusive_scan_u32_u64(ctx, P->cnt, P->off, n, &ctx->d_flags[2]));
@@ -493,7 +516,7 @@ int pb_window_end(pfpb200_ctx *ctx, const PbPlan &P, u64 ka, u64 cap, u64 *kb, u
 int pb_window(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 ka, u64 kb, u64 hcap,
               bool held, PbEmit *E) {
     const bool want_sa = (in.flags & (PFPB200_PFBWT_SA | PFPB200_PFBWT_SSA | PFPB200_PFBWT_ESA)) != 0;
-    const PbView V{in.d, W.wid, in.occ, W.istart, W.wend, P.mrec, P.mc, P.n, in.w};
+    const PbView V{in.d, in.occ, W.istart, W.wend, P.mrec, P.mc, P.n, in.w};
     // the window's first and last char and hard occurrence
     u64 *h = &ctx->h_flags[12];
     PFP_CUDA(ctx, cudaMemcpyAsync(&h[0], &P.off[ka], sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
@@ -571,15 +594,8 @@ int pb_window(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPla
     return PFPB200_OK;
 }
 
-template <class Slots>
-int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
-            PbEmit *E) {
-    PbPlan P;
-    PFP_TRY(pb_plan(ctx, in, W, sl, n, newgrp, gscan, &P));
-    return pb_window(ctx, in, W, P, 0, n, P.n_hard, held, E);
-}
-template int pb_emit<PbSplitSlots>(pfpb200_ctx *, const PbInput &, const PbWords &, PbSplitSlots, u64, bool, u8 *, u32 *,
-                                   PbEmit *);
+template int pb_plan<PbSplitSlots>(pfpb200_ctx *, const PbInput &, const PbWords &, PbSplitSlots, u64, u8 *, u32 *,
+                                   PbPlan *);
 
 int pb_samples(pfpb200_ctx *ctx, const PbEmit &E, int at_end, int prev, int next, u64 off, bool held, u8 **out,
                u64 *n_out) {
@@ -621,9 +637,7 @@ static void pb_drop_own_outputs(pfpb200_ctx *ctx) {
     pfp_release_scratch(ctx);
 }
 
-// The device memory the outputs of a file call may take once its plan is done: PFPB200_PFBWT_BUDGET=<bytes>,
-// or the free memory plus what the context's arena holds unused (as pfpb200_parse_file counts it).
-static int pb_budget(pfpb200_ctx *ctx, u64 *budget) {
+int pb_budget(pfpb200_ctx *ctx, int share, u64 *budget) {
     const char *ev = getenv("PFPB200_PFBWT_BUDGET");
     if (ev && atoll(ev) > 0) {
         *budget = (u64)atoll(ev);
@@ -631,12 +645,28 @@ static int pb_budget(pfpb200_ctx *ctx, u64 *budget) {
     }
     size_t fr = 0, tot = 0;
     PFP_CUDA(ctx, cudaMemGetInfo(&fr, &tot));
-    *budget = (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
+    // a context alone on its device counts its arena's unused part; contexts that share the device do
+    // not: a window's arrays do not fit into scattered holes, and the growth of their arenas would then
+    // take memory the other contexts count on
+    *budget = share > 1 ? (u64)fr / (u64)share : (u64)fr + (u64)(ctx->arena.total - ctx->arena.in_use);
     return PFPB200_OK;
 }
 
-// appends host bytes to an output file at file_off
-static int pb_put_host(pfpb200_ctx *ctx, int fd, u64 file_off, const u8 *p, u64 bytes, const char *name) {
+u64 pb_window_bytes(const PbPlan &P, u32 flags, u64 cap) {
+    return pb_out_bytes(cap < P.chars ? cap : P.chars, P.n_hard, flags);
+}
+
+u64 pb_window_chars(const PbPlan &P, u32 flags, u64 budget) {
+    if (pb_out_bytes(P.chars, P.n_hard, flags) <= budget) return P.chars;
+    u64 lo = 0, hi = P.chars;                                // pb_out_bytes grows with c: the largest c that fits
+    while (lo < hi) {
+        const u64 mid = lo + (hi - lo + 1) / 2;
+        if (pb_out_bytes(mid, P.n_hard, flags) <= budget) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+int pb_put_host(pfpb200_ctx *ctx, int fd, u64 file_off, const u8 *p, u64 bytes, const char *name) {
     u64 done = 0;
     while (done < bytes) {
         const ssize_t r = pwrite(fd, p + done, bytes - done, (off_t)(file_off + done));
@@ -646,21 +676,90 @@ static int pb_put_host(pfpb200_ctx *ctx, int fd, u64 file_off, const u8 *p, u64 
     return PFPB200_OK;
 }
 
-// The outputs of a plan in windows of whole groups of at most cap chars (DESIGN.md §6c): each window's
-// chars and SA values go to <base>.bwt / .sa at their offsets, its run samples are appended to
-// <base>.ssa / .esa.  Samples across a window border: a window's first char knows the char in front of
-// it (-s); the last run end of a window (-e) waits on the host until the next window's first char shows
-// whether the run goes on.
-struct PbOutFiles {
-    int fd[4] = {-1, -1, -1, -1};              // bwt, sa, ssa, esa
-    char name[4][4096];
-    ~PbOutFiles() {
-        for (int i = 0; i < 4; i++)
-            if (fd[i] >= 0) close(fd[i]);
+static double pb_ms(const struct timespec &a) {
+    struct timespec b;
+    clock_gettime(CLOCK_MONOTONIC, &b);
+    return 1e3 * (double)(b.tv_sec - a.tv_sec) + 1e-6 * (double)(b.tv_nsec - a.tv_nsec);
+}
+
+// Samples across a window border: a window's first char knows the char in front of it (-s); the last
+// run end of a window (-e) waits on the host until the next window's first char shows whether the run
+// goes on.  Across the piece's own borders nothing is known here: its first char starts a run and its
+// last char ends one (the sharded path drops those records when a neighbouring piece continues the run).
+int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 cap, PbOutFiles &F,
+                     u64 off, PbPiece *pc) {
+    const u64 S2 = 2 * PFP_IBYTES;                            // one sample: (BWT position, SA value)
+    u64 ka = 0, n_s = 0, n_e = 0;
+    int prev = -1;                                           // last char of the windows so far (-1: none yet)
+    bool pending = false;                                    // the last run end so far, not yet written
+    u8 pend[2 * PFP_IBYTES];
+    *pc = PbPiece();
+    struct timespec t;
+    while (ka < P.n) {
+        u64 kb = 0, cend = 0;
+        clock_gettime(CLOCK_MONOTONIC, &t);
+        PFP_TRY(pb_window_end(ctx, P, ka, cap, &kb, &cend));
+        PbEmit E;
+        PFP_TRY(pb_window(ctx, in, W, P, ka, kb, cap, false, &E));
+        PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        pc->ms_emit += pb_ms(t);
+        pc->windows++;
+        const u64 n = E.chars, gb = off + E.base;             // the window's chars: BWT positions [gb, gb + n)
+        if (n) {
+            clock_gettime(CLOCK_MONOTONIC, &t);
+            u8 *cf = reinterpret_cast<u8 *>(&ctx->h_flags[9]), *cl = reinterpret_cast<u8 *>(&ctx->h_flags[10]);
+            PFP_CUDA(ctx, cudaMemcpyAsync(cf, E.bwt, 1, cudaMemcpyDeviceToHost, ctx->stream));
+            PFP_CUDA(ctx, cudaMemcpyAsync(cl, E.bwt + n - 1, 1, cudaMemcpyDeviceToHost, ctx->stream));
+            PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            const int c_first = *cf, c_last = *cl;
+            if (pc->c_first < 0) pc->c_first = c_first;
+            PFP_TRY(pfp_device_to_fd(ctx, F.fd[0], gb, E.bwt, n, F.name[0]));
+            if (F.fd[1] >= 0) {                              // the .sa file has no entry for BWT position 0
+                if (gb == 0) PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], 0, E.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES, F.name[1]));
+                else PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], (gb - 1) * PFP_IBYTES, E.sa5, n * PFP_IBYTES, F.name[1]));
+            }
+            u8 *out = nullptr;
+            u64 m = 0;
+            if (F.fd[2] >= 0) {
+                PFP_TRY(pb_samples(ctx, E, 0, prev, -1, gb, false, &out, &m));
+                PFP_TRY(pfp_device_to_fd(ctx, F.fd[2], n_s * S2, out, m * S2, F.name[2]));
+                PFP_TRY(pfp_free_now(ctx, out));
+                n_s += m;
+            }
+            if (F.fd[3] >= 0) {
+                if (pending && c_first != prev) {
+                    PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
+                    n_e++;
+                }
+                // with no char behind the window its last position ends a run: m >= 1, the last one pending
+                PFP_TRY(pb_samples(ctx, E, 1, -1, -1, gb, false, &out, &m));
+                PFP_TRY(pfp_device_to_fd(ctx, F.fd[3], n_e * S2, out, (m - 1) * S2, F.name[3]));
+                PFP_CUDA(ctx, cudaMemcpyAsync(pend, out + (m - 1) * S2, S2, cudaMemcpyDeviceToHost, ctx->stream));
+                PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+                PFP_TRY(pfp_free_now(ctx, out));
+                n_e += m - 1;
+                pending = true;
+            }
+            prev = c_last;
+            pc->ms_write += pb_ms(t);
+        }
+        PFP_TRY(pfp_free_now(ctx, E.bwt));
+        PFP_TRY(pfp_free_now(ctx, E.sa5));
+        ka = kb;
     }
-};
-static int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 cap,
-                            const char *base, pfpb200_pfbwt_result *res, u64 *windows) {
+    if (pending) {
+        PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
+        n_e++;
+    }
+    pc->c_last = prev;
+    pc->n_ssa = n_s;
+    pc->n_esa = n_e;
+    return PFPB200_OK;
+}
+
+// the one-GPU file outputs in windows: <base>.bwt / .sa created at their final sizes, .ssa / .esa appended
+static int pb_write_files(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 cap,
+                          const char *base, pfpb200_pfbwt_result *res, u64 *windows) {
     static const char *const ext[4] = {"bwt", "sa", "ssa", "esa"};
     const u32 want[4] = {0, PFPB200_PFBWT_SA, PFPB200_PFBWT_SSA, PFPB200_PFBWT_ESA};   // .bwt always
     const u64 size[4] = {P.chars, (P.chars - 1) * PFP_IBYTES, 0, 0};   // .sa: no entry for BWT position 0
@@ -673,62 +772,9 @@ static int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &
         if (size[i] && ftruncate(F.fd[i], (off_t)size[i]) != 0)
             return pfp_fail(ctx, PFPB200_E_IO, "%s: %s", F.name[i], strerror(errno));
     }
-    const u64 S2 = 2 * PFP_IBYTES;                            // one sample: (BWT position, SA value)
-    u64 ka = 0, n_s = 0, n_e = 0;
-    int prev = -1;                                           // last char of the windows so far (-1: none yet)
-    bool pending = false;                                    // the last run end so far, not yet written
-    u8 pend[2 * PFP_IBYTES];
-    *windows = 0;
-    while (ka < P.n) {
-        u64 kb = 0, cend = 0;
-        PFP_TRY(pb_window_end(ctx, P, ka, cap, &kb, &cend));
-        PbEmit E;
-        PFP_TRY(pb_window(ctx, in, W, P, ka, kb, cap, false, &E));
-        ++*windows;
-        const u64 n = E.chars;
-        if (n) {
-            u8 *cf = reinterpret_cast<u8 *>(&ctx->h_flags[9]), *cl = reinterpret_cast<u8 *>(&ctx->h_flags[10]);
-            PFP_CUDA(ctx, cudaMemcpyAsync(cf, E.bwt, 1, cudaMemcpyDeviceToHost, ctx->stream));
-            PFP_CUDA(ctx, cudaMemcpyAsync(cl, E.bwt + n - 1, 1, cudaMemcpyDeviceToHost, ctx->stream));
-            PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            const int c_first = *cf, c_last = *cl;
-            PFP_TRY(pfp_device_to_fd(ctx, F.fd[0], E.base, E.bwt, n, F.name[0]));
-            if (F.fd[1] >= 0) {
-                if (E.base == 0) PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], 0, E.sa5 + PFP_IBYTES, (n - 1) * PFP_IBYTES, F.name[1]));
-                else PFP_TRY(pfp_device_to_fd(ctx, F.fd[1], (E.base - 1) * PFP_IBYTES, E.sa5, n * PFP_IBYTES, F.name[1]));
-            }
-            u8 *out = nullptr;
-            u64 m = 0;
-            if (F.fd[2] >= 0) {
-                PFP_TRY(pb_samples(ctx, E, 0, prev, -1, E.base, false, &out, &m));
-                PFP_TRY(pfp_device_to_fd(ctx, F.fd[2], n_s * S2, out, m * S2, F.name[2]));
-                PFP_TRY(pfp_free_now(ctx, out));
-                n_s += m;
-            }
-            if (F.fd[3] >= 0) {
-                if (pending && c_first != prev) {
-                    PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
-                    n_e++;
-                }
-                // with no char behind the window its last position ends a run: m >= 1, the last one pending
-                PFP_TRY(pb_samples(ctx, E, 1, -1, -1, E.base, false, &out, &m));
-                PFP_TRY(pfp_device_to_fd(ctx, F.fd[3], n_e * S2, out, (m - 1) * S2, F.name[3]));
-                PFP_CUDA(ctx, cudaMemcpyAsync(pend, out + (m - 1) * S2, S2, cudaMemcpyDeviceToHost, ctx->stream));
-                PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-                PFP_TRY(pfp_free_now(ctx, out));
-                n_e += m - 1;
-                pending = true;
-            }
-            prev = c_last;
-        }
-        PFP_TRY(pfp_free_now(ctx, E.bwt));
-        PFP_TRY(pfp_free_now(ctx, E.sa5));
-        ka = kb;
-    }
-    if (pending) {
-        PFP_TRY(pb_put_host(ctx, F.fd[3], n_e * S2, pend, S2, F.name[3]));
-        n_e++;
-    }
+    PbPiece pc;
+    PFP_TRY(pb_write_windows(ctx, in, W, P, cap, F, 0, &pc));
+    *windows = pc.windows;
     for (int i = 0; i < 4; i++) {
         const int fd = F.fd[i];
         F.fd[i] = -1;
@@ -736,8 +782,8 @@ static int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &
     }
     res->n_bwt = P.chars;
     if (in.flags & PFPB200_PFBWT_SA) res->n_sa = P.chars - 1;
-    res->n_ssa = n_s;
-    res->n_esa = n_e;
+    res->n_ssa = pc.n_ssa;
+    res->n_esa = pc.n_esa;
     return PFPB200_OK;
 }
 
@@ -764,6 +810,7 @@ static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, const char *ou
     // ---- 1. word structure ---------------------------------------------------------------------------
     PbWords W;
     PFP_TRY(pb_words(ctx, in, &W));
+    PFP_TRY(pb_word_ids(ctx, in, &W));
     // ---- 2. suffix sort ----------------------------------------------------------------------------------
     u8 *flag = nullptr, *keep = nullptr;
     u64 *k0 = nullptr, *k1 = nullptr;
@@ -828,23 +875,16 @@ static int pfbwt_device_impl(pfpb200_ctx *ctx, const PbInput &in, const char *ou
     // ---- 3. emission --------------------------------------------------------------------------------------------
     PFP_TRY(pfp_free_now(ctx, rank));                        // the ranks travel with the suffix array from here on
     PbPlan P;
-    PFP_TRY(pb_plan(ctx, in, W, PbPackedSlots{sa}, N, flag, escan, &P));
+    PFP_TRY(pb_plan(ctx, in, W, PbPackedSlots{sa, W.wid}, N, flag, escan, &P));
     u64 cap = P.chars;
     if (out_base) {              // one window when the whole output fits, else windows of the most chars that fit
         u64 budget = 0;
-        PFP_TRY(pb_budget(ctx, &budget));
-        if (pb_out_bytes(P.chars, P.n_hard, flags) > budget) {
-            u64 lo = 0, hi = P.chars;                        // pb_out_bytes grows with c: the largest c that fits
-            while (lo < hi) {
-                const u64 mid = lo + (hi - lo + 1) / 2;
-                if (pb_out_bytes(mid, P.n_hard, flags) <= budget) lo = mid; else hi = mid - 1;
-            }
-            cap = lo;                                        // < P.chars; 0: one group per window
-        }
+        PFP_TRY(pb_budget(ctx, 1, &budget));
+        cap = pb_window_chars(P, flags, budget);             // < P.chars: windows; 0: one group per window
     }
     *windows = 1;
     if (cap < P.chars) {
-        PFP_TRY(pb_write_windows(ctx, in, W, P, cap, out_base, res, windows));
+        PFP_TRY(pb_write_files(ctx, in, W, P, cap, out_base, res, windows));
     } else {
         PbEmit E;
         PFP_TRY(pb_window(ctx, in, W, P, 0, N, P.n_hard, true, &E));

@@ -3,23 +3,21 @@
 // pfp_multi.cu owns the threads and the barriers and calls the steps below on every rank.
 //
 // The word structure, the emission and the sampled suffix array are the ones of pfp_pfbwt.cu (pb_words,
-// pb_emit, pb_samples; its comment says what each step computes).  What is here is the suffix sort
+// pb_plan, pb_write_windows, pb_samples; its comment says what each step computes).  What is here is the suffix sort
 // that one GPU cannot do, with 64-bit positions and ranks and the dictionary suffixes partitioned over
 // the ranks:
 //   * every rank holds the whole dictionary and the parse-side streams and derives the same word
-//     structure and dense alphabet codes;
+//     structure (word ends, no word per position) and dense alphabet codes;
 //   * a suffix belongs to the rank whose range holds its FIRST KEY (h0 dense-coded symbols, cut
 //     behind the terminator); equal first keys never straddle two ranks, so rank g's sorted
 //     suffixes are the global slots [base_g, base_g + M_g) and no group of the doubling is ever split;
 //   * the rank array is stored by position, block g on rank g, and read / written with direct
 //     peer loads and stores (PmRanks); a round is "gather rank(i+h)" | barrier | "sort, scatter
 //     the changed ranks" | barrier, so no rank ever reads a partly updated array;
-//   * the emission runs on each rank's slice (sa_pos / sa_grp, read through PbSplitSlots): a group of
-//     equal suffixes is whole on one rank, so the merge of the .ilist cursors stays local.
+//   * the emission runs on each rank's slice (sa_pos / sa_grp / sa_word, read through PbSplitSlots): a
+//     group of equal suffixes is whole on one rank, so the merge of the .ilist cursors stays local.
 #include "pfp_common.cuh"
 #include "pfp_stages.cuh"
-
-constexpr u64 PM_CHUNK = (u64)1 << 30;          // dictionary positions per pass of the partition
 
 __device__ __forceinline__ u64 pm_rank_get(const PmRanks &R, u64 j) {
     const u64 o = j / R.per;
@@ -68,13 +66,15 @@ __global__ void __launch_bounds__(PB_T) pm_in_k(const u8 *__restrict__ d, u64 N,
     if (t < n) flag[t] = pm_in(rg, pb_first_key(d, N, code, h0, bs, c0 + t)) ? 1 : 0;
 }
 
-// the owned positions of chunk [c0, c0 + n), in position order from element e0 on: position, length
-// to the terminator, first key; val = element id, slot = local slot of the first sort
+// the owned positions of chunk [c0, c0 + n), in position order from element e0 on: position, word,
+// length to the terminator, first key; val = element id, slot = local slot of the first sort.  The word
+// of s is the first k with wend[k] >= s (nw word ends): a binary search, on the same path for the
+// neighbouring positions of a warp.
 __global__ void __launch_bounds__(PB_T) pm_collect_k(const u8 *__restrict__ d, u64 N, PbCodes cd, int h0, int bs,
                                                      const u8 *__restrict__ flag, const u32 *__restrict__ scan, u64 c0,
-                                                     u64 n, u64 e0, const u32 *__restrict__ wid,
-                                                     const u64 *__restrict__ wend, u64 *__restrict__ pos,
-                                                     u32 *__restrict__ sl, u64 *__restrict__ key, u32 *__restrict__ val,
+                                                     u64 n, u64 e0, const u64 *__restrict__ wend, u64 nw,
+                                                     u64 *__restrict__ pos, u32 *__restrict__ we, u32 *__restrict__ sl,
+                                                     u64 *__restrict__ key, u32 *__restrict__ val,
                                                      u32 *__restrict__ slot) {
     __shared__ u8 code[256];
     code[threadIdx.x] = cd.code[threadIdx.x];
@@ -82,8 +82,14 @@ __global__ void __launch_bounds__(PB_T) pm_collect_k(const u8 *__restrict__ d, u
     const u64 t = (u64)blockIdx.x * PB_T + threadIdx.x;
     if (t >= n || !flag[t]) return;
     const u64 s = c0 + t, e = e0 + scan[t];
+    u64 a = 0, b = nw - 1;                                       // wend[nw - 1] = N - 1 >= s
+    while (a < b) {
+        const u64 m = (a + b) >> 1;
+        if (wend[m] < s) a = m + 1; else b = m;
+    }
     pos[e] = s;
-    sl[e] = (u32)(wend[wid[s]] - s);
+    we[e] = (u32)a;
+    sl[e] = (u32)(wend[a] - s);
     key[e] = pb_first_key(d, N, code, h0, bs, s);
     val[e] = (u32)e;
     slot[e] = (u32)e;
@@ -104,8 +110,9 @@ __global__ void __launch_bounds__(PB_T) pm_update_k(const u8 *__restrict__ flag,
                                                     const u32 *__restrict__ slot, const u32 *__restrict__ val,
                                                     const u64 *__restrict__ key, int hi_shift,
                                                     const u32 *__restrict__ head, const u64 *__restrict__ pos,
-                                                    const u32 *__restrict__ sl, u64 M, u64 h, u64 base, PmRanks R,
-                                                    u64 *__restrict__ sa_pos, u32 *__restrict__ sa_grp,
+                                                    const u32 *__restrict__ sl, const u32 *__restrict__ we, u64 M,
+                                                    u64 h, u64 base, PmRanks R, u64 *__restrict__ sa_pos,
+                                                    u32 *__restrict__ sa_grp, u32 *__restrict__ sa_word,
                                                     u32 *__restrict__ rs, u8 *__restrict__ keep) {
     const u64 k = (u64)blockIdx.x * PB_T + threadIdx.x;
     if (k >= M) return;
@@ -122,6 +129,7 @@ __global__ void __launch_bounds__(PB_T) pm_update_k(const u8 *__restrict__ flag,
     if (!stay) {
         sa_pos[slot[k]] = s;
         sa_grp[slot[k]] = r;
+        sa_word[slot[k]] = we[e];
     }
 }
 
@@ -190,6 +198,7 @@ int pm_collect(pfpb200_ctx *ctx, PmState &S, int split) {
     S.bn = pb_bits(N);
     S.bm = pb_bits(M);
     PFP_TRY(pfp_alloc_t(ctx, &S.pos, M));
+    PFP_TRY(pfp_alloc_t(ctx, &S.we, M));
     PFP_TRY(pfp_alloc_t(ctx, &S.sl, M));
     PFP_TRY(pfp_alloc_t(ctx, &S.k0, M));
     PFP_TRY(pfp_alloc_t(ctx, &S.k1, M));
@@ -204,13 +213,14 @@ int pm_collect(pfpb200_ctx *ctx, PmState &S, int split) {
     PFP_TRY(pfp_alloc_t(ctx, &S.keep, M));
     PFP_TRY(pfp_alloc_t(ctx, &S.sa_pos, M));
     PFP_TRY(pfp_alloc_t(ctx, &S.sa_grp, M));
+    PFP_TRY(pfp_alloc_t(ctx, &S.sa_word, M));
     if (split) {
         PFP_TRY(pfp_alloc_t(ctx, &S.hi, M));
         PFP_TRY(pfp_alloc_t(ctx, &S.lo, M));
     }
     const PmRange rg{S.rg_lo, S.rg_hi, S.rg_has_lo, S.rg_has_hi};
     if (M) {
-        const u64 chunk = N < PM_CHUNK ? N : PM_CHUNK;
+        const u64 chunk = N < PB_CHUNK ? N : PB_CHUNK;
         u8 *cf = nullptr;
         u32 *cs = nullptr;
         PFP_TRY(pfp_alloc_t(ctx, &cf, chunk));
@@ -222,7 +232,8 @@ int pm_collect(pfpb200_ctx *ctx, PmState &S, int split) {
             PFP_LAUNCHED(ctx);
             PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, cf, cs, n, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
             pm_collect_k<<<pfp_blocks(n, PB_T), PB_T, 0, ctx->stream>>>(S.in.d, N, S.wd.cd, S.wd.h0, S.wd.bs, cf, cs, c0, n, e0,
-                                                                        S.wd.wid, S.wd.wend, S.pos, S.sl, S.k0, S.v0, S.slot);
+                                                                        S.wd.wend, S.in.dwords + 1, S.pos, S.we, S.sl, S.k0,
+                                                                        S.v0, S.slot);
             PFP_LAUNCHED(ctx);
             PFP_TRY(pb_sync_read(ctx, 1, 1));
             e0 += (u32)ctx->h_flags[1];
@@ -245,8 +256,8 @@ int pm_update(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h, int first, 
     else PB_LAUNCH(ctx, M, pb_gflags_k, S.ks, M, S.flag);
     PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, S.flag, S.escan, M, nullptr));
     PB_LAUNCH(ctx, M, pb_heads_k, S.flag, S.escan, S.slot, M, S.head);
-    PB_LAUNCH(ctx, M, pm_update_k, S.flag, S.escan, S.slot, S.vs, S.ks, hi_shift, S.head, S.pos, S.sl, M, h, S.base, R,
-              S.sa_pos, S.sa_grp, S.rs, S.keep);
+    PB_LAUNCH(ctx, M, pm_update_k, S.flag, S.escan, S.slot, S.vs, S.ks, hi_shift, S.head, S.pos, S.sl, S.we, M, h, S.base,
+              R, S.sa_pos, S.sa_grp, S.sa_word, S.rs, S.keep);
     PFP_TRY(pfp_exclusive_scan_u8_u32(ctx, S.keep, S.escan, M, reinterpret_cast<u32 *>(&ctx->d_flags[1])));
     PFP_TRY(pb_sync_read(ctx, 1, 1));
     S.M2 = M ? (u32)ctx->h_flags[1] : 0;
@@ -282,24 +293,18 @@ int pm_sort_done(pfpb200_ctx *ctx, PmState &S) {
     PFP_TRY(pfp_free_now(ctx, S.v1)); PFP_TRY(pfp_free_now(ctx, S.slot)); PFP_TRY(pfp_free_now(ctx, S.slot2));
     PFP_TRY(pfp_free_now(ctx, S.head)); PFP_TRY(pfp_free_now(ctx, S.keep)); PFP_TRY(pfp_free_now(ctx, S.rs));
     PFP_TRY(pfp_free_now(ctx, S.pos)); PFP_TRY(pfp_free_now(ctx, S.sl)); PFP_TRY(pfp_free_now(ctx, S.hi));
-    PFP_TRY(pfp_free_now(ctx, S.lo));
+    PFP_TRY(pfp_free_now(ctx, S.lo)); PFP_TRY(pfp_free_now(ctx, S.we));
     S.lo = nullptr;
     S.k0 = S.k1 = S.ks = nullptr; S.v0 = S.v1 = S.vs = nullptr;
-    S.slot = S.slot2 = S.head = S.rs = S.hi = nullptr; S.keep = nullptr; S.pos = nullptr; S.sl = nullptr;
+    S.slot = S.slot2 = S.head = S.rs = S.hi = S.we = nullptr; S.keep = nullptr; S.pos = nullptr; S.sl = nullptr;
     return PFPB200_OK;
 }
 
 
-// the emission on this rank's slice, and the first / last char of its piece for the runs across pieces
-int pm_emit(pfpb200_ctx *ctx, PmState &S) {
-    PFP_TRY(pb_emit(ctx, S.in, S.wd, PbSplitSlots{S.sa_pos, S.sa_grp}, S.M0, false, S.flag, S.escan, &S.em));
-    const u64 n = S.em.chars;
-    if (n) {
-        PFP_CUDA(ctx, cudaMemcpyAsync(&ctx->h_flags[9], S.em.bwt, 1, cudaMemcpyDeviceToHost, ctx->stream));
-        PFP_CUDA(ctx, cudaMemcpyAsync(&ctx->h_flags[10], S.em.bwt + n - 1, 1, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    PFP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    S.c_first = n ? (int)*(const u8 *)&ctx->h_flags[9] : -1;
-    S.c_last = n ? (int)*(const u8 *)&ctx->h_flags[10] : -1;
+// the plan of the emission on this rank's slice; the sorted slots are not read after it
+int pm_plan(pfpb200_ctx *ctx, PmState &S) {
+    PFP_TRY(pb_plan(ctx, S.in, S.wd, PbSplitSlots{S.sa_pos, S.sa_grp, S.sa_word}, S.M0, S.flag, S.escan, &S.plan));
+    PFP_TRY(pfp_free_now(ctx, S.sa_pos)); PFP_TRY(pfp_free_now(ctx, S.sa_grp)); PFP_TRY(pfp_free_now(ctx, S.sa_word));
+    S.sa_pos = nullptr; S.sa_grp = S.sa_word = nullptr;
     return PFPB200_OK;
 }

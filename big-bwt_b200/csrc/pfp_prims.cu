@@ -94,6 +94,21 @@ int pfp_arena_consolidate(pfpb200_ctx *ctx) {
     return PFPB200_OK;
 }
 
+void pfp_arena_trim(pfpb200_ctx *ctx) {
+    PfpArena &A = ctx->arena;
+    cudaStreamSynchronize(ctx->stream);
+    for (size_t i = 0; i < A.slabs.size();) {
+        const PfpBlock s = A.slabs[i];
+        size_t f = 0;
+        while (f < A.free_list.size() && !(A.free_list[f].p == s.p && A.free_list[f].n == s.n)) f++;
+        if (f == A.free_list.size()) { i++; continue; }          // something in it is in use
+        cudaFree(s.p);
+        A.free_list.erase(A.free_list.begin() + f);
+        A.slabs.erase(A.slabs.begin() + i);
+        A.total -= s.n;
+    }
+}
+
 int pfp_alloc(pfpb200_ctx *ctx, void **p, size_t bytes, bool held) {
     *p = nullptr;
     if (bytes == 0) bytes = 16;

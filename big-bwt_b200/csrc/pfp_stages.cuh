@@ -1,6 +1,7 @@
 // pfp_stages.cuh -- data layout in HBM shared by the stages, and the stage entry points.
 #pragma once
 #include "pfp_common.cuh"
+#include <unistd.h>
 
 // ---- text view ---------------------------------------------------------------------------------
 // A shard buffer T[0..n_buf) whose first byte is global text position pos0.  Global positions
@@ -202,25 +203,29 @@ struct PbInput {
 
 // the word structure of the dictionary and the coding of the first key (pb_words)
 struct PbWords {
-    u32 *wid = nullptr;         // [N] word of every position (terminators before it)
+    u32 *wid = nullptr;         // [N] word of every position (terminators before it): pb_word_ids, one-GPU path only
     u64 *wend = nullptr;        // [words + 1] position of every word's terminator
     u32 *istart = nullptr;      // [words] first .ilist entry of every word, less one
     PbCodes cd;
     int bs = 0, h0 = 0;         // bits of a code, symbols in the first key
 };
 
-// slot k of the sorted dictionary suffixes -> its position and its group (the slot where the group
-// starts).  The one-GPU sort leaves (group << 32) | position in one u64, the sharded sort two arrays.
+// slot k of the sorted dictionary suffixes -> its position, its group (the slot where the group
+// starts) and its word.  The one-GPU sort leaves (group << 32) | position in one u64 and reads the word
+// from the per-position word ids; the sharded sort leaves three arrays per slot.
 struct PbPackedSlots {
     const u64 *sa;
+    const u32 *wid;
     __device__ __forceinline__ u32 pos(u64 k) const { return (u32)sa[k]; }
     __device__ __forceinline__ u32 grp(u64 k) const { return (u32)(sa[k] >> 32); }
+    __device__ __forceinline__ u32 word(u64 k) const { return wid[pos(k)]; }
 };
 struct PbSplitSlots {
     const u64 *sa_pos;
-    const u32 *sa_grp;
+    const u32 *sa_grp, *sa_word;
     __device__ __forceinline__ u64 pos(u64 k) const { return sa_pos[k]; }
     __device__ __forceinline__ u32 grp(u64 k) const { return sa_grp[k]; }
+    __device__ __forceinline__ u32 word(u64 k) const { return sa_word[k]; }
 };
 
 // what the emission leaves: the BWT chars of the slots (of one window: chars [base, base + chars) of the
@@ -255,7 +260,11 @@ constexpr u64 PB_UNIT[5] = {1, 4, 4, 1, PFP_IBYTES};
 int pb_read_file(pfpb200_ctx *ctx, const char *base, int k, void **d, u64 *count);   // one of them
 int pb_read_inputs(pfpb200_ctx *ctx, const char *base, u32 flags, void *in[5], u64 n[5]);
 int pb_sync_read(pfpb200_ctx *ctx, int slot, int n);   // h_flags[slot, slot + n) <- d_flags, then synchronise
+// word ends, first .ilist entries and first-key coding; the word ends are found in chunks of at most
+// PB_CHUNK positions, so the scratch does not grow with the dictionary
+constexpr u64 PB_CHUNK = (u64)1 << 30;
 int pb_words(pfpb200_ctx *ctx, const PbInput &in, PbWords *W);
+int pb_word_ids(pfpb200_ctx *ctx, const PbInput &in, PbWords *W);   // W->wid[N] (the one-GPU sort reads it)
 // the plan of the emission over n sorted slots; newgrp / gscan: scratch of n entries
 template <class Slots>
 int pb_plan(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, u8 *newgrp, u32 *gscan, PbPlan *P);
@@ -267,10 +276,37 @@ int pb_window_end(pfpb200_ctx *ctx, const PbPlan &P, u64 ka, u64 cap, u64 *kb, u
 // occurrences; held: the outputs are held buffers recorded in ctx->pb_out[0..1], otherwise scratch
 int pb_window(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 ka, u64 kb, u64 hcap,
               bool held, PbEmit *E);
-// pb_plan and one window over all n slots
-template <class Slots>
-int pb_emit(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, Slots sl, u64 n, bool held, u8 *newgrp, u32 *gscan,
-            PbEmit *E);
+// The device memory a pfbwt output call may use once its plan is done: PFPB200_PFBWT_BUDGET=<bytes> if
+// set; otherwise, for a context alone on its device, the free memory plus what its arena holds unused,
+// and for one of `share` > 1 contexts on the device, its share of the free memory.
+int pb_budget(pfpb200_ctx *ctx, int share, u64 *budget);
+// the device bytes of a window of at most cap chars (pb_out_bytes)
+u64 pb_window_bytes(const PbPlan &P, u32 flags, u64 cap);
+// the most chars of a window whose output fits the budget: P.chars when the whole output fits, else the
+// largest c with pb_out_bytes(c) <= budget (0: one group per window)
+u64 pb_window_chars(const PbPlan &P, u32 flags, u64 budget);
+// the output files of one piece: .bwt, .sa (positioned writes), .ssa, .esa (appended from offset 0)
+struct PbOutFiles {
+    int fd[4] = {-1, -1, -1, -1};
+    char name[4][4096];
+    ~PbOutFiles() {
+        for (int i = 0; i < 4; i++)
+            if (fd[i] >= 0) close(fd[i]);
+    }
+};
+// what writing a piece left: its windows, its run samples, its first / last char (-1: empty) and times
+struct PbPiece {
+    u64 windows = 0, n_ssa = 0, n_esa = 0;
+    int c_first = -1, c_last = -1;
+    double ms_emit = 0, ms_write = 0;
+};
+// The outputs of a plan, whose chars are BWT positions [off, off + P.chars), in windows of whole groups
+// of at most cap chars, into the files F (DESIGN.md §6c, §6d).  The run samples are those of the piece
+// on its own: the run start at its first char and the run end at its last char are always written.
+int pb_write_windows(pfpb200_ctx *ctx, const PbInput &in, const PbWords &W, const PbPlan &P, u64 cap, PbOutFiles &F,
+                     u64 off, PbPiece *pc);
+// host bytes to [file_off, + bytes) of an open file
+int pb_put_host(pfpb200_ctx *ctx, int fd, u64 file_off, const u8 *p, u64 bytes, const char *name);
 // pfpb200_pfbwt_file from the inputs in HBM: the outputs to <base>.bwt [.sa | .ssa .esa], in windows when they
 // do not fit the device memory left once the plan is done; records the plan for pfpb200_pfbwt_plan
 int pb_to_files(pfpb200_ctx *ctx, const PbInput &in, const char *base, pfpb200_pfbwt_result *res);
@@ -289,22 +325,20 @@ struct PmRanks {
 // one rank's state of a sharded pfbwt call (pfpb200_multi_pfbwt_file)
 struct PmState {
     PbInput in;                                     // the whole dictionary and parse-side streams, on this rank
-    PbWords wd;
+    PbWords wd;                                     // without wid: words come from the word ends
     // the owned first-key range and suffixes
     u64 rg_lo = 0, rg_hi = 0; int rg_has_lo = 0, rg_has_hi = 0;
     u64 M0 = 0, base = 0, M = 0, M2 = 0;
     int bn = 0, bm = 0, split = 0;                  // key layout: bits of N, bits of M0, two sorts
-    u64 *pos = nullptr, *lo = nullptr; u32 *sl = nullptr, *hi = nullptr;   // per element (hi, lo: split key form)
+    u64 *pos = nullptr, *lo = nullptr; u32 *sl = nullptr, *we = nullptr, *hi = nullptr;   // per element (hi, lo: split key form)
     u64 *k0 = nullptr, *k1 = nullptr, *ks = nullptr, *ko = nullptr;
     u32 *v0 = nullptr, *v1 = nullptr, *vs = nullptr, *vo = nullptr;
     u32 *slot = nullptr, *slot2 = nullptr, *head = nullptr, *escan = nullptr, *rs = nullptr;
     u8 *flag = nullptr, *keep = nullptr;
-    u64 *sa_pos = nullptr; u32 *sa_grp = nullptr;  // per local slot
-    // emission
-    PbEmit em;
-    u8 *ssa = nullptr, *esa = nullptr;
-    u64 n_ssa = 0, n_esa = 0;
-    int c_first = -1, c_last = -1;                  // first / last char of the piece (-1: empty)
+    u64 *sa_pos = nullptr; u32 *sa_grp = nullptr, *sa_word = nullptr;   // per local slot
+    // emission: the plan over the slice, then the piece in windows
+    PbPlan plan;
+    PbPiece piece;
 };
 int pm_sample(pfpb200_ctx *ctx, PmState &S, u64 lo, u64 hi, u32 want, u64 *h_out, u32 *got);
 int pm_count(pfpb200_ctx *ctx, PmState &S, u64 klo, u64 khi, int has_lo, int has_hi, u64 *count);
@@ -313,4 +347,4 @@ int pm_update(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h, int first, 
 int pm_gather(pfpb200_ctx *ctx, PmState &S, const PmRanks &R, u64 h);
 int pm_sort(pfpb200_ctx *ctx, PmState &S);
 int pm_sort_done(pfpb200_ctx *ctx, PmState &S);
-int pm_emit(pfpb200_ctx *ctx, PmState &S);
+int pm_plan(pfpb200_ctx *ctx, PmState &S);

@@ -131,6 +131,7 @@ SYMBOLS = ["pfpb200_create", "pfpb200_destroy", "pfpb200_set_stream", "pfpb200_p
            "pfpb200_shard_ranks_back", "pfpb200_multi_create", "pfpb200_multi_destroy", "pfpb200_multi_n_gpus",
            "pfpb200_multi_parse_host", "pfpb200_multi_parse_file", "pfpb200_multi_last_error",
            "pfpb200_multi_phase_ms", "pfpb200_multi_pfbwt_file", "pfpb200_multi_pfbwt_ranks",
+           "pfpb200_multi_pfbwt_windows",
            "pfpb200_check_dict_order",
            "pfpb200_bwtparse_device", "pfpb200_bwtparse_host", "pfpb200_bwtparse_file",
            "pfpb200_unparse_device", "pfpb200_unparse_file",
@@ -199,6 +200,8 @@ def load_library():
     L.pfpb200_multi_pfbwt_file.restype = C.c_int
     L.pfpb200_multi_pfbwt_ranks.argtypes = [vp, C.POINTER(PfbwtRank), C.c_int]
     L.pfpb200_multi_pfbwt_ranks.restype = C.c_int
+    L.pfpb200_multi_pfbwt_windows.argtypes = [vp, C.POINTER(u64), C.c_int]
+    L.pfpb200_multi_pfbwt_windows.restype = C.c_int
     _lib = L
     return L
 
@@ -538,13 +541,17 @@ class MultiScanner:
     def pfbwt_file(self, basename, w=10, flags=0) -> dict:
         """`pfbwt.x -w W [-S | -s -e] <basename>` sharded over the ranks: reads .dict .occ .ilist .bwlast
         [.bwsai], writes the same .bwt [.sa | .ssa .esa] as Scanner.pfbwt_file.  Returns the summed counts,
-        the slowest rank's times and, under "ranks", each rank's suffixes, chars and times."""
+        the slowest rank's times and, under "ranks", each rank's suffixes, chars, times and output
+        "windows" (PFPB200_PFBWT_BUDGET, per rank, sets their size)."""
         r = PfbwtResult()
         self._check(self.L.pfpb200_multi_pfbwt_file(self.h, os.fsencode(basename), w, flags, C.byref(r)))
         d = r.as_dict()
-        buf = (PfbwtRank * len(self.gpu_ids))()
-        k = self.L.pfpb200_multi_pfbwt_ranks(self.h, buf, len(self.gpu_ids))
-        d["ranks"] = [buf[i].as_dict() for i in range(k)]
+        n = len(self.gpu_ids)
+        buf = (PfbwtRank * n)()
+        k = self.L.pfpb200_multi_pfbwt_ranks(self.h, buf, n)
+        wn = (C.c_uint64 * n)()
+        kw = self.L.pfpb200_multi_pfbwt_windows(self.h, wn, n)
+        d["ranks"] = [dict(buf[i].as_dict(), windows=wn[i] if i < kw else 0) for i in range(k)]
         return d
 
     def phase_ms(self):

@@ -412,10 +412,20 @@ int pfpb200_pfbwt_plan(const pfpb200_ctx *ctx, uint64_t *windows, uint64_t *peak
  * travel peer to peer, so every rank holds the dictionary and the parse-side streams; the dictionary
  * suffixes are partitioned by their first symbols, sorted by prefix doubling with the rank array
  * spread over the GPUs (direct peer loads and stores: two different devices in the list need peer
- * access), and every rank writes its contiguous piece of .bwt / .sa / .ssa / .esa into files rank 0
- * created at their final sizes.  res: counts summed over the ranks, device pointers NULL, times the
- * maximum over the ranks.  Limits: fewer than 2^32 suffixes per rank and fewer than 2^32 occurrences
- * in one group of equal suffixes (PFPB200_E_LIMIT: list more GPUs), parse < 2^32-2 words. */
+ * access).  No rank holds an array over the whole dictionary other than the dictionary itself: the words
+ * of its own suffixes come from the word ends.  Every rank writes its contiguous piece of .bwt / .sa into
+ * the files rank 0 created at their final sizes, in windows of whole groups of equal suffixes as
+ * pfpb200_pfbwt_file does when its outputs do not fit: one window when the piece's output fits the rank's
+ * budget, which is PFPB200_PFBWT_BUDGET=<bytes> per rank if set, else the free memory plus the rank's
+ * unused arena for a rank alone on its device, and its share of the free memory for one of several ranks
+ * listed on the same device.  The run samples of .ssa / .esa go to part files
+ * <basename>.ssa.<g> / .esa.<g> first; once the ranks know each other's first and last chars, every rank
+ * copies its part, less a record the run across a rank border makes redundant, into the final file at its
+ * offset, and the part files are removed (on failure as well).  res: counts summed over the ranks, device
+ * pointers NULL, times the maximum over the ranks; pfpb200_multi_pfbwt_windows gives the windows per rank.
+ * Limits: fewer than 2^32 suffixes per rank and fewer than 2^32 occurrences in one group of equal suffixes
+ * (PFPB200_E_LIMIT: list more GPUs), parse < 2^32-2 words; a group of equal suffixes is written in one
+ * window, whatever the budget. */
 int pfpb200_multi_pfbwt_file(pfpb200_multi *m, const char *basename, uint32_t w, uint32_t flags,
                              pfpb200_pfbwt_result *res);
 typedef struct pfpb200_pfbwt_rank {
@@ -423,10 +433,14 @@ typedef struct pfpb200_pfbwt_rank {
     uint64_t chars;                          /* BWT chars (and SA values) it wrote                   */
     uint64_t hard;                           /* of those, through the merge of the .ilist cursors    */
     uint64_t peak_bytes;                     /* peak device memory of its context                    */
-    float ms_read, ms_sort, ms_emit, ms_write;   /* wall clock: inputs, suffix sort, emission, files */
+    float ms_read, ms_sort, ms_emit, ms_write;   /* wall clock: inputs, suffix sort, emission (plan and
+                                                    windows), files (with the run samples' stitching) */
 } pfpb200_pfbwt_rank;
 /* per-rank figures of the last pfpb200_multi_pfbwt_file call: fills up to cap entries, returns how many */
 int pfpb200_multi_pfbwt_ranks(const pfpb200_multi *m, pfpb200_pfbwt_rank *out, int cap);
+/* output windows each rank of the last pfpb200_multi_pfbwt_file call wrote its piece in (0: the rank owned
+ * no dictionary suffix): fills up to cap entries, returns how many; m or windows NULL: PFPB200_E_ARG */
+int pfpb200_multi_pfbwt_windows(const pfpb200_multi *m, uint64_t *windows, int cap);
 
 /* ---- the whole pipeline in one call --------------------------------------------------------------------- *
  * What `bigbwt <file> -w W -p P [-f] [-S | -s -e] [-k]` does with three processes and the files between
