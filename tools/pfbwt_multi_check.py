@@ -16,14 +16,10 @@ rank's windows, device peak and times.
               the sharded .ssa / .esa must equal its files (sha256); .bwt is checked as with -S.
   --reps K    the sharded call K times; the per-rank medians of sort / emission wall clock and peaks.
 
-The linear checks of the written .sa / .bwt (the suffix-array row 0 is the end-of-text suffix, which
-.sa leaves out):
-  * the suffix array is a permutation of [0, n];
-  * bwt[i] == T[sa[i] - 1], and the EOF char 0 sits at the row of the suffix at position 0;
-  * adjacent rows: T[sa[i]] < T[sa[i+1]], or they are equal and ISA[sa[i]+1] < ISA[sa[i+1]+1]
-    (Burkhardt-Kaerkkaeinen), the end of the text smaller than every char.
-This checks the files; it is not a second suffix sort.  A case that does not fit (device memory, disk,
-too few GPUs) prints a "not run" line with the reason and exits 0; a failed check exits 1.
+The linear checks of the written .sa / .bwt are oracle/sa_check.py's (permutation, bwt[i] == T[sa[i] - 1],
+the EOF row, Burkhardt-Kaerkkaeinen order of adjacent rows); they check the files, not a second suffix
+sort.  A case that does not fit (device memory, disk, too few GPUs) prints a "not run" line with the
+reason and exits 0; a failed check exits 1.
 usage: pfbwt_multi_check.py --config {2,3,4} [--ranks 0,0,0,0] [--flags S|se] [--reps K] [--dir DIR]"""
 import argparse
 import hashlib
@@ -39,7 +35,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 
-CHUNK = 1 << 28
+from oracle.sa_check import linear_checks, load_sa  # noqa: E402
 
 
 def emit(d):
@@ -54,61 +50,6 @@ def sha(path):
             if not b:
                 return h.hexdigest()
             h.update(b)
-
-
-def load_sa(path, n):
-    """.sa (n values of 5 bytes, rows 1..n) -> int64 suffix array of rows 0..n on the device"""
-    sa = torch.empty(n + 1, dtype=torch.int64, device="cuda")
-    sa[0] = n
-    w = torch.tensor([1 << (8 * j) for j in range(5)], dtype=torch.int64, device="cuda")
-    with open(path, "rb") as f:
-        i = 1
-        while i <= n:
-            k = min(CHUNK, n + 1 - i)
-            b = torch.frombuffer(bytearray(f.read(5 * k)), dtype=torch.uint8).cuda().view(k, 5).to(torch.int64)
-            sa[i:i + k] = (b * w).sum(1)
-            i += k
-    return sa
-
-
-def linear_checks(T, sa, bwt):
-    """T: text (uint8, n), sa: int64 (n + 1 rows), bwt: uint8 (n + 1) -- all on the device"""
-    n = T.numel()
-    fails = []
-    if bwt.numel() != n + 1 or sa.numel() != n + 1:
-        return [f"sizes: bwt {bwt.numel()}, sa {sa.numel()}, text {n}"]
-    if int(sa.min()) < 0 or int(sa.max()) > n:
-        return ["suffix array values outside [0, n]"]
-    isa = torch.full((n + 2,), -1, dtype=torch.int64, device="cuda")
-    for a in range(0, n + 1, CHUNK):
-        b = min(n + 1, a + CHUNK)
-        isa[sa[a:b]] = torch.arange(a, b, dtype=torch.int64, device="cuda")
-    if bool((isa[:n + 1] < 0).any()):
-        fails.append("the suffix array is not a permutation of [0, n]")
-        return fails
-    isa[n + 1] = -1
-    Tx = torch.empty(n + 1, dtype=torch.int16, device="cuda")
-    Tx[:n] = T.to(torch.int16)
-    Tx[n] = -1                                                    # the end of the text: smaller than every char
-    bad_bwt = bad_order = 0
-    for a in range(0, n + 1, CHUNK):
-        b = min(n + 1, a + CHUNK)
-        s = sa[a:b]
-        prev = torch.where(s > 0, Tx[(s - 1).clamp(min=0)], torch.zeros_like(s, dtype=torch.int16))
-        bad_bwt += int((prev != bwt[a:b].to(torch.int16)).sum())
-        e = min(b, n)                                             # rows a..e-1 against rows a+1..e
-        if e > a:
-            s0, s1 = sa[a:e], sa[a + 1:e + 1]
-            c0, c1 = Tx[s0], Tx[s1]
-            r0 = isa[(s0 + 1).clamp(max=n + 1)]
-            r1 = isa[(s1 + 1).clamp(max=n + 1)]
-            ok = (c0 < c1) | ((c0 == c1) & (r0 < r1))
-            bad_order += int((~ok).sum())
-    if bad_bwt:
-        fails.append(f"bwt[i] != T[sa[i]-1] at {bad_bwt} rows")
-    if bad_order:
-        fails.append(f"adjacent rows out of order at {bad_order} places")
-    return fails
 
 
 def prepare(pkg, sc, text, w, p, base):
