@@ -45,6 +45,7 @@ static int multi_bigbwt(const char *path, const pfpb200_opts *opts, unsigned fla
     pfpb200_stats st;
     pfpb200_bwtparse_result bp;
     pfpb200_pfbwt_result r;
+    uint64_t bp_windows = 0, bp_peak = 0;
     int rc = pfpb200_multi_create(n_dev, devices, &multi);
     if (rc != PFPB200_OK) {
         fprintf(stderr, "gpubigbwt: cannot use the %d listed CUDA devices: %s\n", n_dev, pfpb200_strerror(rc));
@@ -57,6 +58,7 @@ static int multi_bigbwt(const char *path, const pfpb200_opts *opts, unsigned fla
         rc = pfpb200_create(devices[0], &ctx);
         if (rc == PFPB200_OK) rc = pfpb200_bwtparse_file(ctx, path, 1, 0, &bp);
         if (rc == PFPB200_OK) {
+            pfpb200_bwtparse_plan(ctx, &bp_windows, &bp_peak);
             pfpb200_destroy(ctx);                 /* its HBM goes back before the last stage */
             ctx = NULL;
             stage = "pfbwt";
@@ -85,6 +87,7 @@ static int multi_bigbwt(const char *path, const pfpb200_opts *opts, unsigned fla
         printf("Plan: output windows per rank:");
         for (int g = 0; g < k; g++) printf("%s%llu", g ? "," : " ", (unsigned long long)wn[g]);
         printf("\n");
+        printf("Plan: bwtparse %llu windows, peak %.3f GB\n", (unsigned long long)bp_windows, (double)bp_peak * 1e-9);
     }
     if (!keep) {
         char name[4096];
@@ -171,6 +174,9 @@ int main(int argc, char **argv) {
     pfpb200_pfbwt_plan(ctx, &windows, &pfbwt_peak);
     printf("Plan: parse %llu chunks (0: in one piece), peak %.3f GB; pfbwt %llu windows, peak %.3f GB\n",
            (unsigned long long)chunks, (double)parse_peak * 1e-9, (unsigned long long)windows, (double)pfbwt_peak * 1e-9);
+    uint64_t bp_windows = 0, bp_peak = 0;
+    pfpb200_bwtparse_plan(ctx, &bp_windows, &bp_peak);
+    printf("Plan: bwtparse %llu windows, peak %.3f GB\n", (unsigned long long)bp_windows, (double)bp_peak * 1e-9);
     printf("==== Elapsed time: %.3f wall clock seconds\n",
            (double)(t1.tv_sec - t0.tv_sec) + 1e-9 * (double)(t1.tv_nsec - t0.tv_nsec));
     pfpb200_destroy(ctx);

@@ -63,6 +63,9 @@ int main(int argc, char **argv) {
            (unsigned long long)r.n_out * 4ull);
     printf("GPU bwtparse: %.3f ms (suffix array %.3f in %u doubling rounds, BWT + lists %.3f), %u kernel launches\n",
            r.ms_total, r.ms_sa, r.rounds, r.ms_lists, r.launches);
+    uint64_t windows = 0, peak = 0;
+    pfpb200_bwtparse_plan(ctx, &windows, &peak);
+    printf("Plan: bwtparse %llu windows, peak %.3f GB\n", (unsigned long long)windows, (double)peak * 1e-9);
     printf("==== Elapsed time: %.0f wall clock seconds\n", difftime(time(NULL), start));
     pfpb200_destroy(ctx);
     return 0;

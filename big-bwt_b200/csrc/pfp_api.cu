@@ -570,7 +570,8 @@ extern "C" int pfpb200_parse_plan(const pfpb200_ctx *ctx, uint64_t *chunks, uint
 // != 0 also the intermediate files the reference leaves behind with `bigbwt -k`.  An input that does not
 // fit (the rule of pfpb200_parse_file) goes through the files as the reference's stages do: the streamed
 // parse writes them, bwtparse reads them, and pfbwt reads .dict / .occ and takes the parse's BWT from
-// HBM.  Either way pfbwt writes its outputs in windows when they do not fit (DESIGN.md §6c).
+// HBM, or from the files when bwtparse took its bounded path (DESIGN.md §6e).  Either way pfbwt writes
+// its outputs in windows when they do not fit (DESIGN.md §6c).
 extern "C" int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, uint32_t pfbwt_flags,
                                    int keep_files, pfpb200_stats *stats, pfpb200_bwtparse_result *bp_out,
                                    pfpb200_pfbwt_result *res) {
@@ -583,6 +584,7 @@ extern "C" int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfp
     o.nseg = 0;
     ctx->plan_chunks = ctx->plan_peak = 0;
     ctx->pb_windows = ctx->pb_peak = 0;
+    ctx->bp_windows = ctx->bp_peak = 0;
     bool streamed = false;
     u64 budget = 0;
     PFP_TRY(parse_route(ctx, path, &o, &streamed, &budget));
@@ -601,7 +603,10 @@ extern "C" int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfp
         PFP_TRY(parse_file_impl(ctx, path, &o, &st, keep_files != 0, &dv));
         ctx->plan_peak = ctx->arena.peak;
         t0 = wall_sec();
+        ctx->arena.peak = ctx->arena.in_use;                   // pfpb200_bwtparse_plan reports the bwtparse step's peak
         PFP_TRY(pfpb200_bwtparse_device(ctx, dv.parse, dv.n_phrases, dv.last, dv.sai, &bp));
+        ctx->bp_windows = 1;
+        ctx->bp_peak = ctx->arena.peak;
         if (keep_files) {
             PFP_TRY(put("ilist", bp.ilist, bp.n_out * 4));
             PFP_TRY(put("bwlast", bp.bwlast, bp.n_out));
@@ -618,15 +623,19 @@ extern "C" int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfp
         pfp_release_held(ctx);
         t0 = wall_sec();
         if (rc == PFPB200_OK) rc = pfpb200_bwtparse_file(ctx, path, 1, 0, &bp);
-        void *f[2] = {nullptr, nullptr};
-        u64 n[2] = {0, 0};
-        for (int k = 0; k < 2 && rc == PFPB200_OK; k++) rc = pb_read_file(ctx, path, k, &f[k], &n[k]);
+        // the bounded bwtparse leaves its outputs in the files only: pfbwt reads them from there
+        const int nf = rc == PFPB200_OK && !bp.ilist ? 5 : 2;
+        void *f[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+        u64 n[5] = {0, 0, 0, 0, 0};
+        for (int k = 0; k < nf && rc == PFPB200_OK; k++) rc = pb_read_file(ctx, path, k, &f[k], &n[k]);
         in.d = static_cast<u8 *>(f[0]); in.N = n[0]; in.occ = static_cast<u32 *>(f[1]); in.dwords = n[1];
+        in.ilist = static_cast<u32 *>(f[2]); in.bwlast = static_cast<u8 *>(f[3]); in.bwsai = static_cast<u8 *>(f[4]);
     }
     if (rc == PFPB200_OK) {
         if (stats) *stats = st;
         if (bp_out) *bp_out = bp;
-        in.ilist = bp.ilist; in.bwlast = bp.bwlast; in.bwsai = bp.bwsai; in.psize = bp.n_out;
+        if (bp.ilist) { in.ilist = bp.ilist; in.bwlast = bp.bwlast; in.bwsai = bp.bwsai; }
+        in.psize = bp.n_out;
         ctx->arena.peak = ctx->arena.in_use;                   // pfpb200_pfbwt_plan reports the pfbwt step's peak
         rc = pb_to_files(ctx, in, path, res);
     }

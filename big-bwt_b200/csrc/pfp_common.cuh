@@ -79,6 +79,7 @@ struct pfpb200_ctx {
     double dedup_ratio = 0.0;      // distinct words / phrases of the previous parse (table sizing hint)
     u64 plan_chunks = 0, plan_peak = 0;   // pfpb200_parse_plan: chunks (0: one-shot) and arena peak of the last parse_file
     u64 pb_windows = 0, pb_peak = 0;      // pfpb200_pfbwt_plan: output windows and arena peak of the last pfbwt file call
+    u64 bp_windows = 0, bp_peak = 0;      // pfpb200_bwtparse_plan: round-1 windows (1: in HBM) and arena peak of the last bwtparse file call
     char err[512] = {0};
     std::vector<void *> scratch;   // freed at the end of every call
     std::vector<void *> held;      // outputs: freed at the start of the next call / destroy

@@ -133,7 +133,7 @@ SYMBOLS = ["pfpb200_create", "pfpb200_destroy", "pfpb200_set_stream", "pfpb200_p
            "pfpb200_multi_phase_ms", "pfpb200_multi_pfbwt_file", "pfpb200_multi_pfbwt_ranks",
            "pfpb200_multi_pfbwt_windows",
            "pfpb200_check_dict_order",
-           "pfpb200_bwtparse_device", "pfpb200_bwtparse_host", "pfpb200_bwtparse_file",
+           "pfpb200_bwtparse_device", "pfpb200_bwtparse_host", "pfpb200_bwtparse_file", "pfpb200_bwtparse_plan",
            "pfpb200_unparse_device", "pfpb200_unparse_file",
            "pfpb200_pfbwt_device", "pfpb200_pfbwt_file", "pfpb200_pfbwt_plan", "pfpb200_bigbwt_file",
            "pfpb200_launch_count", "pfpb200_last_error", "pfpb200_abi_version"]
@@ -184,6 +184,8 @@ def load_library():
     L.pfpb200_bwtparse_host.restype = C.c_int
     L.pfpb200_bwtparse_file.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.POINTER(BwtParseResult)]
     L.pfpb200_bwtparse_file.restype = C.c_int
+    L.pfpb200_bwtparse_plan.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
+    L.pfpb200_bwtparse_plan.restype = C.c_int
     L.pfpb200_multi_create.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(vp)]
     L.pfpb200_multi_create.restype = C.c_int
     L.pfpb200_multi_destroy.argtypes = [vp]
@@ -362,9 +364,19 @@ class Scanner:
         return BwtParseFiles(il.tobytes(), bl.tobytes(), bs.tobytes() if sai else b"", r.as_dict())
 
     def bwtparse_file(self, basename, sai=False, nseg=0) -> dict:
+        """Writes <basename>.ilist .bwlast [.bwsai]; returns the result and, under "windows" and
+        "peak_device_bytes", how the call ran (windows 1: in HBM; see pfpb200_bwtparse_plan)."""
         r = BwtParseResult()
         self._check(self.L.pfpb200_bwtparse_file(self.h, os.fsencode(basename), 1 if sai else 0, nseg, C.byref(r)))
-        return r.as_dict()
+        d = r.as_dict()
+        d["windows"], d["peak_device_bytes"] = self.bwtparse_plan()
+        return d
+
+    def bwtparse_plan(self):
+        """(windows, peak device bytes) of the bwtparse step of the last bwtparse_file / bigbwt_file call."""
+        n, pk = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.L.pfpb200_bwtparse_plan(self.h, C.byref(n), C.byref(pk)))
+        return n.value, pk.value
 
     # -- the last stage: pfbwt (pfbwt.cpp) ------------------------------------------------------------------
     def pfbwt_device(self, dict_ptr, dict_bytes, occ_ptr, n_words, ilist_ptr, bwlast_ptr, bwsai_ptr, parse_size,
@@ -400,7 +412,8 @@ class Scanner:
     def bigbwt_file(self, path, w=10, p=100, fasta=False, flags=0, keep=False) -> dict:
         """The whole pipeline for a file: <path>.bwt (+ .sa / .ssa / .esa) written, stages in HBM, or through
         the files for a text larger than the device.  The plans of the parse ("chunks") and of pfbwt
-        ("windows"), each with its "peak_device_bytes", are in the "parse" and "pfbwt" entries."""
+        ("windows"), each with its "peak_device_bytes", are in the "parse" and "pfbwt" entries, and the plan
+        of bwtparse ("windows") in the "bwtparse" entry."""
         self.L.pfpb200_bigbwt_file.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(Opts), C.c_uint32, C.c_int,
                                                C.POINTER(Stats), C.POINTER(BwtParseResult), C.POINTER(PfbwtResult)]
         self.L.pfpb200_bigbwt_file.restype = C.c_int
@@ -411,6 +424,7 @@ class Scanner:
         d = {"parse": self.stats.as_dict(), "bwtparse": bp.as_dict(), "pfbwt": r.as_dict()}
         d["parse"]["chunks"], d["parse"]["peak_device_bytes"] = self.parse_plan()
         d["pfbwt"]["windows"], d["pfbwt"]["peak_device_bytes"] = self.pfbwt_plan()
+        d["bwtparse"]["windows"], d["bwtparse"]["peak_device_bytes"] = self.bwtparse_plan()
         return d
 
     def bwt_of_text(self, text, w=10, p=100, flags=0):

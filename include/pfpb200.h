@@ -346,7 +346,13 @@ int pfpb200_bwtparse_host(pfpb200_ctx *ctx, const uint32_t *parse, uint64_t n_ph
                           uint8_t *bwsai, pfpb200_bwtparse_result *res);
 /* `bwtparse <basename> [-s] [-t nseg]`: reads <basename>.parse, .last and (sa_info) .sai -- as nseg
  * segment files <basename>.<i>.last|sai when nseg > 0 (utils.c:57-110) -- and writes .ilist,
- * .bwlast and .bwsai (the device copies stay available through res, as above). */
+ * .bwlast and .bwsai (the device copies stay available through res, as above).  That is when the
+ * in-HBM suffix sort fits the device memory available to the call (free memory plus what the
+ * context's arena holds unused); a larger parse takes the bounded path: a few bytes per phrase stay
+ * resident, the sort runs in windows of whole symbol ranges and groups of suffixes, and the outputs
+ * are written to the files in windows.  res then carries counts, rounds and CUDA-event times with NULL
+ * device pointers.  PFPB200_BWTPARSE_BUDGET=<bytes> in the environment replaces the available-memory
+ * figure.  PFPB200_E_NOMEM when even the resident arrays and one window do not fit. */
 int pfpb200_bwtparse_file(pfpb200_ctx *ctx, const char *basename, int sa_info, int nseg,
                           pfpb200_bwtparse_result *res);
 
@@ -455,6 +461,12 @@ int pfpb200_multi_pfbwt_windows(const pfpb200_multi *m, uint64_t *windows, int c
 int pfpb200_bigbwt_file(pfpb200_ctx *ctx, const char *path, const pfpb200_opts *opts, uint32_t pfbwt_flags,
                         int keep_files, pfpb200_stats *stats, pfpb200_bwtparse_result *bp,
                         pfpb200_pfbwt_result *res);
+
+/* How the last pfpb200_bwtparse_file / pfpb200_bigbwt_file call ran bwtparse: *windows (1: the in-HBM
+ * path; otherwise the windows of the bounded path's first round) and *peak_device_bytes, the
+ * high-water mark of the context's device arena during that step.  NULL outputs are skipped; ctx NULL:
+ * PFPB200_E_ARG. */
+int pfpb200_bwtparse_plan(const pfpb200_ctx *ctx, uint64_t *windows, uint64_t *peak_device_bytes);
 
 const char *pfpb200_strerror(int code);
 /* Message of the last failure on this context (CUDA error string, file name, ...). */
